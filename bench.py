@@ -32,6 +32,11 @@ rank 0 in the same run) and the speed-up over it.
 
 ``--impl reference`` times the CPU arm alone and prints the same JSON line with
 ``"impl": "reference"``.
+
+``--dump-outputs DIR`` writes, on rank 0, what each timed GPU call returned in its last step as
+``DIR/<leg>_<op>.npy`` (float32, float64 where float32 would not hold the values), so that two
+builds can be compared output for output on the same seeded inputs: the whole array up to
+DUMP_CELLS cells, else DUMP_CELLS cells at fixed, seeded positions of the flattened array.
 """
 import argparse
 import json
@@ -40,6 +45,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 
@@ -50,6 +56,8 @@ METRIC = "fused raster chain throughput (Reclassify+Clip+Step+IsData)"
 UNIT = "Gpixel/s"
 BYTES_PER_PIXEL = 7  # int16 + float32 in, bool out
 ALL_LEGS = "chain,stencils,zonal,temporal"
+DUMP_CELLS = 1 << 19        # per output: 2 MB as float32; the 17 outputs of all legs stay under DUMP_BYTES
+DUMP_BYTES = 64 << 20
 
 
 def parse_args():
@@ -71,7 +79,11 @@ def parse_args():
     ap.add_argument("--no-single", action="store_true", help="skip the single-GPU reference runs at N > 1")
     ap.add_argument("--profile", action="store_true",
                     help="kernel-resident chain loop only (for ncu): no e2e, no CPU baseline, no other legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last step's output of every timed GPU call as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.leg_steps < 1 or args.e2e_steps < 1:
+        ap.error("--steps, --leg-steps and --e2e-steps must be at least 1")
     args.legs = [x for x in args.legs.split(",") if x]
     if args.no_zonal and "zonal" in args.legs:
         args.legs.remove("zonal")
@@ -317,6 +329,17 @@ class Context(object):
             self.traffic = json.load(open(path))
         # a group of rank 0 alone: the single-GPU reference runs of the striped legs
         self.solo = dist.new_group([0]) if world > 1 else None
+        self.outputs = {} if args.dump_outputs and rank == 0 else None
+
+    def keep(self, name, result):
+        """--dump-outputs: a sample of the arrays a timed call returned (see DUMP_CELLS)."""
+        if self.outputs is None:
+            return
+        if isinstance(result, tuple):       # zonal_striped: (per-polygon values, polygons without cells)
+            result = result[0]
+        if isinstance(result, dict):        # a block's payload
+            result = result["values"]
+        self.outputs[name] = output_sample(self.torch, result, zlib.crc32(name.encode()))
 
     def barrier(self):
         self.torch.cuda.synchronize()
@@ -366,10 +389,50 @@ def wrap(t):
     return _native.DeviceArray(tuple(t.shape), str(t.dtype).replace("torch.", ""), ptr=t.data_ptr(), owner=t)
 
 
+class _CudaArrayView(object):
+    """A DeviceArray as a torch CUDA tensor sharing its memory (``torch.as_tensor``)."""
+
+    def __init__(self, array):
+        self.__cuda_array_interface__ = {"shape": array.shape, "typestr": array.dtype.str,
+                                         "data": (array.ptr, False), "version": 2}
+        self.array = array
+
+
+def output_sample(torch, values, seed):
+    """Host copy of one output (DeviceArray, torch tensor or NumPy array): the whole array up to
+    DUMP_CELLS cells, else DUMP_CELLS cells at `seed`-determined flat positions, gathered on the
+    device; float32, or float64 where float32 would not hold every value."""
+    from dask_geomodeling_b200 import _native
+
+    if isinstance(values, _native.DeviceArray):
+        values = torch.as_tensor(_CudaArrayView(values), device="cuda")
+    elif not torch.is_tensor(values):
+        values = torch.from_numpy(np.ascontiguousarray(values))
+    shape = tuple(values.shape)
+    values = values.reshape(-1)
+    if values.numel() > DUMP_CELLS:
+        index = np.sort(np.random.default_rng(seed).integers(0, values.numel(), DUMP_CELLS))
+        values = values[torch.from_numpy(index).to(values.device)]
+        shape = (DUMP_CELLS,)
+    host = values.cpu().numpy().reshape(shape)
+    exact32 = host.dtype.itemsize <= 2 or host.dtype == np.float32
+    return host.astype(np.float32 if exact32 else np.float64)
+
+
+def write_outputs(directory, outputs):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError("{} bytes of outputs exceed the dump limit of {}".format(total, DUMP_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, array in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), array)
+
+
 def striped_entry(ctx, name, fn_striped, fn_single, pixels, nbytes, kernel, iters, traffic_key=None):
     """Time one operation on the sharded workload (all ranks) and, at N > 1, on the whole
-    workload on rank 0 alone; returns the JSON object of the entry."""
-    ms, launches, _ = ctx.time_calls(fn_striped, iters)
+    workload on rank 0 alone; returns the JSON object of the entry.  `name` is <leg>_<op>."""
+    ms, launches, out = ctx.time_calls(fn_striped, iters)
+    ctx.keep(name, out)
     entry = {"ms": ms, "gpx_s": pixels / ms / 1e6, "gpu_launches_per_call": launches,
              "roofline": ctx.roofline(nbytes, ms, kernel, traffic_key=traffic_key)}
     if ctx.world > 1 and not ctx.args.no_single:      # (every rank takes this branch: broadcast below)
@@ -437,7 +500,7 @@ def run_stencils(ctx):
             stored_whole = parallel.pad_columns(
                 parallel.exchange_halo(whole, halo_rows, nodata, group=ctx.solo), halo_cols, nodata, pitch)
         entry = striped_entry(
-            ctx, name,
+            ctx, "stencils_" + name,
             lambda: parallel.stencil_haloed(process, stored, nodata, halo_rows, halo_cols, *extra),
             None if stored_whole is None else (lambda: parallel.stencil_haloed(
                 process, stored_whole, nodata, halo_rows, halo_cols, *extra, group=ctx.solo)),
@@ -505,7 +568,7 @@ def run_zonal(ctx, host_raster):
             if whole is not None:
                 def single(stat=stat, q=q):
                     return parallel.zonal_striped(soup, whole, nodata, bbox, n, (0, n), stat, q, group=ctx.solo)
-            entry = striped_entry(ctx, label, striped, single, px, px * 4, kernels[label], args.leg_steps,
+            entry = striped_entry(ctx, "zonal_" + label, striped, single, px, px * 4, kernels[label], args.leg_steps,
                                   traffic_key="zonal_" + label)
             with _native.use_stream(ctx.stream.cuda_stream):
                 res, no_cells = striped()
@@ -556,6 +619,7 @@ def zonal_e2e(ctx, host_raster):
                 frame = view.get_data(**request)["features"]
             _native.synchronize()
             seconds = (time.perf_counter() - t0) / 3
+            ctx.keep("zonal_e2e_" + label, frame["agg"].values)
             e2e[label] = {"value": size * size / seconds / 1e9, "ms_per_request": seconds * 1e3,
                           "d2h_bytes_per_step": 4 * len(frame),
                           "checksum": float(np.nansum(frame["agg"].values.astype(np.float64)))}
@@ -598,7 +662,7 @@ def run_temporal(ctx):
     for stat in ("sum", "max"):
         kw = kwargs_for(stat)
         entry = striped_entry(
-            ctx, stat,
+            ctx, "temporal_" + stat,
             lambda kw=kw: raster.TemporalAggregate.process(kw, {"time": times}, {"values": sd, "no_data_value": nodata}),
             None if whole is None else (lambda kw=kw: raster.TemporalAggregate.process(
                 kw, {"time": times}, {"values": whole, "no_data_value": nodata})),
@@ -614,16 +678,18 @@ def run_temporal(ctx):
         for stat, kernel in (("mean", "temporal_stream_kernel<float, mean>"), ("std", "temporal_moments_stream_kernel"),
                              ("median", "temporal_sort_reg_kernel")):
             kw = dict(kwargs_for(stat), start=sub_times[-1])
-            ms, launches, _ = ctx.time_calls(lambda kw=kw: raster.TemporalAggregate.process(
+            ms, launches, res = ctx.time_calls(lambda kw=kw: raster.TemporalAggregate.process(
                 kw, {"time": sub_times}, {"values": sub, "no_data_value": nodata}), iters)
+            ctx.keep("temporal_{}_{}frames".format(stat, t64), res)
             nb = (2 if stat == "std" else 1) * px64 * 4 + (r1 - r0) * m * 4     # std reads the frames twice
             out["{}_{}frames".format(stat, t64)] = {
                 "ms": ms, "gpx_s": px64 / ms / 1e6, "gpu_launches_per_call": launches,
                 "roofline": ctx.roofline(nb, ms, kernel, traffic_key="temporal_" + stat)}
         kw = dict(mode="vals", start=sub_times[0], stop=sub_times[-1], frequency=None, timezone=None,
                   closed="right", label="right", dtype="<f4", statistic="sum")
-        ms, launches, _ = ctx.time_calls(lambda: raster.Cumulative.process(
+        ms, launches, res = ctx.time_calls(lambda: raster.Cumulative.process(
             kw, {"time": sub_times}, {"values": sub, "no_data_value": nodata}), iters)
+        ctx.keep("temporal_cumulative_sum_{}frames".format(t64), res)
         out["cumulative_sum_{}frames".format(t64)] = {
             "ms": ms, "gpx_s": px64 / ms / 1e6, "gpu_launches_per_call": launches,
             "roofline": ctx.roofline(2 * px64 * 4, ms, "temporal_cumulative_stream_kernel", traffic_key="cumulative_sum"),
@@ -643,8 +709,9 @@ def run_temporal(ctx):
         si = wrap(i16)
         for stat, out_bytes in (("sum", 4), ("max", 2)):
             kw = kwargs_for(stat, dtype="i4" if stat == "sum" else "i2")
-            ms, launches, _ = ctx.time_calls(lambda kw=kw: raster.TemporalAggregate.process(
+            ms, launches, res = ctx.time_calls(lambda kw=kw: raster.TemporalAggregate.process(
                 kw, {"time": times}, {"values": si, "no_data_value": 32767}), iters)
+            ctx.keep("temporal_{}_int16".format(stat), res)
             nb = T * m * m * 2 + m * m * out_bytes
             out["{}_int16".format(stat)] = {
                 "ms": ms, "gpx_s": px / ms / 1e6, "gpu_launches_per_call": launches,
@@ -783,6 +850,7 @@ def run_b200(args):
         elapsed_ms = start.elapsed_time(stop)
         clocks = sampler.stop() if sampler else None
         checksum = int(np.asarray(out.to_host()).sum())
+        ctx.keep("chain", out)
         del inputs, leaf_payloads, out
     assert e2e_checksum is None or e2e_checksum == checksum, "e2e result differs from the resident result"
 
@@ -847,6 +915,8 @@ def run_b200(args):
                 "sample": "the whole {0}x{0} request, 2048 x 2048 tiles on a thread pool, best of 3 "
                           "({1:.2f} s); result equal to the GPU arm's".format(size, best),
             }
+        if ctx.outputs is not None:
+            write_outputs(args.dump_outputs, ctx.outputs)
         json_out.write(json.dumps(line) + "\n")
         json_out.flush()
     if world > 1:
