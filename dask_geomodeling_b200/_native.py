@@ -109,6 +109,21 @@ class GmZonalPartial(ctypes.Structure):
     ]
 
 
+class GmWarp(ctypes.Structure):
+    _fields_ = [
+        ("dst_kind", ctypes.c_int32),
+        ("dst_zone", ctypes.c_int32),
+        ("src_kind", ctypes.c_int32),
+        ("src_zone", ctypes.c_int32),
+        ("dst_geo", ctypes.c_double * 6),
+        ("src_geo", ctypes.c_double * 6),
+        ("src_height", ctypes.c_int64),
+        ("src_width", ctypes.c_int64),
+        ("win_row0", ctypes.c_int64),
+        ("win_col0", ctypes.c_int64),
+    ]
+
+
 # every symbol include/geokernels.h declares: name -> (restype, argtypes)
 _vp, _i, _i64, _d = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
 _P = ctypes.POINTER
@@ -143,6 +158,7 @@ SYMBOLS = {
     "gm_jit_check": (_i, [_P(GmProgram), _P(ctypes.c_int32), _P(ctypes.c_int32), _P(_i64)]),
     "gm_jit_compile_count": (_i64, []),
     "gm_resample_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _d, _d, _d, _d, _vp]),
+    "gm_warp_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _P(GmWarp), _P(_i64), _vp]),
     "gm_hillshade": (_i, [_P(GmArray), _P(GmArray), _vp, _i, _d, _d, _d, _d, _d, _vp]),
     "gm_moving_max": (_i, [_P(GmArray), _P(GmArray), _vp, _i, _i, _vp]),
     "gm_dilate": (_i, [_P(GmArray), _P(GmArray), _vp, _i, _vp]),

@@ -45,6 +45,11 @@ inline int dtype_size(int dt) {
   return 0;
 }
 
+// non-finite float source values become no data in the resample / warp gathers
+template <typename T> __device__ __forceinline__ bool is_finite(T v) { return true; }
+template <> __device__ __forceinline__ bool is_finite<float>(float v) { return isfinite(v); }
+template <> __device__ __forceinline__ bool is_finite<double>(double v) { return isfinite(v); }
+
 inline int64_t array_count(const GmArray& a) { return a.shape[0] * a.shape[1] * a.shape[2]; }
 inline int64_t array_bytes(const GmArray& a) { return array_count(a) * dtype_size(a.dtype); }
 

@@ -11,9 +11,6 @@ __global__ void fill_kernel(T* __restrict__ dst, T value, int64_t n) {
     dst[i] = value;
 }
 
-template <typename T> __device__ __forceinline__ bool is_finite(T v) { return true; }
-template <> __device__ __forceinline__ bool is_finite<float>(float v) { return isfinite(v); }
-template <> __device__ __forceinline__ bool is_finite<double>(double v) { return isfinite(v); }
 
 // out[b, i, j] = src[b, floor(row0 + i*row_step), floor(col0 + j*col_step)], or
 // nodata outside the source window; non-finite floats become nodata

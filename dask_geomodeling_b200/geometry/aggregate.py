@@ -85,6 +85,16 @@ def _read_cells(values, rows, cols):
     return out
 
 
+class _LazyTransformed(object):
+    """``geometries[i]`` transformed from ``src`` to ``dst`` on access."""
+
+    def __init__(self, geometries, src, dst):
+        self.geometries, self.src, self.dst = geometries, src, dst
+
+    def __getitem__(self, i):
+        return utils.shapely_transform(self.geometries[i], self.src, self.dst)
+
+
 def aggregate_polygons(geometries, values, no_data_value, agg_bbox, agg_srs, threshold_values,
                        statistic, percentile):
     """Statistic of ``values`` (t, h, w) under every geometry.
@@ -285,7 +295,18 @@ class AggregateRaster(GeometryBlock):
                 else:
                     soup = full.subset(positions)
         else:
-            agg_geometries = [utils.shapely_transform(g, req_srs, agg_srs) for g in column]
+            # the vertices are transformed in one vectorised call on the CSR form; geometry
+            # objects in the raster's CRS are built only for the centroid fallback below
+            from .sources import prepared_soup_of
+
+            prepared = prepared_soup_of(features)
+            if prepared is not None:
+                full, positions, _ = prepared
+                soup = full if len(positions) == full.n_polygons else full.subset(positions)
+            else:
+                soup = utils.PolygonSoup(list(column.values))
+            soup = soup.transformed(req_srs, agg_srs)
+            agg_geometries = _LazyTransformed(column.values, req_srs, agg_srs)
 
         statistic, percentile = utils.parse_percentile_statistic(process_kwargs["statistic"])
         extensive = AggregateRaster.STATISTICS[statistic]["extensive"]

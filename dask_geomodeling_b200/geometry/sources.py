@@ -4,7 +4,8 @@ The reference ships only file/WKT based geometry sources (geometry/sources.py,
 out of scope: vector file I/O); its tests feed AggregateRaster/Rasterize from
 ``MockGeometry`` (tests/factories.py:193-282).  ``MemoryGeometrySource`` is that
 idea as a supported block: polygons (lists of rings or shapely-like objects)
-plus per-feature properties, answered without reprojection.
+plus per-feature properties, answered in the request's projection (EPSG:4326, EPSG:3857 and
+the WGS 84 UTM zones; see crs.py).
 """
 import numpy as np
 import pandas as pd
@@ -79,22 +80,29 @@ def _bounds(soup, geometries):
     return bounds
 
 
-def _prepared(polygons):
-    """Geometry objects, CSR soup and bounding boxes of a polygon list, built once per list
-    object (the list is an argument of the block, i.e. it lives as long as the view)."""
+def _prepared(polygons, projection=None, target=None):
+    """Geometry objects, CSR soup and bounding boxes of a polygon list in CRS ``target``, built
+    once per list object and target (the list is an argument of the block, i.e. it lives as long
+    as the view).  In another CRS than the list's ``projection`` the soup's vertices are
+    transformed in one vectorised call and the geometry objects vertex by vertex."""
     # the list must not be edited in place afterwards; a sample of its elements' identities
     # (first, last, 30 in between) catches the edits that keep its length
     n = len(polygons)
     sample = tuple(id(polygons[i]) for i in sorted(set(np.linspace(0, n - 1, 32).astype(int).tolist()))) if n else ()
-    hit = _PREPARED.get(id(polygons))
+    same = target is None or utils.same_projection(projection, target)
+    key = (id(polygons), None if same else (utils.get_epsg_or_wkt(projection), utils.get_epsg_or_wkt(target)))
+    hit = _PREPARED.get(key)
     if hit is not None and hit[0] is polygons and len(hit[1]) == n and hit[4] == sample:
         return hit[1], hit[2], hit[3]
     geometries = [_as_geometry(p) for p in polygons]
     soup = utils.PolygonSoup(geometries)
+    if not same:
+        soup = soup.transformed(projection, target)
+        geometries = [utils.shapely_transform(g, projection, target) for g in geometries]
     bounds = _bounds(soup, geometries)
     if len(_PREPARED) >= 8:
         _PREPARED.pop(next(iter(_PREPARED)))
-    _PREPARED[id(polygons)] = (polygons, geometries, soup, bounds, sample)
+    _PREPARED[key] = (polygons, geometries, soup, bounds, sample)
     return geometries, soup, bounds
 
 
@@ -137,13 +145,7 @@ class MemoryGeometrySource(GeometryBlock):
             polygons = polygons[:limit]
             properties = properties[:limit] if properties is not None else None
         mode = request.get("mode", "intersects")
-        same = utils.same_projection(projection, request["projection"])
-        geometries, soup, bounds = _prepared(polygons) if same else (None, None, None)
-        if geometries is None:
-            geometries = [utils.shapely_transform(_as_geometry(p), projection, request["projection"])
-                          for p in polygons]
-            soup = utils.PolygonSoup(geometries)
-            bounds = _bounds(soup, geometries)
+        geometries, soup, bounds = _prepared(polygons, projection, request["projection"])
         if mode == "extent":
             extent = None
             if len(geometries):

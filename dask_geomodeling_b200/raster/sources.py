@@ -6,7 +6,9 @@ nearest-neighbour warp (raster/sources.py:119-149) by: upload of only the
 source window the request touches (pinned host memory -> HBM), followed by a
 nearest-neighbour gather kernel that also pads with no data outside the
 source.  For aligned requests this equals the crop/pad GDAL produces.
-Requests in another projection than the source need GDAL/pyproj and raise.
+Requests in another projection than the source take the nearest-neighbour warp
+(``warp_window``, gm_warp_nn) when both CRSs are EPSG:4326, EPSG:3857 or a WGS 84
+UTM zone (``dask_geomodeling_b200/crs.py``); other pairs need GDAL/pyproj and raise.
 
 ``RasterFileSource`` (raster/sources.py:396-564) reads a GeoTIFF or VRT without GDAL
 (``dask_geomodeling_b200/geotiff.py``): only the tiles under the requested window are inflated,
@@ -18,7 +20,7 @@ from datetime import datetime, timedelta, timezone
 
 import numpy as np
 
-from .. import _native, _state, geotiff, utils
+from .. import _native, _state, crs, geotiff, utils
 from .._compat import config
 from .base import RasterBlock
 
@@ -95,6 +97,32 @@ def source_window(geo_transform, bbox, height, width, src_h, src_w):
     return r_lo, max(r_hi, r_lo), c_lo, max(c_hi, c_lo)
 
 
+def upload_window(array, b0, window, target):
+    """Copy cells ``window = (r_lo, r_hi, c_lo, c_hi)`` of bands b0.. of a host array into the
+    DeviceArray ``target`` of shape (bands, r_hi - r_lo, c_hi - c_lo)."""
+    lib = _native.lib()
+    stream = _native.current_stream()
+    r_lo, r_hi, c_lo, c_hi = window
+    n_bands, win_h, win_w = target.shape
+    src_h, src_w = array.shape[1:]
+    item = array.dtype.itemsize
+    if win_w == src_w and array.flags.c_contiguous:
+        for band in range(n_bands):
+            src_ptr = array.ctypes.data + ((b0 + band) * src_h + r_lo) * src_w * item
+            _native.check(lib.gm_memcpy_h2d(
+                target.ptr + band * win_h * win_w * item, src_ptr, win_h * win_w * item, stream))
+    else:
+        strides = array.strides
+        if strides[2] != item:
+            array = np.ascontiguousarray(array)
+            strides = array.strides
+        for band in range(n_bands):
+            src_ptr = array.ctypes.data + (b0 + band) * strides[0] + r_lo * strides[1] + c_lo * item
+            _native.check(lib.gm_memcpy2d_h2d(
+                target.ptr + band * win_h * win_w * item, win_w * item, src_ptr, strides[1],
+                win_w * item, win_h, stream))
+
+
 def resample_window(array, bands, geo_transform, no_data_value, bbox, height, width, keep_on_device,
                     row_range=None, origin=(0, 0)):
     """Nearest-neighbour resample of ``array[bands[0]:bands[1]]`` into the request grid.
@@ -135,28 +163,13 @@ def resample_window(array, bands, geo_transform, no_data_value, bbox, height, wi
             ctypes.byref(src_desc), ctypes.byref(dst_desc), nodata_ptr,
             col0, col_step, row0, row_step, stream))
     else:
-        item = dtype.itemsize
         exact = (
             dtype.kind != "f" and col_step == 1.0 and row_step == 1.0
             and c_lo == int(np.floor(col0)) and r_lo == int(np.floor(row0))
             and win_h == height and win_w == width
         )
         target = out if exact else _native.DeviceArray((n_bands, win_h, win_w), dtype)
-        if win_w == src_w and array.flags.c_contiguous:
-            for band in range(n_bands):
-                src_ptr = array.ctypes.data + ((b0 + band) * src_h + r_lo) * src_w * item
-                _native.check(lib.gm_memcpy_h2d(
-                    target.ptr + band * win_h * win_w * item, src_ptr, win_h * win_w * item, stream))
-        else:
-            strides = array.strides
-            if strides[2] != item:
-                array = np.ascontiguousarray(array)
-                strides = array.strides
-            for band in range(n_bands):
-                src_ptr = array.ctypes.data + (b0 + band) * strides[0] + r_lo * strides[1] + c_lo * item
-                _native.check(lib.gm_memcpy2d_h2d(
-                    target.ptr + band * win_h * win_w * item, win_w * item, src_ptr, strides[1],
-                    win_w * item, win_h, stream))
+        upload_window(array, b0, (r_lo, r_hi, c_lo, c_hi), target)
         if not exact:
             src_desc = _native.as_gm_array(target)
             dst_desc = _native.as_gm_array(out)
@@ -164,6 +177,111 @@ def resample_window(array, bands, geo_transform, no_data_value, bbox, height, wi
                 ctypes.byref(src_desc), ctypes.byref(dst_desc), nodata_ptr,
                 col0 - c_lo, col_step, row0 - r_lo, row_step, stream))
     return out if keep_on_device else out.to_host()
+
+
+WINDOW_EDGE_POINTS = 64   # outline points per edge of a request mapped into the source CRS
+WINDOW_MARGIN = 2         # cells added around the mapped outline
+
+
+def request_outline(bbox, n=WINDOW_EDGE_POINTS):
+    """Points along the outline of a request bbox, ``n`` intervals per edge."""
+    x1, y1, x2, y2 = bbox
+    t = np.linspace(0.0, 1.0, n + 1)
+    xs, ys = x1 + t * (x2 - x1), y1 + t * (y2 - y1)
+    return np.concatenate([
+        np.stack([xs, np.full_like(t, y1)], 1), np.stack([xs, np.full_like(t, y2)], 1),
+        np.stack([np.full_like(t, x1), ys], 1), np.stack([np.full_like(t, x2), ys], 1),
+    ])
+
+
+def warp_source_window(geo_transform, bbox, projection, source_projection, src_h, src_w):
+    """(r_lo, r_hi, c_lo, c_hi): the source cells a request in another CRS reads, estimated from
+    its outline mapped into the source CRS plus a margin.  Cells the estimate leaves out are
+    counted by the warp kernel, and the caller then repeats the warp with the whole source."""
+    p, a, _, q, _, d = geo_transform
+    xy = crs.transform(request_outline(bbox), projection, source_projection)
+    with np.errstate(invalid="ignore"):
+        cols = np.floor((xy[:, 0] - p) / a + 1e-10)
+        rows = np.floor((xy[:, 1] - q) / d + 1e-10)
+    finite = np.isfinite(cols) & np.isfinite(rows)
+    if not finite.any():
+        return 0, 0, 0, 0
+    cols, rows = cols[finite], rows[finite]
+    r_lo = int(np.clip(rows.min() - WINDOW_MARGIN, 0, src_h))
+    r_hi = int(np.clip(rows.max() + 1 + WINDOW_MARGIN, r_lo, src_h))
+    c_lo = int(np.clip(cols.min() - WINDOW_MARGIN, 0, src_w))
+    c_hi = int(np.clip(cols.max() + 1 + WINDOW_MARGIN, c_lo, src_w))
+    return r_lo, r_hi, c_lo, c_hi
+
+
+def _warp_call(src, origin, src_shape, geo_transform, source_projection, no_data_value, bbox,
+               height, width, projection, count_misses):
+    """One gm_warp_nn call from the DeviceArray ``src`` (source cells from ``origin`` = (row, col)
+    on) into a new DeviceArray; returns it with the number of reads outside ``src`` (None when not
+    counted, which saves the stream synchronisation)."""
+    (src_kind, src_zone), (dst_kind, dst_zone) = crs.crs_pair(source_projection, projection)
+    warp = _native.GmWarp()
+    warp.dst_kind, warp.dst_zone, warp.src_kind, warp.src_zone = dst_kind, dst_zone, src_kind, src_zone
+    warp.dst_geo[:] = utils.GeoTransform.from_bbox(bbox, height, width)
+    warp.src_geo[:] = geo_transform
+    warp.src_height, warp.src_width = src_shape
+    warp.win_row0, warp.win_col0 = origin
+    out = _native.DeviceArray((src.shape[0], height, width), src.dtype)
+    nodata_holder, nodata_ptr = _native.scalar_ptr(no_data_value, src.dtype)
+    src_desc, dst_desc = _native.as_gm_array(src), _native.as_gm_array(out)
+    misses = ctypes.c_int64(0)
+    _native.check(_native.lib().gm_warp_nn(
+        ctypes.byref(src_desc), ctypes.byref(dst_desc), nodata_ptr, ctypes.byref(warp),
+        ctypes.byref(misses) if count_misses else None, _native.current_stream()))
+    return out, (misses.value if count_misses else None)
+
+
+def _count_window_miss():
+    _native.STATS["warp_window_misses"] = _native.STATS.get("warp_window_misses", 0) + 1
+
+
+def warp_window(array, bands, geo_transform, no_data_value, bbox, height, width, projection,
+                source_projection, keep_on_device):
+    """Nearest-neighbour warp of ``array[bands[0]:bands[1]]`` (a source in ``source_projection``)
+    into a request grid in ``projection`` (the reference's gdal.ReprojectImage,
+    raster/sources.py:119-149).  Uploads only the window the request reads, or reads the
+    resident copy (``geomodeling.device-cache-bytes``)."""
+    b0, b1 = bands
+    n_bands = b1 - b0
+    _, src_h, src_w = array.shape
+    crs.crs_pair(source_projection, projection)     # unsupported pairs raise before any upload
+    args = (geo_transform, source_projection, no_data_value, bbox, height, width, projection)
+    resident = resident_copy(array) if n_bands > 0 else None
+    if resident is not None:
+        item = array.dtype.itemsize
+        view = _native.DeviceArray((n_bands, src_h, src_w), array.dtype,
+                                   ptr=resident.ptr + b0 * src_h * src_w * item, owner=resident)
+        out, _ = _warp_call(view, (0, 0), (src_h, src_w), *args, count_misses=False)
+    else:
+        window = warp_source_window(geo_transform, bbox, projection, source_projection, src_h, src_w)
+        r_lo, r_hi, c_lo, c_hi = window
+        src = _native.DeviceArray((n_bands, r_hi - r_lo, c_hi - c_lo), array.dtype)
+        upload_window(array, b0, window, src)
+        out, misses = _warp_call(src, (r_lo, c_lo), (src_h, src_w), *args, count_misses=True)
+        if misses:
+            _count_window_miss()
+            src = _native.DeviceArray((n_bands, src_h, src_w), array.dtype)
+            upload_window(array, b0, (0, src_h, 0, src_w), src)
+            out, _ = _warp_call(src, (0, 0), (src_h, src_w), *args, count_misses=False)
+    return out if keep_on_device else out.to_host()
+
+
+def point_cell(geo_transform, src_shape, bbox, projection, source_projection):
+    """Cell of a point request (raster/sources.py:95-117) as (row, col), or None outside the
+    source; the point is first transformed into the source CRS."""
+    point = np.array([[bbox[0], bbox[1]]], dtype=np.float64)
+    if not utils.same_projection(projection, source_projection):
+        point = crs.transform(point, projection, source_projection)
+        if not np.isfinite(point).all():
+            return None
+    rows, cols = geo_transform.get_indices(point)
+    i, j = int(rows[0]), int(cols[0])
+    return (i, j) if 0 <= i < src_shape[0] and 0 <= j < src_shape[1] else None
 
 
 class RasterSourceBase(RasterBlock):
@@ -201,22 +319,21 @@ class RasterSourceBase(RasterBlock):
         if dataset is not None:
             process_kwargs = dict(process_kwargs, source_projection=dataset.projection,
                                   geo_transform=dataset.geo_transform)
-        if not utils.same_projection(process_kwargs["projection"], process_kwargs["source_projection"]):
-            raise NotImplementedError(
-                "raster source: reprojection {} -> {} needs GDAL and is outside the CUDA raster "
-                "path".format(process_kwargs["source_projection"], process_kwargs["projection"])
-            )
+        projection, source_projection = process_kwargs["projection"], process_kwargs["source_projection"]
+        same = utils.same_projection(projection, source_projection)
+        if not same:
+            crs.crs_pair(source_projection, projection)    # NotImplementedError for other CRSs
         geo_transform = utils.GeoTransform(process_kwargs["geo_transform"])
         if dataset is not None:
-            return _file_values(dataset, (b0, b1), geo_transform, dtype, no_data_value, bbox, height, width)
+            return _file_values(dataset, (b0, b1), geo_transform, dtype, no_data_value, bbox, height, width,
+                                projection)
 
         if bbox[0] == bbox[2] or bbox[1] == bbox[3]:
             # point request: the cell that contains the point (raster/sources.py:95-117)
-            rows, cols = geo_transform.get_indices(np.array([[bbox[0], bbox[1]]]))
-            i, j = int(rows[0]), int(cols[0])
+            cell = point_cell(geo_transform, array.shape[1:], bbox, projection, source_projection)
             result = np.full((array.shape[0], 1, 1), no_data_value, dtype=dtype)
-            if 0 <= i < array.shape[1] and 0 <= j < array.shape[2]:
-                result[:, 0, 0] = array[:, i, j]
+            if cell is not None:
+                result[:, 0, 0] = array[:, cell[0], cell[1]]
             result = result[b0:b1]
             if result.dtype.kind == "f":
                 result[~np.isfinite(result)] = no_data_value
@@ -224,6 +341,10 @@ class RasterSourceBase(RasterBlock):
 
         if config.get("geomodeling.pin-sources", True):
             _native.pin(array)
+        if not same:
+            values = warp_window(array, (b0, b1), geo_transform, no_data_value, bbox, height, width,
+                                 projection, source_projection, _state.keep_on_device())
+            return {"values": values, "no_data_value": no_data_value}
         values = resample_window(
             array, (b0, b1), geo_transform, no_data_value, bbox, height, width,
             _state.keep_on_device(),
@@ -246,20 +367,24 @@ def open_dataset(path):
     return hit[1]
 
 
-def _file_values(dataset, bands, geo_transform, dtype, no_data_value, bbox, height, width):
+def _file_values(dataset, bands, geo_transform, dtype, no_data_value, bbox, height, width, projection):
     """'vals' response of a file source: point requests read one cell, other requests inflate the
-    tiles under their window and resample it on the device."""
+    tiles under their window and resample (or, in another projection, warp) it on the device."""
     b0, b1 = bands
     n_all, src_h, src_w = dataset.shape
     if bbox[0] == bbox[2] or bbox[1] == bbox[3]:
-        rows, cols = geo_transform.get_indices(np.array([[bbox[0], bbox[1]]]))
-        i, j = int(rows[0]), int(cols[0])
+        cell = point_cell(geo_transform, (src_h, src_w), bbox, projection, dataset.projection)
         result = np.full((b1 - b0, 1, 1), no_data_value, dtype=dtype)
-        if 0 <= i < src_h and 0 <= j < src_w:
+        if cell is not None:
+            i, j = cell
             result[:, 0, 0] = dataset.read_window(b0, b1, i, i + 1, j, j + 1)[:, 0, 0]
         if result.dtype.kind == "f":
             result[~np.isfinite(result)] = no_data_value
         return {"values": result, "no_data_value": no_data_value}
+    if not utils.same_projection(projection, dataset.projection):
+        return {"values": _file_warp(dataset, bands, geo_transform, dtype, no_data_value, bbox, height,
+                                     width, projection),
+                "no_data_value": no_data_value}
     r_lo, r_hi, c_lo, c_hi = source_window(geo_transform, bbox, height, width, src_h, src_w)
     window = dataset.read_window(b0, b1, r_lo, r_hi, c_lo, c_hi)
     if window.dtype != dtype:
@@ -269,6 +394,32 @@ def _file_values(dataset, bands, geo_transform, dtype, no_data_value, bbox, heig
     values = resample_window(window, (0, b1 - b0), geo_transform, no_data_value, bbox, height, width,
                              _state.keep_on_device(), origin=(r_lo, c_lo))
     return {"values": values, "no_data_value": no_data_value}
+
+
+def _file_warp(dataset, bands, geo_transform, dtype, no_data_value, bbox, height, width, projection):
+    """Warp of a file source into a request in another CRS: the tiles under the estimated window
+    are decoded; when the warp reads outside it, the whole file is."""
+    b0, b1 = bands
+    _, src_h, src_w = dataset.shape
+    args = (geo_transform, dataset.projection, no_data_value, bbox, height, width, projection)
+
+    def decoded(window):
+        r_lo, r_hi, c_lo, c_hi = window
+        host = np.ascontiguousarray(dataset.read_window(b0, b1, r_lo, r_hi, c_lo, c_hi), dtype=dtype)
+        src = _native.DeviceArray((b1 - b0, r_hi - r_lo, c_hi - c_lo), dtype)
+        if src.size:
+            upload_window(host.reshape(src.shape), 0, (0, r_hi - r_lo, 0, c_hi - c_lo), src)
+            _native.synchronize()     # the decoded window is a temporary
+        return src
+
+    window = warp_source_window(geo_transform, bbox, projection, dataset.projection, src_h, src_w)
+    out, misses = _warp_call(decoded(window), (window[0], window[2]), (src_h, src_w), *args,
+                             count_misses=True)
+    if misses:
+        _count_window_miss()
+        out, _ = _warp_call(decoded((0, src_h, 0, src_w)), (0, 0), (src_h, src_w), *args,
+                            count_misses=False)
+    return out if _state.keep_on_device() else out.to_host()
 
 
 class MemorySource(RasterSourceBase):

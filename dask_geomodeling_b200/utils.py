@@ -3,7 +3,8 @@
 Mirrors the names the reference blocks import from ``dask_geomodeling.utils``
 (utils.py; line numbers cited per function).  CRS handling is limited to what
 works without GDAL/pyproj: projections are compared by their normalised
-string, and anything that needs an actual coordinate transformation raises.
+string, coordinates are transformed between EPSG:4326, EPSG:3857 and the WGS 84
+UTM zones (``crs.py``), and every other transformation raises.
 """
 import math
 import os
@@ -127,12 +128,16 @@ class Extent(object):
         self.projection = get_epsg_or_wkt(projection)
 
     def transformed(self, projection):
+        """The bounds of the box's corners transformed into ``projection``.  Only the four
+        corners are transformed; whether the reference densifies the box edges first is not
+        pinned (it transforms the box polygon through GDAL/OGR)."""
         if same_projection(self.projection, projection):
             return Extent(self.bbox, projection)
-        raise NotImplementedError(
-            "coordinate transformation {} -> {} needs pyproj/GDAL, which this build "
-            "does not use".format(self.projection, projection)
-        )
+        from . import crs
+
+        x1, y1, x2, y2 = self.bbox
+        xy = crs.transform([(x2, y1), (x2, y2), (x1, y2), (x1, y1)], self.projection, projection)
+        return Extent((xy[:, 0].min(), xy[:, 1].min(), xy[:, 0].max(), xy[:, 1].max()), projection)
 
     @classmethod
     def from_geometry(cls, geometry, projection=None):
@@ -434,12 +439,33 @@ def shapely_from_wkt(wkt):
     raise WKTReadingError("unsupported geometry type '{}'".format(kind))
 
 
+def _map_coords(geometry, fn):
+    """``geometry`` with every vertex array passed through ``fn`` (N x 2 -> N x 2); the classes
+    above and shapely-like objects (rebuilt as the classes above)."""
+    if geometry is None or getattr(geometry, "is_empty", False):
+        return geometry
+    if hasattr(geometry, "geoms"):
+        return MultiPolygon([_map_coords(part, fn) for part in geometry.geoms])
+    if hasattr(geometry, "exterior"):
+        shell = fn(np.asarray(geometry.exterior.coords, dtype=np.float64)[:, :2])
+        return Polygon(shell, [fn(np.asarray(r.coords, dtype=np.float64)[:, :2]) for r in geometry.interiors])
+    kind = getattr(geometry, "geom_type", type(geometry).__name__)
+    if kind == "Point":
+        x, y = fn(np.array([[float(geometry.x), float(geometry.y)]]))[0]
+        return Point(x, y)
+    raise NotImplementedError("cannot transform geometries of type '{}'".format(kind))
+
+
 def shapely_transform(geometry, src_srs, dst_srs):
+    """``geometry`` with every vertex transformed from ``src_srs`` to ``dst_srs``, as
+    shapely.ops.transform with a pyproj transformer does.  Unsupported CRS pairs raise
+    NotImplementedError (see crs.py)."""
     if same_projection(src_srs, dst_srs):
         return geometry
-    raise NotImplementedError(
-        "coordinate transformation {} -> {} needs pyproj/GDAL".format(src_srs, dst_srs)
-    )
+    from . import crs
+
+    crs.crs_pair(src_srs, dst_srs)
+    return _map_coords(geometry, lambda xy: crs.transform(xy, src_srs, dst_srs))
 
 
 def _ring_moments(c):
@@ -548,6 +574,18 @@ class PolygonSoup(object):
         sub.ring_offsets = np.concatenate([[0], np.cumsum(v_n)]).astype(np.int64)
         sub.poly_offsets = np.concatenate([[0], np.cumsum(ring_n)]).astype(np.int64)
         return sub
+
+    def transformed(self, src_srs, dst_srs):
+        """The soup with every vertex transformed from ``src_srs`` to ``dst_srs`` in one call."""
+        if same_projection(src_srs, dst_srs):
+            return self
+        from . import crs
+
+        out = PolygonSoup([])
+        out.has_points = self.has_points
+        out.xy = np.ascontiguousarray(crs.transform(self.xy, src_srs, dst_srs))
+        out.ring_offsets, out.poly_offsets = self.ring_offsets, self.poly_offsets
+        return out
 
     def bounds(self):
         """(n, 4) array of (xmin, ymin, xmax, ymax) per polygon (NaN for empty ones)."""

@@ -209,6 +209,31 @@ int  gm_resample_nn(const GmArray* src, GmArray* dst, const void* nodata,
                     double col0, double col_step, double row0, double row_step,
                     void* stream);
 
+/* input adaptor across projections: nearest-neighbour warp of a source window into a request
+ * grid in another CRS (raster/sources.py:119-149, the reference's gdal.ReprojectImage).  Target
+ * cell (i, j) takes the value of source cell (floor(row), floor(col)) where (col, row) =
+ * ((x - src_geo[0]) / src_geo[1] + 1e-10, (y - src_geo[3]) / src_geo[5] + 1e-10) and (x, y) is
+ * the centre (dst_geo[0] + (j + 0.5) dst_geo[1], dst_geo[3] + (i + 0.5) dst_geo[5]) transformed
+ * exactly in float64 into the source CRS; no data outside the source, for non-finite source values
+ * and for coordinates the source CRS cannot represent.  CRSs are WGS 84 only: EPSG:4326
+ * (x = lon, y = lat in degrees), EPSG:3857, and UTM (zone +z north / -z south, transverse
+ * Mercator by Krueger's series to sixth order).  `src` holds rows/cols [win_row0, +shape[1]) x
+ * [win_col0, +shape[2]) of the whole (src_height x src_width) source described by src_geo.
+ * Reads of source cells outside that window give no data and are counted: with misses != NULL
+ * (host pointer) the call synchronises `stream` and stores the count, and the caller repeats the
+ * call with a larger window when it is not 0.                                                   */
+enum GmCrsKind { GM_CRS_GEOGRAPHIC = 0, GM_CRS_MERCATOR = 1, GM_CRS_UTM = 2 };
+typedef struct GmWarp {
+  int32_t dst_kind, dst_zone;     /* GmCrsKind; UTM zone (+north / -south), else 0 */
+  int32_t src_kind, src_zone;
+  double  dst_geo[6];             /* geotransform of the request grid              */
+  double  src_geo[6];             /* geotransform of the whole source              */
+  int64_t src_height, src_width;  /* whole source                                  */
+  int64_t win_row0, win_col0;     /* source cell of src[:, 0, 0]                   */
+} GmWarp;
+int  gm_warp_nn(const GmArray* src, GmArray* dst, const void* nodata, const GmWarp* warp,
+                int64_t* misses, void* stream);
+
 /* stencils (raster/spatial.py): src carries the halo the reference requests.  gm_hillshade and
  * gm_moving_max accept rows with extra columns on the right (src.shape[2] >= dst.shape[2] + halo):
  * on a 16-byte row pitch HillShade reads four columns per load and MovingMax stages tiles by TMA */
