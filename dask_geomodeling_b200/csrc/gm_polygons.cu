@@ -9,15 +9,25 @@
 // The fill rule restates GDAL's alg/llrasterize.cpp::GDALdllImageFilledPolygon
 // (see oracle/polyfill.c for the CPU restatement it is tested against): vertices in
 // pixel space through the inverse geotransform, scanline at y + 0.5, crossing
-// x = floor(intersect + 0.5), even-odd pairs over all rings of a feature.
-//
-// One thread block owns one polygon; its warps take scanlines round-robin.  A warp
-// finds the crossings of its scanline with a ballot-compacted edge loop, sorts them
-// in shared memory and then walks the spans cooperatively, so that raster reads are
-// coalesced 128-byte segments.  Zonal statistics read the raster directly under the
-// spans -- no label raster is ever materialised -- and order statistics are selected
-// by an MSD radix select over the polygon's values held in shared memory (global
-// scratch for polygons that do not fit).
+// x = floor(intersect + 0.5), even-odd pairs over all rings of a feature, bottom
+// horizontal edges filled on their own.  The per-edge part of the rule is written once,
+// in edge_crossing; rows reach it through one of two routines:
+//   generic_scanline  the whole warp on one row, any number of vertices and crossings
+//   row_crossings     lane per row, for polygons of <= ZW_MAXV vertices staged in shared
+//                     memory; a row it cannot describe (a bottom horizontal edge, more
+//                     than ZW_MAXC crossings) goes to generic_scanline
+// Zonal statistics read the raster directly under the spans; no label raster is ever
+// materialised.  Which kernel takes which polygon:
+//   - count / sum / mean / min / max: zonal_reduce_warp_kernel, one warp per polygon, for
+//     polygons of <= ZW_MAXV vertices, <= ZW_BIG_ROWS rows and a bounding box of <= ZW_BIG_CELLS
+//     cells; the rest is deferred to zonal_reduce_kernel, one block per polygon (scan_polygon).
+//   - median / percentile of float32 and integer rasters up to 4 bytes without thresholds: the
+//     streaming select, one warp per polygon in three kernels (bracket, main, final) under the
+//     same limits; the polygons it defers, and every other raster, go to zonal_select_kernel,
+//     one block per polygon with an MSD radix select over the polygon's values.
+//   - rasterize: rasterize_tile_kernel, one block per tile of the output, one warp per polygon.
+//   - stripes of the multi-GPU path: the reduce kernels above, or zonal_values_kernel for the
+//     values that segment_select_kernel selects from.
 #include "gm_common.cuh"
 #include <cfloat>
 #include <cstdlib>
@@ -34,8 +44,8 @@ constexpr int PG_WARPS = PG_THREADS / 32;
 constexpr int PG_MAX_CROSSINGS = 4096;        // per scanline
 constexpr int PG_MAX_HSPANS = 8;
 constexpr int SEL_THREADS = 256;
-constexpr int PG_FAST_MAXV = 64;             // vertices of a polygon handled lane-per-scanline
-constexpr int PG_FAST_MAXC = 8;              // crossings per scanline on that path
+constexpr int ZW_MAXV = 64;                  // vertices of a polygon handled lane-per-scanline
+constexpr int ZW_MAXC = 8;                   // crossings per scanline on that path
 constexpr int PG_FAST_WARPS = SEL_THREADS / 32;
 constexpr int PG_BATCH = 4;                 // single-span rows handed to a visitor at once
 
@@ -177,6 +187,38 @@ __device__ __forceinline__ void span_batch(GatherVisitor<T>& vis, int n, const i
 template <typename T>
 __device__ __forceinline__ void span_batch(ReduceVisitor<T>& vis, int n, const int* ys, const int* x0, const int* x1);
 
+// The fill rule of GDALdllImageFilledPolygon for ONE edge, from vertex i1 (its predecessor on
+// the ring) to vertex i2, against the scanline at dy = y + 0.5.  Every path that converts
+// polygons to rows decides through this function.  Returns
+//   EDGE_CROSS   the edge crosses the scanline at column *x = floor(intersect + 0.5)
+//   EDGE_BOTTOM  the edge is a bottom horizontal edge on the scanline, columns [*x, *x2),
+//                which GDAL fills on its own (not part of the even-odd pairs)
+//   EDGE_NONE    neither
+enum { EDGE_NONE = 0, EDGE_CROSS = 1, EDGE_BOTTOM = 2 };
+template <typename I>
+__device__ __forceinline__ int edge_crossing(const double* px, const double* py, I i1, I i2, double dy,
+                                             int* x, int* x2) {
+  double dy1 = py[i1], dy2 = py[i2];
+  if ((dy1 < dy && dy2 < dy) || (dy1 > dy && dy2 > dy)) return EDGE_NONE;
+  double dx1, dx2;
+  if (dy1 < dy2) {
+    dx1 = px[i1]; dx2 = px[i2];
+  } else if (dy1 > dy2) {
+    const double t = dy1; dy1 = dy2; dy2 = t;
+    dx2 = px[i1]; dx1 = px[i2];
+  } else {
+    const double xa = px[i1], xb = px[i2];
+    if (!(xa > xb)) return EDGE_NONE;
+    *x = clamp_to_int(floor(xb + 0.5));
+    *x2 = clamp_to_int(floor(xa + 0.5));
+    return EDGE_BOTTOM;
+  }
+  if (!(dy < dy2 && dy >= dy1)) return EDGE_NONE;
+  const double intersect = (dy - dy1) * (dx2 - dx1) / (dy2 - dy1) + dx1;
+  *x = clamp_to_int(floor(intersect + 0.5));
+  return EDGE_CROSS;
+}
+
 // Visitor interface (all calls are warp-uniform):
 //   span(y, x0, x1)                       regular even-odd span, inclusive, clipped
 //   hspan(y, x0, x1, buf, count)          bottom horizontal edge on the scanline
@@ -195,35 +237,11 @@ __device__ __forceinline__ void generic_scanline(const PolyDev& P, int64_t r0, i
     for (int64_t base = a; base < b; base += 32) {
       const int64_t i = base + lane;
       bool cross = false, hs = false;
-      int xi = 0, hx1 = 0, hx2 = 0;
+      int xi = 0, hx2 = 0;      // the crossing, or the bottom horizontal edge [xi, hx2)
       if (i < b) {
-        const int64_t ind1 = (i == a) ? b - 1 : i - 1;
-        double dy1 = P.py[ind1], dy2 = P.py[i];
-        if (!((dy1 < dy && dy2 < dy) || (dy1 > dy && dy2 > dy))) {
-          double dx1, dx2;
-          if (dy1 < dy2) {
-            dx1 = P.px[ind1]; dx2 = P.px[i];
-            cross = true;
-          } else if (dy1 > dy2) {
-            const double t = dy1; dy1 = dy2; dy2 = t;
-            dx2 = P.px[ind1]; dx1 = P.px[i];
-            cross = true;
-          } else {
-            const double xa = P.px[ind1], xb = P.px[i];
-            if (xa > xb) {  // bottom horizontal edge: filled on its own
-              hx1 = clamp_to_int(floor(xb + 0.5));
-              hx2 = clamp_to_int(floor(xa + 0.5));
-              hs = !(hx1 > maxx || hx2 <= 0);
-            }
-          }
-          if (cross) {
-            cross = (dy < dy2 && dy >= dy1);
-            if (cross) {
-              const double intersect = (dy - dy1) * (dx2 - dx1) / (dy2 - dy1) + dx1;
-              xi = clamp_to_int(floor(intersect + 0.5));
-            }
-          }
-        }
+        const int e = edge_crossing(P.px, P.py, (i == a) ? b - 1 : i - 1, i, dy, &xi, &hx2);
+        cross = e == EDGE_CROSS;
+        hs = e == EDGE_BOTTOM && !(xi > maxx || hx2 <= 0);
       }
       const unsigned cm = __ballot_sync(0xffffffffu, cross);
       if (cross) {
@@ -234,7 +252,7 @@ __device__ __forceinline__ void generic_scanline(const PolyDev& P, int64_t r0, i
       const unsigned hm = __ballot_sync(0xffffffffu, hs);
       if (hs) {
         const int pos = hcount + __popc(hm & ((1u << lane) - 1u));
-        if (pos < PG_MAX_HSPANS) { hbuf[2 * pos] = hx1; hbuf[2 * pos + 1] = hx2; }
+        if (pos < PG_MAX_HSPANS) { hbuf[2 * pos] = xi; hbuf[2 * pos + 1] = hx2; }
       }
       hcount += __popc(hm);
     }
@@ -261,6 +279,75 @@ __device__ __forceinline__ void generic_scanline(const PolyDev& P, int64_t r0, i
   __syncwarp();
 }
 
+// Lane per scanline, for polygons of at most ZW_MAXV vertices staged in shared memory: vertex i
+// at (px[i], py[i]), its predecessor on its ring at prev[i].
+//
+// Vertex v0 + i of the polygon made of rings r0..r1 and its ring predecessor to shared memory;
+// returns the vertex' x.
+__device__ __forceinline__ double stage_vertex(const PolyDev& P, int64_t r0, int64_t r1, int64_t v0, int i,
+                                               double* px, double* py, int* prev) {
+  const double x = P.px[v0 + i];
+  px[i] = x; py[i] = P.py[v0 + i];
+  int pr = i - 1;
+  for (int64_t r = r0; r < r1; ++r)
+    if ((int64_t)i + v0 == P.ring_offsets[r]) pr = (int)(P.ring_offsets[r + 1] - v0) - 1;
+  prev[i] = pr;
+  return x;
+}
+
+// the nv vertices of a polygon to the warp's shared memory; returns the width of the bounding
+// box clipped to the raster, fmin(xmax, width) - fmax(xmin, 0) (negative when it misses)
+__device__ __forceinline__ double stage_polygon(const PolyDev& P, int64_t r0, int64_t r1, int64_t v0, int nv,
+                                                double* px, double* py, int* prev, int lane) {
+  double xmin = DBL_MAX, xmax = -DBL_MAX;
+  __syncwarp();
+  for (int i = lane; i < nv; i += 32) {
+    const double x = stage_vertex(P, r0, r1, v0, i, px, py, prev);
+    xmin = fmin(xmin, x); xmax = fmax(xmax, x);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    xmin = fmin(xmin, __shfl_xor_sync(0xffffffffu, xmin, o));
+    xmax = fmax(xmax, __shfl_xor_sync(0xffffffffu, xmax, o));
+  }
+  __syncwarp();
+  return fmin(xmax, (double)P.width) - fmax(xmin, 0.0);
+}
+
+// sorted crossings of row y with the staged polygon into column `lane` of `cross`; returns their
+// number, or -1 for a row that needs the generic scanline (a bottom horizontal edge on the
+// scanline, more than ZW_MAXC crossings).  Inlined into the reduce kernels; the select and
+// rasterize kernels call row_crossings_call.
+__device__ __forceinline__ int row_crossings(const double* px, const double* py, const int* prev, int nv,
+                                             int y, int (*cross)[32], int lane) {
+  const double dy = y + 0.5;
+  int cnt = 0;
+  bool complex_row = false;
+  for (int i = 0; i < nv; ++i) {
+    int x = 0, x2 = 0;
+    const int e = edge_crossing(px, py, prev[i], i, dy, &x, &x2);
+    if (e == EDGE_BOTTOM) complex_row = true;
+    if (e == EDGE_CROSS) {
+      if (cnt < ZW_MAXC) cross[cnt][lane] = x;
+      ++cnt;
+    }
+  }
+  if (cnt > ZW_MAXC || complex_row) return -1;
+  for (int a = 1; a < cnt; ++a) {  // insertion sort of this lane's column
+    const int v = cross[a][lane];
+    int j = a - 1;
+    while (j >= 0 && cross[j][lane] > v) { cross[j + 1][lane] = cross[j][lane]; --j; }
+    cross[j + 1][lane] = v;
+  }
+  return cnt;
+}
+
+// Not inlined: the select kernels have to stay small enough for the instruction cache (32 warps
+// per SM in different phases).
+__device__ __noinline__ int row_crossings_call(const double* px, const double* py, const int* prev, int nv,
+                                               int y, int (*cross)[32], int lane) {
+  return row_crossings(px, py, prev, nv, y, cross, lane);
+}
+
 template <class Visitor>
 __device__ __forceinline__ void scan_polygon(const PolyDev& P, int64_t p, int* buf, int* hbuf,
                                              Visitor& vis) {
@@ -281,66 +368,28 @@ __device__ __forceinline__ void scan_polygon(const PolyDev& P, int64_t p, int* b
   auto generic_row = [&](int y) { generic_scanline(P, r0, r1, y, P.cap, buf, hbuf, vis); };
 
   const int nv = (int)(v1 - v0);
-  if (nv > PG_FAST_MAXV) {
+  if (nv > ZW_MAXV) {
     for (int y = miny + warp; y <= maxy; y += nwarps) generic_row(y);
     return;
   }
 
-  // Small polygons (<= PG_FAST_MAXV vertices, the usual case): the vertices are staged in
+  // Small polygons (<= ZW_MAXV vertices, the usual case): the vertices are staged in
   // shared memory once, then each warp takes 32 scanlines at a time -- lane = scanline --
   // so the edge tests of 32 rows run in parallel instead of one row per warp; the
-  // crossings (same arithmetic as generic_row) are sorted per lane in shared memory and
-  // the spans are then walked by the whole warp row by row (coalesced raster reads).
-  // Rows with more than PG_FAST_MAXC crossings or a horizontal bottom edge fall back to
-  // generic_row.
-  __shared__ double s_px[PG_FAST_MAXV], s_py[PG_FAST_MAXV];
-  __shared__ int s_prev[PG_FAST_MAXV];
-  __shared__ int s_cross[PG_FAST_WARPS][PG_FAST_MAXC][32];
+  // crossings are sorted per lane in shared memory and the spans are then walked by the
+  // whole warp row by row (coalesced raster reads).  Rows with more than ZW_MAXC crossings
+  // or a horizontal bottom edge fall back to generic_row.
+  __shared__ double s_px[ZW_MAXV], s_py[ZW_MAXV];
+  __shared__ int s_prev[ZW_MAXV];
+  __shared__ int s_cross[PG_FAST_WARPS][ZW_MAXC][32];
   __syncthreads();
-  for (int i = threadIdx.x; i < nv; i += blockDim.x) {
-    s_px[i] = P.px[v0 + i];
-    s_py[i] = P.py[v0 + i];
-    int prev = i - 1;
-    for (int64_t r = r0; r < r1; ++r)
-      if ((int64_t)i + v0 == P.ring_offsets[r]) prev = (int)(P.ring_offsets[r + 1] - v0) - 1;
-    s_prev[i] = prev;
-  }
+  for (int i = threadIdx.x; i < nv; i += blockDim.x) stage_vertex(P, r0, r1, v0, i, s_px, s_py, s_prev);
   __syncthreads();
   for (int base = miny + 32 * warp; base <= maxy; base += 32 * nwarps) {
     const int y = base + lane;
-    const double dy = y + 0.5;
     int cnt = 0;
-    bool complex_row = false;
-    if (y <= maxy) {
-      for (int i = 0; i < nv; ++i) {
-        const int ind1 = s_prev[i];
-        double dy1 = s_py[ind1], dy2 = s_py[i];
-        if ((dy1 < dy && dy2 < dy) || (dy1 > dy && dy2 > dy)) continue;
-        double dx1, dx2;
-        if (dy1 < dy2) {
-          dx1 = s_px[ind1]; dx2 = s_px[i];
-        } else if (dy1 > dy2) {
-          const double t = dy1; dy1 = dy2; dy2 = t;
-          dx2 = s_px[ind1]; dx1 = s_px[i];
-        } else {
-          if (s_px[ind1] > s_px[i]) complex_row = true;  // bottom horizontal edge on the scanline
-          continue;
-        }
-        if (dy < dy2 && dy >= dy1) {
-          const double intersect = (dy - dy1) * (dx2 - dx1) / (dy2 - dy1) + dx1;
-          if (cnt < PG_FAST_MAXC) s_cross[warp][cnt][lane] = clamp_to_int(floor(intersect + 0.5));
-          ++cnt;
-        }
-      }
-      if (cnt > PG_FAST_MAXC) complex_row = true;
-      if (!complex_row)
-        for (int a = 1; a < cnt; ++a) {  // insertion sort of this lane's column
-          const int v = s_cross[warp][a][lane];
-          int j = a - 1;
-          while (j >= 0 && s_cross[warp][j][lane] > v) { s_cross[warp][j + 1][lane] = s_cross[warp][j][lane]; --j; }
-          s_cross[warp][j + 1][lane] = v;
-        }
-    }
+    if (y <= maxy) cnt = row_crossings(s_px, s_py, s_prev, nv, y, s_cross[warp], lane);
+    const bool complex_row = cnt < 0;
     __syncwarp();
     const unsigned complex_mask = __ballot_sync(0xffffffffu, complex_row);
     const int n_rows = min(32, maxy - base + 1);
@@ -461,6 +510,11 @@ struct ActiveTest {
     return true;
   }
 };
+// the test for polygon p (thresholds: one per polygon, or nullptr)
+template <typename T>
+__device__ __forceinline__ ActiveTest<T> active_test(T nodata, int has_nodata, const float* thresholds, int64_t p) {
+  return ActiveTest<T>{nodata, has_nodata, thresholds != nullptr, thresholds ? thresholds[p] : 0.0f};
+}
 
 // min / max are tracked in the raster dtype (one FMNMX / IMNMX per value; NaN never wins,
 // as with the `d < vmin` form) and the count in 32 bits per lane; only the sum needs the
@@ -560,9 +614,7 @@ zonal_reduce_kernel(const PolyDev P, const T* __restrict__ raster, T nodata, int
     const int64_t p = work[2 + item];
     ReduceVisitor<T> vis;
     vis.raster = raster; vis.width = P.width;
-    vis.active.nodata = nodata; vis.active.has_nodata = has_nodata;
-    vis.active.has_threshold = thresholds != nullptr;
-    vis.active.threshold = thresholds ? thresholds[p] : 0.0f;
+    vis.active = active_test(nodata, has_nodata, thresholds, p);
     vis.reset();
     scan_polygon(P, p, buf, hbuf, vis);
     long long count = vis.count;
@@ -601,8 +653,6 @@ zonal_reduce_kernel(const PolyDev P, const T* __restrict__ raster, T nodata, int
 // one unsigned compare.  Everything else (many vertices, many rows, wide boxes) is appended to
 // a list that zonal_reduce_kernel (one block per polygon) works off afterwards.
 constexpr int ZW_WARPS = 8;
-constexpr int ZW_MAXV = PG_FAST_MAXV;
-constexpr int ZW_MAXC = PG_FAST_MAXC;
 constexpr int ZW_ROWS = 4;
 constexpr int ZW_MIN_BLOCKS = 4;
 constexpr int ZW_BIG_ROWS = 256;
@@ -759,6 +809,59 @@ struct WarpReduce {
   }
 };
 
+// The row table of the batched walk (WarpReduce / WarpSelect issue + consume) for the 32 rows
+// base + lane, one per lane, from their crossings (row_crossings: cnt of them in column `lane` of
+// `cross`, -1 for a row that needs the generic scanline).  A row that is one span gets its span
+// [x0, xe) clipped to the raster and its part [xh, xt) made of whole quads of VEC cells aligned to
+// 16 bytes, in lines 0..3 of `cross`; its cells are added to `cells`.  Rows of more spans, and
+// rows on the raster's first / last line when a quad could reach outside the array
+// (edge_scalar), are handed to scalar.span(y, x0, x1) span by span first, while their raw
+// crossings are still there.  Returns the ballot of the generic-scanline rows; *single = the
+// ballot of the rows in the table.
+template <int VEC, class Scalar>
+__device__ __forceinline__ unsigned row_table(const PolyDev& P, int mis, int edge_scalar, int base, int cnt,
+                                              int (*cross)[32], long long& cells, unsigned* single,
+                                              Scalar& scalar) {
+  const int lane = threadIdx.x & 31;
+  const int maxx = P.width - 1;
+  const int y = base + lane;
+  const bool complex_row = cnt < 0;
+  const bool edge = edge_scalar && (y == 0 || y == P.height - 1);
+  const bool scalar_row = !complex_row && cnt >= 2 && (cnt > 2 || edge);
+  int fx0 = 0, fxe = 0, xh = 0, xt = 0;
+  if (!complex_row && !scalar_row && cnt == 2) {
+    const int xa = cross[0][lane], xb = cross[1][lane];
+    if (xa <= maxx && xb > 0 && (xa < 0 ? 0 : xa) < (xb > P.width ? P.width : xb)) {
+      fx0 = xa < 0 ? 0 : xa; fxe = xb > P.width ? P.width : xb;
+      cells += fxe - fx0;
+      const int64_t off = (int64_t)y * P.width + mis;      // element offset from the 16-byte grid
+      xh = fx0 + (int)((VEC - ((off + fx0) & (VEC - 1))) & (VEC - 1));
+      xt = fxe - (int)((off + fxe) & (VEC - 1));
+      if (xt < xh) xt = xh;
+    }
+  }
+  __syncwarp();
+  const unsigned complex_mask = __ballot_sync(0xffffffffu, complex_row);
+  unsigned scalar_mask = __ballot_sync(0xffffffffu, scalar_row);
+  *single = __ballot_sync(0xffffffffu, fx0 < fxe);
+  while (scalar_mask) {
+    const int r = __ffs(scalar_mask) - 1;
+    scalar_mask &= scalar_mask - 1;
+    const int c = __shfl_sync(0xffffffffu, cnt, r);
+    for (int i = 0; i + 1 < c; i += 2) {
+      const int xa = cross[i][r], xb = cross[i + 1][r];
+      if (xa <= maxx && xb > 0) {
+        const int x0 = xa < 0 ? 0 : xa, x1 = xb - 1 > maxx ? maxx : xb - 1;
+        if (x0 <= x1) scalar.span(base + r, x0, x1);
+      }
+    }
+  }
+  __syncwarp();
+  cross[0][lane] = fx0; cross[1][lane] = fxe; cross[2][lane] = xh; cross[3][lane] = xt;
+  __syncwarp();
+  return complex_mask;
+}
+
 template <typename T, int NEED>
 __global__ void __launch_bounds__(32 * ZW_WARPS, ZW_MIN_BLOCKS)
 zonal_reduce_warp_kernel(const PolyDev P, const T* __restrict__ raster, T nodata, int has_nodata,
@@ -779,8 +882,6 @@ zonal_reduce_warp_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
   int* hbuf = buf + ZW_MAXV;
   WarpReduce<T, NEED> vis;
   vis.raster = raster; vis.width = P.width;
-  vis.active.nodata = nodata; vis.active.has_nodata = has_nodata;
-  vis.active.has_threshold = thresholds != nullptr;
   const bool f32_fast = std::is_same<T, float>::value && has_nodata && thresholds == nullptr;
   // (with an active list the partials of the other polygons were cleared by the caller)
   const int64_t n_work = P.active ? (int64_t)*P.n_active : P.n_polygons;
@@ -798,29 +899,12 @@ zonal_reduce_warp_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
     int64_t v0 = 0, v1 = 0;
     if (r1 > r0) { v0 = P.ring_offsets[r0]; v1 = P.ring_offsets[r1]; }
     const int nv = (int)min((int64_t)(ZW_MAXV + 1), v1 - v0);
-    vis.active.threshold = thresholds ? thresholds[p] : 0.0f;
+    vis.active = active_test(nodata, has_nodata, thresholds, p);
     vis.reset();
     bool defer = nv > ZW_MAXV || maxy - miny >= ZW_BIG_ROWS;
     if (!defer && nv > 1 && miny <= maxy) {
-      // vertices (and each vertex' predecessor on its ring) to this warp's shared memory
-      double xmin = DBL_MAX, xmax = -DBL_MAX;
-      __syncwarp();
-      for (int i = lane; i < nv; i += 32) {
-        const double x = P.px[v0 + i];
-        px[i] = x; py[i] = P.py[v0 + i];
-        xmin = fmin(xmin, x); xmax = fmax(xmax, x);
-        int pr = i - 1;
-        for (int64_t r = r0; r < r1; ++r)
-          if ((int64_t)i + v0 == P.ring_offsets[r]) pr = (int)(P.ring_offsets[r + 1] - v0) - 1;
-        prev[i] = pr;
-      }
-      for (int o = 16; o > 0; o >>= 1) {
-        xmin = fmin(xmin, __shfl_xor_sync(0xffffffffu, xmin, o));
-        xmax = fmax(xmax, __shfl_xor_sync(0xffffffffu, xmax, o));
-      }
-      const double wide = fmin(xmax, (double)P.width) - fmax(xmin, 0.0);
+      const double wide = stage_polygon(P, r0, r1, v0, nv, px, py, prev, lane);
       defer = wide * (double)(maxy - miny + 1) > (double)ZW_BIG_CELLS;
-      __syncwarp();
     }
     if (defer) {
       if (lane == 0) work[2 + atomicAdd(work, 1)] = (int)p;
@@ -834,81 +918,11 @@ zonal_reduce_warp_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
     } else if (nv > 1) {
       for (int base = miny; base <= maxy; base += 32) {
         const int y = base + lane;
-        const double dy = y + 0.5;
         int cnt = 0;
-        bool complex_row = false;
-        if (y <= maxy) {
-          for (int i = 0; i < nv; ++i) {
-            const int ind1 = prev[i];
-            double dy1 = py[ind1], dy2 = py[i];
-            if ((dy1 < dy && dy2 < dy) || (dy1 > dy && dy2 > dy)) continue;
-            double dx1, dx2;
-            if (dy1 < dy2) {
-              dx1 = px[ind1]; dx2 = px[i];
-            } else if (dy1 > dy2) {
-              const double t = dy1; dy1 = dy2; dy2 = t;
-              dx2 = px[ind1]; dx1 = px[i];
-            } else {
-              if (px[ind1] > px[i]) complex_row = true;  // bottom horizontal edge on the scanline
-              continue;
-            }
-            if (dy < dy2 && dy >= dy1) {
-              const double intersect = (dy - dy1) * (dx2 - dx1) / (dy2 - dy1) + dx1;
-              if (cnt < ZW_MAXC) s_cross[warp][cnt][lane] = clamp_to_int(floor(intersect + 0.5));
-              ++cnt;
-            }
-          }
-          if (cnt > ZW_MAXC) complex_row = true;
-          if (!complex_row)
-            for (int a = 1; a < cnt; ++a) {  // insertion sort of this lane's column
-              const int v = s_cross[warp][a][lane];
-              int j = a - 1;
-              while (j >= 0 && s_cross[warp][j][lane] > v) { s_cross[warp][j + 1][lane] = s_cross[warp][j][lane]; --j; }
-              s_cross[warp][j + 1][lane] = v;
-            }
-        }
-        // The row table of the batched walk: first span of the row [fx0, fxe) clipped to the
-        // raster, and its part [xh, xt) made of whole quads aligned to 16 bytes.  Rows with
-        // more spans, or on the raster's first / last line when a quad could reach outside
-        // the array, are walked span by span with scalar loads.
-        const bool edge = edge_scalar && (y == 0 || y == P.height - 1);
-        const bool scalar_row = !complex_row && cnt >= 2 && (cnt > 2 || edge);
-        int fx0 = 0, fxe = 0, xh = 0, xt = 0;
-        if (!complex_row && !scalar_row && cnt == 2) {
-          constexpr int VEC = WarpReduce<T, NEED>::VEC;
-          const int xa = s_cross[warp][0][lane], xb = s_cross[warp][1][lane];
-          if (xa <= maxx && xb > 0 && (xa < 0 ? 0 : xa) < (xb > P.width ? P.width : xb)) {
-            fx0 = xa < 0 ? 0 : xa; fxe = xb > P.width ? P.width : xb;
-            vis.cells += fxe - fx0;
-            const int64_t off = (int64_t)y * P.width + mis;      // element offset from the 16-byte grid
-            xh = fx0 + (int)((VEC - ((off + fx0) & (VEC - 1))) & (VEC - 1));
-            xt = fxe - (int)((off + fxe) & (VEC - 1));
-            if (xt < xh) xt = xh;
-          }
-        }
-        __syncwarp();
-        const unsigned complex_mask = __ballot_sync(0xffffffffu, complex_row);
-        unsigned scalar_mask = __ballot_sync(0xffffffffu, scalar_row);
-        const unsigned single_mask = __ballot_sync(0xffffffffu, fx0 < fxe);
-        // the scalar rows first: they still need their raw crossings
-        while (scalar_mask) {
-          const int r = __ffs(scalar_mask) - 1;
-          scalar_mask &= scalar_mask - 1;
-          const int c = __shfl_sync(0xffffffffu, cnt, r);
-          for (int i = 0; i + 1 < c; i += 2) {
-            const int xa = s_cross[warp][i][r], xb = s_cross[warp][i + 1][r];
-            if (xa <= maxx && xb > 0) {
-              const int x0 = xa < 0 ? 0 : xa, x1 = xb - 1 > maxx ? maxx : xb - 1;
-              if (x0 <= x1) vis.span(base + r, x0, x1);
-            }
-          }
-        }
-        __syncwarp();
-        s_cross[warp][0][lane] = fx0;
-        s_cross[warp][1][lane] = fxe;
-        s_cross[warp][2][lane] = xh;
-        s_cross[warp][3][lane] = xt;
-        __syncwarp();
+        if (y <= maxy) cnt = row_crossings(px, py, prev, nv, y, s_cross[warp], lane);
+        unsigned single_mask;
+        const unsigned complex_mask = row_table<WarpReduce<T, NEED>::VEC>(
+            P, mis, edge_scalar, base, cnt, s_cross[warp], vis.cells, &single_mask, vis);
         {
           typename WarpReduce<T, NEED>::Batch A;
           const int* tab = &s_cross[warp][0][0];
@@ -1170,6 +1184,20 @@ template <typename T> __device__ __forceinline__ float percentile_of(T lo, T hi,
   return (float)((double)lo + part * (double)diff);
 }
 
+// the 0-based ranks lo <= hi among n values that the median / q-th percentile combines, and
+// the percentile's weight of the upper one (scipy's median; measurements.percentile)
+__device__ __forceinline__ void order_ranks(int stat, double q, int n, long long* lo, long long* hi, double* part) {
+  *part = 0.0;
+  if (stat == GM_STAT_MEDIAN) {
+    *lo = (n - 1) / 2; *hi = n / 2;
+  } else {
+    const double frac = (double)(n - 1) * (q / 100.0);
+    *lo = (long long)floor(frac);
+    *hi = (long long)ceil(frac);
+    *part = frac - floor(frac);
+  }
+}
+
 // median / percentile of the n keys in `keys` in the reference's arithmetic (block-wide
 // call; `keys` is consumed)
 template <typename T>
@@ -1179,15 +1207,8 @@ __device__ float order_statistic(typename KeyOf<T>::type* keys, int n, int stat,
   float result = __int_as_float(0x7fc00000);
   if (n > 0) {
     long long lo_rank, hi_rank;
-    double part = 0.0;
-    if (stat == GM_STAT_MEDIAN) {
-      lo_rank = (n - 1) / 2; hi_rank = n / 2;
-    } else {
-      const double frac = (double)(n - 1) * (q / 100.0);
-      lo_rank = (long long)floor(frac);
-      hi_rank = (long long)ceil(frac);
-      part = frac - floor(frac);
-    }
+    double part;
+    order_ranks(stat, q, n, &lo_rank, &hi_rank, &part);
     K klo, khi;
     block_select2<K>(keys, n, lo_rank, hi_rank, &klo, &khi, hist, scratch);
     const T lo = KeyOf<T>::value(klo), hi = KeyOf<T>::value(khi);
@@ -1227,9 +1248,7 @@ zonal_select_kernel(const PolyDev P, const T* __restrict__ raster, T nodata, int
     __syncthreads();
     GatherVisitor<T> vis;
     vis.raster = raster; vis.width = P.width;
-    vis.active.nodata = nodata; vis.active.has_nodata = has_nodata;
-    vis.active.has_threshold = thresholds != nullptr;
-    vis.active.threshold = thresholds ? thresholds[p] : 0.0f;
+    vis.active = active_test(nodata, has_nodata, thresholds, p);
     vis.keys = keys; vis.cursor = &cursor; vis.capacity = a;
     scan_polygon(P, p, buf, hbuf, vis);
     __threadfence_block();
@@ -1606,44 +1625,6 @@ __device__ __noinline__ void select_complex_row(const PolyDev& P, int64_t r0, in
   generic_scanline(P, r0, r1, y, ZW_MAXV, buf, hbuf, vis);
 }
 
-// sorted crossings of row y with the polygon staged in (px, py, prev) into column `lane` of
-// `cross`; returns their number, or -1 for a row that needs the generic scanline (a horizontal
-// bottom edge on the scanline, more than ZW_MAXC crossings).  Same arithmetic as generic_scanline.
-__device__ __noinline__ int row_crossings(const double* px, const double* py, const int* prev, int nv,
-                                          int y, int (*cross)[32], int lane) {
-  const double dy = y + 0.5;
-  int cnt = 0;
-  bool complex_row = false;
-  for (int i = 0; i < nv; ++i) {
-    const int ind1 = prev[i];
-    double dy1 = py[ind1], dy2 = py[i];
-    if ((dy1 < dy && dy2 < dy) || (dy1 > dy && dy2 > dy)) continue;
-    double dx1, dx2;
-    if (dy1 < dy2) {
-      dx1 = px[ind1]; dx2 = px[i];
-    } else if (dy1 > dy2) {
-      const double t = dy1; dy1 = dy2; dy2 = t;
-      dx2 = px[ind1]; dx1 = px[i];
-    } else {
-      if (px[ind1] > px[i]) complex_row = true;
-      continue;
-    }
-    if (dy < dy2 && dy >= dy1) {
-      const double intersect = (dy - dy1) * (dx2 - dx1) / (dy2 - dy1) + dx1;
-      if (cnt < ZW_MAXC) cross[cnt][lane] = clamp_to_int(floor(intersect + 0.5));
-      ++cnt;
-    }
-  }
-  if (cnt > ZW_MAXC || complex_row) return -1;
-  for (int a = 1; a < cnt; ++a) {
-    const int v = cross[a][lane];
-    int j = a - 1;
-    while (j >= 0 && cross[j][lane] > v) { cross[j + 1][lane] = cross[j][lane]; --j; }
-    cross[j + 1][lane] = v;
-  }
-  return cnt;
-}
-
 // The select runs as THREE kernels, each a loop of warps over polygons (atomic counter) that
 // executes ONE phase: with all phases in a single kernel the 32 warps of an SM sat in different
 // parts of ~100 KB of code and 40-55 % of the issue slots were lost to instruction-cache misses
@@ -1658,29 +1639,6 @@ __device__ __noinline__ int row_crossings(const double* px, const double* py, co
 enum { WS_SKIP = 0, WS_TABLE = 1, WS_EXACT = 2 };
 struct SelectState { unsigned lo, hi; int what; int n_active; int below; int kept; };
 constexpr int WS_TABLE_WORDS = WS_CAP * 32 + 32;     // cells + per-lane counts
-
-// vertices of polygon p (and each vertex' predecessor on its ring) to the warp's shared memory;
-// returns the width of the bounding box clipped to the raster (+ 1)
-__device__ __forceinline__ double stage_polygon(const PolyDev& P, int64_t r0, int64_t r1, int64_t v0, int nv,
-                                                double* px, double* py, int* prev, int lane) {
-  double xmin = DBL_MAX, xmax = -DBL_MAX;
-  __syncwarp();
-  for (int i = lane; i < nv; i += 32) {
-    const double x = P.px[v0 + i];
-    px[i] = x; py[i] = P.py[v0 + i];
-    xmin = fmin(xmin, x); xmax = fmax(xmax, x);
-    int pr = i - 1;
-    for (int64_t r = r0; r < r1; ++r)
-      if ((int64_t)i + v0 == P.ring_offsets[r]) pr = (int)(P.ring_offsets[r + 1] - v0) - 1;
-    prev[i] = pr;
-  }
-  for (int o = 16; o > 0; o >>= 1) {
-    xmin = fmin(xmin, __shfl_xor_sync(0xffffffffu, xmin, o));
-    xmax = fmax(xmax, __shfl_xor_sync(0xffffffffu, xmax, o));
-  }
-  __syncwarp();
-  return fmax(fmin(xmax, (double)P.width) - fmax(xmin, 0.0), 0.0) + 1.0;
-}
 
 #define WS_SHARED_TABLES                                                              \
   __shared__ double s_px[WS_WARPS][ZW_MAXV], s_py[WS_WARPS][ZW_MAXV];                 \
@@ -1733,7 +1691,7 @@ zonal_select_bracket_kernel(const PolyDev P, const T* __restrict__ raster, T nod
     bool defer = nv > ZW_MAXV || nv < 2 || nrows > ZW_BIG_ROWS;
     double boxw = 0.0;
     if (!defer) {
-      boxw = stage_polygon(P, r0, r1, v0, nv, px, py, prev, lane);
+      boxw = fmax(stage_polygon(P, r0, r1, v0, nv, px, py, prev, lane), 0.0) + 1.0;
       defer = boxw * (double)nrows > (double)ZW_BIG_CELLS;
     }
     if (defer) {
@@ -1749,7 +1707,7 @@ zonal_select_bracket_kernel(const PolyDev P, const T* __restrict__ raster, T nod
       int sx0 = 0, sxe = 0;
       if (lane < n_sr) {
         const int y = miny + lane * stride;
-        const int c = row_crossings(px, py, prev, nv, y, cross, lane);
+        const int c = row_crossings_call(px, py, prev, nv, y, cross, lane);
         if (c == 2) {
           const int xa = cross[0][lane], xb = cross[1][lane];
           if (xa <= maxx && xb > 0) { sx0 = xa < 0 ? 0 : xa; sxe = xb > P.width ? P.width : xb; }
@@ -1853,7 +1811,6 @@ zonal_select_main_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
   __shared__ int s_buf[WS_WARPS][ZW_MAXV + 2 * PG_MAX_HSPANS];
   int* buf = s_buf[warp];
   int* hbuf = buf + ZW_MAXV;
-  const int maxx = P.width - 1;
   WarpSelect<T> w;
   w.raster = raster; w.width = P.width; w.nodata = nodata; w.no_nodata = !has_nodata;
   w.hist_at = (unsigned)__cvta_generic_to_shared(hist);
@@ -1884,48 +1841,14 @@ zonal_select_main_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
     }
     w.n_active = 0; w.below = 0; w.cnt = 0; w.cells = 0;
     if (exact) zero_hist();
+    WarpSelectVisitor<T> scalar{w, main_mode};
     for (int base = miny; base <= maxy; base += 32) {
       const int y = base + lane;
       int cnt = 0;
-      if (y <= maxy) cnt = row_crossings(px, py, prev, nv, y, cross, lane);
-      const bool complex_row = cnt < 0;
-      const bool edge = edge_scalar && (y == 0 || y == P.height - 1);
-      const bool scalar_row = !complex_row && cnt >= 2 && (cnt > 2 || edge);
-      int fx0 = 0, fxe = 0, xh = 0, xt = 0;
-      if (!complex_row && !scalar_row && cnt == 2) {
-        constexpr int VEC = WarpSelect<T>::VEC;
-        const int xa = cross[0][lane], xb = cross[1][lane];
-        if (xa <= maxx && xb > 0 && (xa < 0 ? 0 : xa) < (xb > P.width ? P.width : xb)) {
-          fx0 = xa < 0 ? 0 : xa; fxe = xb > P.width ? P.width : xb;
-          w.cells += fxe - fx0;
-          const int64_t off = (int64_t)y * P.width + mis;
-          xh = fx0 + (int)((VEC - ((off + fx0) & (VEC - 1))) & (VEC - 1));
-          xt = fxe - (int)((off + fxe) & (VEC - 1));
-          if (xt < xh) xt = xh;
-        }
-      }
-      __syncwarp();
-      const unsigned complex_mask = __ballot_sync(0xffffffffu, complex_row);
-      unsigned scalar_mask = __ballot_sync(0xffffffffu, scalar_row);
-      const unsigned single_mask = __ballot_sync(0xffffffffu, fx0 < fxe);
-      while (scalar_mask) {            // the scalar rows first: they still need their raw crossings
-        const int r = __ffs(scalar_mask) - 1;
-        scalar_mask &= scalar_mask - 1;
-        const int c = __shfl_sync(0xffffffffu, cnt, r);
-        for (int i = 0; i + 1 < c; i += 2) {
-          const int xa = cross[i][r], xb = cross[i + 1][r];
-          if (xa <= maxx && xb > 0) {
-            const int x0 = xa < 0 ? 0 : xa, x1 = xb - 1 > maxx ? maxx : xb - 1;
-            if (x0 <= x1) {
-              if (lane == 0) w.cells += x1 - x0 + 1;
-              select_span(w, main_mode, base + r, x0, x1);
-            }
-          }
-        }
-      }
-      __syncwarp();
-      cross[0][lane] = fx0; cross[1][lane] = fxe; cross[2][lane] = xh; cross[3][lane] = xt;
-      __syncwarp();
+      if (y <= maxy) cnt = row_crossings_call(px, py, prev, nv, y, cross, lane);
+      unsigned single_mask;
+      const unsigned complex_mask = row_table<WarpSelect<T>::VEC>(P, mis, edge_scalar, base, cnt, cross, w.cells,
+                                                                   &single_mask, scalar);
       constexpr unsigned BM = (1u << ZW_ROWS) - 1u;
       if (sizeof(T) != 1 && exact) {
         // (rare: few distinct keys in a raster of wider cells) span by span with scalar loads
@@ -1975,15 +1898,8 @@ zonal_select_main_kernel(const PolyDev P, const T* __restrict__ raster, T nodata
       continue;
     }
     long long rank_lo, rank_hi;
-    double part = 0.0;
-    if (stat == GM_STAT_MEDIAN) {
-      rank_lo = (n - 1) / 2; rank_hi = n / 2;
-    } else {
-      const double frac = (double)(n - 1) * (q / 100.0);
-      rank_lo = (long long)floor(frac);
-      rank_hi = (long long)ceil(frac);
-      part = frac - floor(frac);
-    }
+    double part;
+    order_ranks(stat, q, n, &rank_lo, &rank_hi, &part);
     const long long in_lo = rank_lo - below, in_hi = rank_hi - below;
     __syncwarp();
     int e0, c0, e1, c1;
@@ -2028,15 +1944,8 @@ zonal_select_final_kernel(int stat, double q, int64_t p_begin, int64_t p_end, in
     const unsigned lo = state[p].lo, hi = state[p].hi;
     const unsigned* column = tables + (size_t)(p - p_begin) * WS_TABLE_WORDS + lane;
     long long rank_lo, rank_hi;
-    double part = 0.0;
-    if (stat == GM_STAT_MEDIAN) {
-      rank_lo = (n - 1) / 2; rank_hi = n / 2;
-    } else {
-      const double frac = (double)(n - 1) * (q / 100.0);
-      rank_lo = (long long)floor(frac);
-      rank_hi = (long long)ceil(frac);
-      part = frac - floor(frac);
-    }
+    double part;
+    order_ranks(stat, q, n, &rank_lo, &rank_hi, &part);
     long long in_lo = rank_lo - below, in_hi = rank_hi - below;
     unsigned klo = 0u, khi = 0u;
     bool found = false;
@@ -2256,7 +2165,7 @@ rasterize_tile_kernel(const PolyDev P, const int* __restrict__ tile_offsets, con
     for (int base = ya; base <= yb; base += 32) {
       const int y = base + lane;
       int cnt = 0;
-      if (y <= yb) cnt = row_crossings(s_px[warp], s_py[warp], s_prev[warp], nv, y, s_cross[warp], lane);
+      if (y <= yb) cnt = row_crossings_call(s_px[warp], s_py[warp], s_prev[warp], nv, y, s_cross[warp], lane);
       __syncwarp();
       const int rows_here = min(32, yb - base + 1);
       for (int r = 0; r < rows_here; ++r) {
@@ -2338,9 +2247,7 @@ zonal_values_kernel(const PolyDev P, const T* __restrict__ raster, T nodata, int
     __syncthreads();
     ValueVisitor<T> vis;
     vis.raster = raster; vis.width = P.width;
-    vis.active.nodata = nodata; vis.active.has_nodata = has_nodata;
-    vis.active.has_threshold = thresholds != nullptr;
-    vis.active.threshold = thresholds ? thresholds[p] : 0.0f;
+    vis.active = active_test(nodata, has_nodata, thresholds, p);
     vis.out = values + offsets[p]; vis.cursor = &cursor; vis.capacity = offsets[p + 1] - offsets[p];
     scan_polygon(P, p, buf, hbuf, vis);
     __syncthreads();
@@ -2365,17 +2272,6 @@ segment_select_kernel(const T* __restrict__ values, const long long* __restrict_
     if (threadIdx.x == 0) out[seg] = result;
     __syncthreads();
   }
-}
-
-__global__ void big_offsets_kernel(const long long* __restrict__ area, int64_t n, int smem_capacity,
-                                   long long* __restrict__ offsets, long long* __restrict__ total) {
-  // single thread: exclusive scan over the few polygons that exceed shared memory
-  long long acc = 0;
-  for (int64_t p = 0; p < n; ++p) {
-    offsets[p] = acc;
-    if (area[p] > smem_capacity) acc += area[p];
-  }
-  *total = acc;
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -2589,6 +2485,47 @@ static unsigned poly_grid(int64_t n) {
   return (unsigned)(n < cap ? (n > 0 ? n : 1) : cap);
 }
 
+// Where a raster of H x W cells stands against the grid of VEC-cell loads of the batched row
+// walk: *mis = offset of its first cell from that grid; *edge_scalar = a load on its first or last
+// row could reach outside the array (or the cells are not aligned to their own size), so those
+// rows are read with scalar loads.
+template <typename T>
+static void raster_alignment(const void* raster, int vec, int H, int W, int* mis, int* edge_scalar) {
+  *mis = (int)(((uintptr_t)raster / sizeof(T)) & (uintptr_t)(vec - 1));
+  *edge_scalar = ((uintptr_t)raster % sizeof(T)) != 0 || *mis != 0 || (((int64_t)H * W + *mis) % vec) != 0;
+}
+
+// Partials and covered cells of every polygon: zonal_reduce_warp_kernel takes the usual polygons
+// (`need`: the accumulators it keeps), zonal_reduce_kernel the ones it deferred to `work`, on a
+// grid of `deferred_grid` blocks.
+template <typename T>
+static cudaError_t launch_reduce(const PolyUpload& u, const Staged& raster, T nd, int has_nodata,
+                                 const float* thresholds, int need, unsigned deferred_grid, size_t smem_scan,
+                                 GmZonalPartial* partial, long long* cells, int* work, cudaStream_t s) {
+  const int64_t np_ = u.dev.n_polygons;
+  int mis, edge_scalar;
+  raster_alignment<T>(raster.dev, WarpReduce<T, ZW_ALL>::VEC, u.dev.height, u.dev.width, &mis, &edge_scalar);
+  int64_t wblocks = (np_ + ZW_WARPS - 1) / ZW_WARPS;
+  if (wblocks > (int64_t)sm_count() * ZW_MIN_BLOCKS) wblocks = (int64_t)sm_count() * ZW_MIN_BLOCKS;
+  auto* warp_kernel = need == ZW_SUM ? &zonal_reduce_warp_kernel<T, ZW_SUM>
+                    : need == ZW_MIN ? &zonal_reduce_warp_kernel<T, ZW_MIN>
+                    : need == ZW_MAX ? &zonal_reduce_warp_kernel<T, ZW_MAX>
+                    : &zonal_reduce_warp_kernel<T, ZW_ALL>;
+  warp_kernel<<<(unsigned)wblocks, 32 * ZW_WARPS, 0, s>>>(u.dev, (const T*)raster.dev, nd, has_nodata, thresholds,
+                                                           mis, edge_scalar, partial, cells, work);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  count_launch();
+  zonal_reduce_kernel<T><<<deferred_grid, PG_THREADS, smem_scan, s>>>(
+      u.dev, (const T*)raster.dev, nd, has_nodata, thresholds, partial, cells, work);
+  e = cudaGetLastError();
+  if (e == cudaSuccess) count_launch();
+  return e;
+}
+
+// on a CUDA error: free what the calling function allocated so far (its `cleanup`) and fail
+#define GM_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(std::string(#expr) + ": " + cudaGetErrorString(_e)); } } while (0)
+
 template <typename T>
 static int run_rasterize(PolyUpload& u, const void* burn, const void* nodata, Staged& out,
                          int64_t n_pixels, cudaStream_t s) {
@@ -2604,7 +2541,6 @@ static int run_rasterize(PolyUpload& u, const void* burn, const void* nodata, St
     void* all[] = {dburn, dminx, dmaxx, doffsets, dcursor, dlist, dtotal};
     for (void* p : all) if (p) cudaFreeAsync(p, s);
   };
-#define GM_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(std::string(#expr) + ": " + cudaGetErrorString(_e)); } } while (0)
   if (upload(&dburn, burn, sizeof(T) * (size_t)(np_ > 0 ? np_ : 1), s)) { cleanup(); return 1; }
   GM_TRY(cudaMallocAsync(&doffsets, sizeof(int) * (size_t)(n_tiles + 1), s));
   GM_TRY(cudaMemsetAsync(doffsets, 0, sizeof(int) * (size_t)(n_tiles + 1), s));
@@ -2640,7 +2576,6 @@ static int run_rasterize(PolyUpload& u, const void* burn, const void* nodata, St
       u.dev, (const int*)doffsets, (const int*)dlist, tiles_x, (const T*)dburn, nd, (T*)out.dev);
   GM_TRY(cudaGetLastError());
   count_launch();
-#undef GM_TRY
   cleanup();
   (void)n_pixels;
   return 0;
@@ -2661,7 +2596,6 @@ static int run_zonal(PolyUpload& u, const Staged& raster, const void* nodata, in
     void* all[] = {darea, dthr, dpartial, dout, doff, dtotal, dbig, scratch_work, scratch_list};
     for (void* p : all) if (p) cudaFreeAsync(p, s);
   };
-#define GM_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(std::string(#expr) + ": " + cudaGetErrorString(_e)); } } while (0)
   GM_TRY(cudaMallocAsync(&darea, sizeof(long long) * np_, s));
   if (thresholds && upload(&dthr, thresholds, sizeof(float) * np_, s)) { cleanup(); return 1; }
   const size_t smem_scan = scan_smem(u.dev.cap, PG_WARPS);
@@ -2686,11 +2620,9 @@ static int run_zonal(PolyUpload& u, const Staged& raster, const void* nodata, in
     scratch_list = dlist;
     // the streaming select takes float32 and integers up to 4 bytes (32-bit sortable keys)
     const bool streaming = sizeof(T) <= 4 && !thresholds && out;
-    constexpr int svec = 4;   // the kernels' cells per load
-    const int mis = (int)(((uintptr_t)raster.dev / sizeof(T)) & (svec - 1));
-    const int edge_scalar = ((uintptr_t)raster.dev % sizeof(T)) != 0 || mis != 0 ||
-                            (((int64_t)u.dev.height * u.dev.width + mis) % svec) != 0;
     if (streaming) {
+      int mis, edge_scalar;
+      raster_alignment<T>(raster.dev, WarpSelect<T>::VEC, u.dev.height, u.dev.width, &mis, &edge_scalar);
       // one warp per polygon, three kernels (bracket, main pass, final ranks) per chunk of
       // polygons; the bracket's cells of a chunk wait in per-polygon tables between the last two
       GM_TRY(cudaMallocAsync(&dout, sizeof(float) * np_, s));
@@ -2805,29 +2737,9 @@ static int run_zonal(PolyUpload& u, const Staged& raster, const void* nodata, in
     GM_TRY(cudaMallocAsync(&dwork, sizeof(int) * (size_t)(np_ + 2), s));
     scratch_work = dwork;
     GM_TRY(cudaMemsetAsync(dwork, 0, 2 * sizeof(int), s));
-    const int vec = WarpReduce<T, ZW_ALL>::VEC;
-    const int mis = (int)(((uintptr_t)raster.dev / sizeof(T)) & (uintptr_t)(vec - 1));
-    const int edge_scalar = ((uintptr_t)raster.dev % sizeof(T)) != 0 || mis != 0 ||
-                            (((int64_t)u.dev.height * u.dev.width + mis) % vec) != 0;
     const int need = partial ? ZW_ALL : stat == GM_STAT_MIN ? ZW_MIN : stat == GM_STAT_MAX ? ZW_MAX : ZW_SUM;
-    int64_t wblocks = (np_ + ZW_WARPS - 1) / ZW_WARPS;
-    if (wblocks > (int64_t)sm_count() * ZW_MIN_BLOCKS) wblocks = (int64_t)sm_count() * ZW_MIN_BLOCKS;
-#define GM_ZW(NEED)                                                                              \
-    zonal_reduce_warp_kernel<T, NEED><<<(unsigned)wblocks, 32 * ZW_WARPS, 0, s>>>(                \
-        u.dev, (const T*)raster.dev, nd, has_nodata, (const float*)dthr, mis, edge_scalar,        \
-        (GmZonalPartial*)dpartial, (long long*)darea, (int*)dwork)
-    if (need == ZW_SUM) GM_ZW(ZW_SUM);
-    else if (need == ZW_MIN) GM_ZW(ZW_MIN);
-    else if (need == ZW_MAX) GM_ZW(ZW_MAX);
-    else GM_ZW(ZW_ALL);
-#undef GM_ZW
-    GM_TRY(cudaGetLastError());
-    count_launch();
-    zonal_reduce_kernel<T><<<poly_grid(np_), PG_THREADS, smem_scan, s>>>(
-        u.dev, (const T*)raster.dev, nd, has_nodata, (const float*)dthr, (GmZonalPartial*)dpartial,
-        (long long*)darea, (const int*)dwork);
-    GM_TRY(cudaGetLastError());
-    count_launch();
+    GM_TRY(launch_reduce<T>(u, raster, nd, has_nodata, (const float*)dthr, need, poly_grid(np_), smem_scan,
+                            (GmZonalPartial*)dpartial, (long long*)darea, (int*)dwork, s));
     if (!order_stat && covered) {
       static_assert(sizeof(long long) == sizeof(int64_t), "covered is int64");
       GM_TRY(cudaMemcpyAsync(covered, darea, sizeof(long long) * np_, cudaMemcpyDeviceToHost, s));
@@ -2879,7 +2791,6 @@ static int run_zonal(PolyUpload& u, const Staged& raster, const void* nodata, in
     GM_TRY(cudaMemcpyAsync(out, dout, sizeof(float) * np_, cudaMemcpyDeviceToHost, s));
   }
   GM_TRY(cudaStreamSynchronize(s));
-#undef GM_TRY
   cleanup();
   return rc;
 }
@@ -2991,7 +2902,6 @@ static int run_zonal_partials_device(PolyUpload& u, const Staged& raster, const 
     void* all[] = {darea, dthr, dpartial, dwork};
     for (void* p : all) if (p) cudaFreeAsync(p, s);
   };
-#define GM_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(std::string(#expr) + ": " + cudaGetErrorString(_e)); } } while (0)
   GM_TRY(cudaMallocAsync(&darea, sizeof(long long) * np_, s));
   GM_TRY(cudaMallocAsync(&dpartial, sizeof(GmZonalPartial) * np_, s));
   GM_TRY(cudaMallocAsync(&dwork, sizeof(int) * (size_t)(np_ + 2), s));
@@ -3004,31 +2914,11 @@ static int run_zonal_partials_device(PolyUpload& u, const Staged& raster, const 
   const size_t smem_scan = scan_smem(u.dev.cap, PG_WARPS);
   if (smem_scan > 48 * 1024)
     GM_TRY(cudaFuncSetAttribute(zonal_reduce_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_scan));
-  const int vec = WarpReduce<T, ZW_ALL>::VEC;
-  const int mis = (int)(((uintptr_t)raster.dev / sizeof(T)) & (uintptr_t)(vec - 1));
-  const int edge_scalar = ((uintptr_t)raster.dev % sizeof(T)) != 0 || mis != 0 ||
-                          (((int64_t)u.dev.height * u.dev.width + mis) % vec) != 0;
-  int64_t wblocks = (np_ + ZW_WARPS - 1) / ZW_WARPS;
-  if (wblocks > (int64_t)sm_count() * ZW_MIN_BLOCKS) wblocks = (int64_t)sm_count() * ZW_MIN_BLOCKS;
   // only what the statistic needs (a stripe call for the mean runs the sum-only kernel)
   const int need = stat == GM_STAT_MIN ? ZW_MIN : stat == GM_STAT_MAX ? ZW_MAX
                  : (stat == GM_STAT_SUM || stat == GM_STAT_MEAN || stat == GM_STAT_COUNT) ? ZW_SUM : ZW_ALL;
-#define GM_ZW(NEED)                                                                              \
-  zonal_reduce_warp_kernel<T, NEED><<<(unsigned)wblocks, 32 * ZW_WARPS, 0, s>>>(                  \
-      u.dev, (const T*)raster.dev, nd, has_nodata, (const float*)dthr, mis, edge_scalar,          \
-      (GmZonalPartial*)dpartial, (long long*)darea, (int*)dwork)
-  if (need == ZW_SUM) GM_ZW(ZW_SUM);
-  else if (need == ZW_MIN) GM_ZW(ZW_MIN);
-  else if (need == ZW_MAX) GM_ZW(ZW_MAX);
-  else GM_ZW(ZW_ALL);
-#undef GM_ZW
-  GM_TRY(cudaGetLastError());
-  count_launch();
-  zonal_reduce_kernel<T><<<poly_grid(np_ < 1024 ? np_ : 1024), PG_THREADS, smem_scan, s>>>(
-      u.dev, (const T*)raster.dev, nd, has_nodata, (const float*)dthr, (GmZonalPartial*)dpartial,
-      (long long*)darea, (const int*)dwork);
-  GM_TRY(cudaGetLastError());
-  count_launch();
+  GM_TRY(launch_reduce<T>(u, raster, nd, has_nodata, (const float*)dthr, need, poly_grid(np_ < 1024 ? np_ : 1024),
+                          smem_scan, (GmZonalPartial*)dpartial, (long long*)darea, (int*)dwork, s));
   zonal_pack_kernel<<<(unsigned)((np_ + 255) / 256), 256, 0, s>>>(
       (const GmZonalPartial*)dpartial, (const long long*)darea, np_, sums, extremes);
   GM_TRY(cudaGetLastError());
