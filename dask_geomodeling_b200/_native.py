@@ -155,6 +155,8 @@ SYMBOLS = {
     "gm_get_eval_mode": (_i, []),
     "gm_jit_source": (_i, [_P(GmProgram), _P(ctypes.c_int32), _P(ctypes.c_int32), ctypes.c_char_p, _i64,
                            _P(_i64)]),
+    "gm_jit_baked_source": (_i, [_P(GmProgram), _P(ctypes.c_int32), _P(ctypes.c_int32), ctypes.c_char_p, _i64,
+                                 _P(_i64)]),
     "gm_jit_check": (_i, [_P(GmProgram), _P(ctypes.c_int32), _P(ctypes.c_int32), _P(_i64)]),
     "gm_jit_compile_count": (_i64, []),
     "gm_resample_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _d, _d, _d, _d, _vp]),

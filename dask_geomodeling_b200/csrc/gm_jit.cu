@@ -12,7 +12,8 @@
 //     is one fully used contiguous segment (no shared-memory staging needed);
 //   * U groups per thread are loaded before the first is evaluated (U*V = 16 pixels,
 //     >= 96 B in flight per thread on cfg2), streaming cache hints on both sides;
-//   * lookup tables live in shared memory.
+//   * a small dense Reclassify table is two 32-bit literal words, other baked lookup tables
+//     live in shared memory (see JitLayout).
 //
 // The interpreter in gm_eval.cu stays the zero-latency path for small rasters; the
 // two are checked against each other and against the oracle by the parity tests.
@@ -102,13 +103,35 @@ static std::string hex(uint64_t v) {
 static std::string num(long long v) { return std::to_string(v); }
 static const char* tf(bool b) { return b ? "true" : "false"; }
 
+// Where each lookup table lives.  A baked table's contents are part of the module (and of the
+// cache key): a dense ND_ONLY Reclassify table of at most 64 entries as two 32-bit literal words
+// (`bits`, reclass_bits), any other baked table in shared memory (`in_smem`).  A table that is not
+// baked is read from global memory through the pointers of the parameter block.
 struct JitLayout {
   int V, U;
   bool baked[GM_MAX_TABLES];
   bool in_smem[GM_MAX_TABLES];
+  bool bits[GM_MAX_TABLES];
 };
 
 static const int kBakeLimit = 2048;  // table entries baked into the module / held in smem
+static const int kBitsLimit = 64;    // entries of a table held as two 32-bit words
+
+// Every use of table t is an ND_ONLY Reclassify of an I32 key, the table is dense, and its key range
+// lies inside int32 (the 32-bit range test of reclass_bits).
+static bool bits_table(const GmProgram* prog, int t) {
+  const GmTable& g = prog->tables[t];
+  if (g.kind != GM_TABLE_DENSE || !g.hit || g.n < 1 || g.n > kBitsLimit || g.base < INT32_MIN ||
+      g.base + g.n - 1 > INT32_MAX)
+    return false;
+  for (int pc = 0; pc < prog->n_instr; ++pc) {
+    const GmInstr& in = prog->instr[pc];
+    if ((in.op == GM_OP_RECLASS || in.op == GM_OP_CLASSIFY) && in.aux == t &&
+        (in.op != GM_OP_RECLASS || !(in.flags & GM_F_ND_T) || in.cls_a != GM_C_I32))
+      return false;
+  }
+  return true;
+}
 
 static JitLayout plan_layout(const GmProgram* prog, const int* in_dtype, const int* out_dtype) {
   JitLayout L;
@@ -121,7 +144,8 @@ static JitLayout plan_layout(const GmProgram* prog, const int* in_dtype, const i
   for (int t = 0; t < prog->n_tables; ++t) total += prog->tables[t].n;
   for (int t = 0; t < GM_MAX_TABLES; ++t) {
     L.baked[t] = t < prog->n_tables && total <= kBakeLimit;
-    L.in_smem[t] = L.baked[t];
+    L.bits[t] = L.baked[t] && bits_table(prog, t);
+    L.in_smem[t] = L.baked[t] && !L.bits[t];
   }
   return L;
 }
@@ -166,12 +190,30 @@ static std::string table_args(const GmProgram* prog, int t) {
   return s;
 }
 
-static std::string emit_instruction(const GmProgram* prog, const GmInstr& in) {
+// IsData / IsNoData at pc + 1 over the result of a Step at pc, folded into the Step (the IsNd arm
+// functor of the prelude).  The Step has no other consumer: the IsData directly follows it and
+// replaces the accumulator.  Only in a baked kernel, where the compares of constant arms become
+// literals: with the constants in the parameter block the fold costs instructions (cfg2: 21.6 ->
+// 25.3 per pixel in tools/jit_sass.py).  Only Step: the same fold over Clip measured more
+// instructions, and Clip / Mask / MaskBelow have at most one constant arm to gain.
+static const GmInstr* folded_is_data(const GmProgram* prog, int pc) {
+  const GmInstr& in = prog->instr[pc];
+  if (!t_bake || pc + 1 >= prog->n_instr) return nullptr;
+  const GmInstr& nd = prog->instr[pc + 1];
+  const bool producer = in.op == GM_OP_STEP;
+  const bool is_data = nd.op == GM_OP_ISDATA || nd.op == GM_OP_ISNODATA;
+  return producer && is_data && (nd.flags & GM_F_ND_A) && class_fits(nd.cls_a, prog->word) ? &nd : nullptr;
+}
+
+// `fold`: the IsData / IsNoData that folded_is_data found for this instruction, or null
+static std::string emit_instruction(const GmProgram* prog, const GmInstr& in, const JitLayout& L,
+                                    const GmInstr* fold) {
   const int word = prog->word;
   const int pc = (int)(&in - prog->instr);
   const bool fa = in.flags & GM_F_ND_A, fb = in.flags & GM_F_ND_B;
   const std::string b = operand_b(in, pc);
-  std::string s;
+  const std::string arm = fold ? std::string(", IsNd<") + class_type(fold->cls_a) + ">{" + kref(pc + 1, 1) + "}" : "";
+  std::string s, call;   // call: a Step, which takes the arm functor
   switch (in.op) {
     case GM_OP_LOAD:
     case GM_OP_MATB: {
@@ -212,6 +254,14 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in) {
       const GmTable& g = prog->tables[in.aux];
       const char* A = in.cls_a == GM_C_I32 ? "int32_t" : "int64_t";
       if (in.cls_a != GM_C_I32 && word != 8) break;
+      if (L.bits[in.aux]) {
+        const unsigned lut = ((in.flags & GM_F_SELECT) ? 0u : 1u) | 2u;   // as in reclass
+        uint32_t w[2] = {0, 0};
+        for (int i = 0; i < g.n; ++i) w[i / 32] |= ((lut >> g.hit[i]) & 1u) << (i % 32);
+        s = std::string("acc = reclass_bits<") + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ">(acc, " +
+            num(w[0]) + "u, " + num(w[1]) + "u, " + num(g.n) + "u, " + num(g.base) + ", " + kref(pc, 1) + ");";
+        break;
+      }
       s = std::string("acc = reclass<") + A + ", " + tf(g.kind == GM_TABLE_DENSE) + ", " +
           tf(in.flags & GM_F_ND_T) + ", " + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ", " +
           tf(in.cls_out == GM_C_F64) + ">(acc, " + table_args(prog, in.aux) + ", " + num(g.n) + ", " +
@@ -242,9 +292,9 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in) {
       break;
     case GM_OP_STEP:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
-        s = std::string("acc = step<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ", " + tf(fa) +
-            ">(acc, " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 2) + ", " + kref(pc, 3) + ", " +
-            kref(pc, 4) + ");";
+        call = std::string("step<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ", " + tf(fa) +
+               ">(acc, " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 2) + ", " + kref(pc, 3) + ", " +
+               kref(pc, 4) + arm + ")";
       break;
     case GM_OP_CLASSIFY:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
@@ -262,12 +312,15 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in) {
       break;
     }
   }
+  if (!call.empty())
+    s = fold ? std::string("acc = data_flag<") + tf(fold->op == GM_OP_ISNODATA) + ">(" + call + ");"
+             : "acc = " + call + ";";
   return s;
 }
 
 static void emit_table_data(std::string& src, const GmProgram* prog, const JitLayout& L) {
   for (int t = 0; t < prog->n_tables; ++t) {
-    if (!L.baked[t]) continue;
+    if (!L.in_smem[t]) continue;
     const GmTable& g = prog->tables[t];
     const std::string id = num(t);
     if (g.keys) {
@@ -301,12 +354,13 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
          num(GM_MAX_INSTR) + "][6]; };\n";
   emit_table_data(src, prog, L);
 
-  // Baked tables are file-scope __shared__ arrays (compile-time addresses); the others
-  // travel as global pointers through pixel() and group().
+  // Tables in shared memory are file-scope __shared__ arrays (compile-time addresses); the others
+  // travel as global pointers through pixel() and group(); bits tables are literals of reclass_bits.
   std::string tab_params, tab_args;
   for (int t = 0; t < prog->n_tables; ++t) {
     const GmTable& g = prog->tables[t];
     const std::string id = num(t), n = num(std::max(g.n, 1));
+    if (L.bits[t]) continue;
     if (L.in_smem[t]) {
       if (g.keys) src += "__shared__ int64_t t" + id + "k[" + n + "];\n";
       if (g.vals) src += "__shared__ uint64_t t" + id + "v[" + n + "];\n";
@@ -325,8 +379,10 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
   for (int i = 0; i < prog->n_outputs; ++i) { src += std::string(first ? "" : ", ") + "S& o" + num(i); first = false; }
   src += tab_params + ") {\n  S acc = 0, r0 = 0, r1 = 0, r2 = 0, r3 = 0;\n";
   for (int pc = 0; pc < prog->n_instr; ++pc) {
-    const std::string line = emit_instruction(prog, prog->instr[pc]);
+    const GmInstr* fold = folded_is_data(prog, pc);
+    const std::string line = emit_instruction(prog, prog->instr[pc], L, fold);
     if (!line.empty()) src += "  " + line + "\n";
+    if (fold && !line.empty()) ++pc;
   }
   src += "  (void)r0; (void)r1; (void)r2; (void)r3;\n}\n";
 
@@ -337,20 +393,28 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
   for (int i = 0; i < prog->n_inputs; ++i) { src += std::string(first ? "" : ", ") + "const uint32_t* a" + num(i); first = false; }
   for (int i = 0; i < prog->n_outputs; ++i) { src += std::string(first ? "" : ", ") + "uint32_t* w" + num(i); first = false; }
   src += tab_params + ") {\n";
+  // 1-byte outputs are packed four pixels to a word (pack_bytes), the others stored per pixel
+  auto packed = [&](int i) { return dtype_size(out_dtype[i]) == 1 && V % 4 == 0; };
   for (int j = 0; j < V; ++j) {
-    src += "  {";
-    for (int i = 0; i < prog->n_outputs; ++i) src += " S o" + num(i) + ";";
-    src += " pixel(p";
+    src += "  ";
+    for (int i = 0; i < prog->n_outputs; ++i) src += "S o" + num(i) + "_" + num(j) + "; ";
+    src += "pixel(p";
     first = false;
     for (int i = 0; i < prog->n_inputs; ++i) {
       src += std::string(first ? "" : ", ") + "element<" + storage_type(in_dtype[i]) + ", " + num(j) + ">(a" + num(i) + ")";
       first = false;
     }
-    for (int i = 0; i < prog->n_outputs; ++i) { src += std::string(first ? "" : ", ") + "o" + num(i); first = false; }
+    for (int i = 0; i < prog->n_outputs; ++i) { src += std::string(first ? "" : ", ") + "o" + num(i) + "_" + num(j); first = false; }
     src += tab_args + ");";
-    for (int i = 0; i < prog->n_outputs; ++i)
-      src += " set_element<" + num(dtype_size(out_dtype[i])) + ", " + num(j) + ">(w" + num(i) + ", o" + num(i) + ");";
-    src += " }\n";
+    for (int i = 0; i < prog->n_outputs; ++i) {
+      const std::string o = "o" + num(i) + "_" + num(j), w = "w" + num(i);
+      if (!packed(i))
+        src += " set_element<" + num(dtype_size(out_dtype[i])) + ", " + num(j) + ">(" + w + ", " + o + ");";
+      else if (j % 4 == 3)
+        src += " " + w + "[" + num(j / 4) + "] = pack_bytes(o" + num(i) + "_" + num(j - 3) + ", o" + num(i) + "_" +
+               num(j - 2) + ", o" + num(i) + "_" + num(j - 1) + ", " + o + ");";
+    }
+    src += "\n";
   }
   src += "}\n";
 
@@ -360,6 +424,7 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
   for (int t = 0; t < prog->n_tables; ++t) {
     const GmTable& g = prog->tables[t];
     const std::string id = num(t);
+    if (L.bits[t]) continue;
     if (L.in_smem[t]) {
       src += "  for (int i = tid; i < " + num(g.n) + "; i += 256) {";
       if (g.keys) src += " t" + id + "k[i] = g_t" + id + "k[i];";
@@ -676,9 +741,15 @@ int jit_launch(const GmProgram* prog, const void* const* in, const int* in_dtype
     p.tv[t] = (const uint64_t*)tvals[t];
     p.th[t] = (const uint8_t*)thit[t];
   }
+  // One block per chunk of 256 * U groups.  A grid of resident blocks that strides over the chunks
+  // streams slower (tools/chain_ceiling.cu on one B200: 0.29-0.30 ms against 0.263 ms for the cfg2
+  // pattern), so the grid is capped at the resident blocks only when every block first copies its
+  // lookup tables into shared memory, which a block per chunk would repeat ~50 times as often.
   const int64_t per_block = 256LL * L.U * L.V;
   int64_t grid = (n + per_block - 1) / per_block;
-  const int64_t cap = (int64_t)sm_count() * k->blocks_per_sm;
+  bool smem_tables = false;
+  for (int t = 0; t < prog->n_tables; ++t) smem_tables = smem_tables || L.in_smem[t];
+  const int64_t cap = smem_tables ? (int64_t)sm_count() * k->blocks_per_sm : (int64_t)INT32_MAX;
   if (grid > cap) grid = cap;
   if (grid < 1) grid = 1;
   void* args[] = {&p};
@@ -694,15 +765,18 @@ int64_t jit_compile_count() { return g_compiles.load(); }
 
 using namespace gm;
 
-// Test / inspection hook: the CUDA source generated for `prog` (no GPU needed).
-extern "C" int gm_jit_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
-                             char* buffer, int64_t capacity, int64_t* length) {
+// Test / inspection hooks: the CUDA source generated for `prog`, with its constants as kernel
+// parameters or baked (no GPU needed).
+static int jit_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype, bool bake,
+                      char* buffer, int64_t capacity, int64_t* length) {
   if (!prog || !length) return fail("gm_jit_source: null argument");
   if (prog->n_instr < 1 || prog->n_instr > GM_MAX_INSTR || prog->n_inputs > GM_MAX_INPUTS ||
       prog->n_outputs > GM_MAX_OUTPUTS || prog->n_tables > GM_MAX_TABLES)
     return fail("gm_jit_source: bad program");
   const JitLayout L = plan_layout(prog, in_dtype, out_dtype);
+  t_bake = bake ? prog : nullptr;
   const std::string source = generate(prog, in_dtype, out_dtype, L);
+  t_bake = nullptr;
   *length = (int64_t)source.size();
   if (buffer && capacity > 0) {
     const size_t n = std::min((size_t)capacity - 1, source.size());
@@ -710,6 +784,16 @@ extern "C" int gm_jit_source(const GmProgram* prog, const int32_t* in_dtype, con
     buffer[n] = 0;
   }
   return 0;
+}
+
+extern "C" int gm_jit_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
+                             char* buffer, int64_t capacity, int64_t* length) {
+  return jit_source(prog, in_dtype, out_dtype, false, buffer, capacity, length);
+}
+
+extern "C" int gm_jit_baked_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
+                                   char* buffer, int64_t capacity, int64_t* length) {
+  return jit_source(prog, in_dtype, out_dtype, true, buffer, capacity, length);
 }
 
 // Compile `prog` with NVRTC without loading it (works without a GPU): used by the CPU

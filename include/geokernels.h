@@ -198,6 +198,10 @@ int  gm_get_eval_mode(void);
  * needs a GPU); number of kernels compiled so far                            */
 int  gm_jit_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
                    char* buffer, int64_t capacity, int64_t* length);
+/* the same with the program's constants as literals: the kernel a program gets
+ * when its constants repeat on large rasters (tools/jit_sass.py)              */
+int  gm_jit_baked_source(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
+                         char* buffer, int64_t capacity, int64_t* length);
 int  gm_jit_check(const GmProgram* prog, const int32_t* in_dtype, const int32_t* out_dtype,
                   int64_t* cubin_bytes);
 int64_t gm_jit_compile_count(void);
