@@ -7,6 +7,7 @@ linked into dask_geomodeling_b200/libgeokernels.so with a static cudart, so the
 library has no dependency on torch or on a CUDA toolkit at run time.
 """
 import os
+import re
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -42,16 +43,33 @@ def sources():
 
 def _deps_mtime():
     hdrs = [os.path.join(HERE, f) for f in os.listdir(HERE) if f.endswith((".cuh", ".h"))]
-    hdrs.append(os.path.join(os.path.dirname(PKG), "include", "geokernels.h"))
+    include = os.path.join(os.path.dirname(PKG), "include")
+    hdrs += [os.path.join(include, f) for f in os.listdir(include) if f.endswith(".h")]
     return max(os.path.getmtime(h) for h in hdrs)
 
 
+_INCLUDE = re.compile(r'^#include "([^"]+)"[ \t]*$', re.M)
+
+
+def _spliced(path, seen):
+    """The text of `path` with every `#include "..."` replaced by the included file (found
+    relative to the including one), itself spliced; a file already spliced is left out."""
+    def include(m):
+        inc = os.path.normpath(os.path.join(os.path.dirname(path), m.group(1)))
+        if inc in seen:
+            return ""
+        seen.add(inc)
+        return _spliced(inc, seen)
+    return _INCLUDE.sub(include, open(path).read())
+
+
 def _embed_prelude():
-    """gm_jit_prelude.cuh -> build/gm_jit_prelude.inc (a C++ raw string literal that
-    gm_jit.cu includes; NVRTC compiles it at run time)."""
+    """gm_jit_prelude.cuh, with the headers it includes spliced in -> build/gm_jit_prelude.inc
+    (a C++ raw string literal that gm_jit.cu includes; NVRTC compiles it at run time, with no
+    include path)."""
     src = os.path.join(HERE, "gm_jit_prelude.cuh")
     dst = os.path.join(BUILD, "gm_jit_prelude.inc")
-    text = 'R"GMJIT(' + open(src).read() + ')GMJIT"\n'
+    text = 'R"GMJIT(' + _spliced(src, {src}) + ')GMJIT"\n'
     if not os.path.exists(dst) or open(dst).read() != text:
         with open(dst, "w") as f:
             f.write(text)

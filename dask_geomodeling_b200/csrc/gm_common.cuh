@@ -35,7 +35,7 @@ void count_launch(int n = 1);
     gm::count_launch();                                                        \
   } while (0)
 
-inline int dtype_size(int dt) {
+__host__ __device__ inline int dtype_size(int dt) {
   switch (dt) {
     case GM_BOOL: case GM_U8: case GM_I8: return 1;
     case GM_U16: case GM_I16: return 2;

@@ -14,13 +14,17 @@
 // Two machines are instantiated: 32-bit slots (classes I32/F32, V = 16) and 64-bit
 // slots (all four classes, V = 8).
 //
-// Reference semantics restated per op: see include/geokernels.h (GmOp) and
-// SURVEY.md Appendix B; reference code raster/elemwise.py:235-299, :551-638,
-// :726-757 and raster/misc.py:98-123, :208-222, :245-251, :309-328, :387-399,
-// :482-515.
+// What each instruction does to a pixel is defined once, in gm_eval_ops.cuh, which the
+// specialised kernels (gm_jit.cu) share; this file owns the staging, the operand addressing and the
+// dispatch of classes and opcodes.
 #include "gm_common.cuh"
 #include "gm_jit.h"
 #include <type_traits>
+
+// The transcendentals and the integer power are kept out of line: rare, large, and they would
+// otherwise dictate the register allocation of the whole interpreter.
+#define GM_OUTLINE __device__ __noinline__
+#include "gm_eval_ops.cuh"
 
 namespace gm {
 
@@ -57,156 +61,9 @@ struct EvalParams {
   GmInstr instr[GM_MAX_INSTR];
 };
 
-__host__ __device__ inline int dsize(int dt) {
-  switch (dt) {
-    case GM_BOOL: case GM_U8: case GM_I8: return 1;
-    case GM_U16: case GM_I16: return 2;
-    case GM_U32: case GM_I32: case GM_F32: return 4;
-    default: return 8;
-  }
-}
-
 template <int W> struct SlotOf;
 template <> struct SlotOf<4> { typedef uint32_t type; };
 template <> struct SlotOf<8> { typedef uint64_t type; };
-
-// ---- raw bits <-> typed value -------------------------------------------------
-template <typename T> struct Raw;
-template <> struct Raw<int32_t> {
-  static constexpr int cls = GM_C_I32;
-  static __device__ __forceinline__ int32_t get(uint64_t b) { return (int32_t)(uint32_t)b; }
-  static __device__ __forceinline__ uint64_t put(int32_t v) { return (uint64_t)(uint32_t)v; }
-};
-template <> struct Raw<float> {
-  static constexpr int cls = GM_C_F32;
-  static __device__ __forceinline__ float get(uint64_t b) { return __uint_as_float((uint32_t)b); }
-  static __device__ __forceinline__ uint64_t put(float v) { return (uint64_t)__float_as_uint(v); }
-};
-template <> struct Raw<int64_t> {
-  static constexpr int cls = GM_C_I64;
-  static __device__ __forceinline__ int64_t get(uint64_t b) { return (int64_t)b; }
-  static __device__ __forceinline__ uint64_t put(int64_t v) { return (uint64_t)v; }
-};
-template <> struct Raw<double> {
-  static constexpr int cls = GM_C_F64;
-  static __device__ __forceinline__ double get(uint64_t b) { return __longlong_as_double((long long)b); }
-  static __device__ __forceinline__ uint64_t put(double v) { return (uint64_t)__double_as_longlong(v); }
-};
-
-template <typename T> struct IsFloat { static constexpr bool value = std::is_floating_point<T>::value; };
-template <typename T> __device__ __forceinline__ T quiet_nan();
-template <> __device__ __forceinline__ float quiet_nan<float>() { return __int_as_float(0x7fc00000); }
-template <> __device__ __forceinline__ double quiet_nan<double>() { return __longlong_as_double(0x7ff8000000000000LL); }
-template <> __device__ __forceinline__ int32_t quiet_nan<int32_t>() { return 0; }
-template <> __device__ __forceinline__ int64_t quiet_nan<int64_t>() { return 0; }
-
-// slot of class `cls` -> T (NumPy astype); the class switch is warp-uniform
-template <typename T, typename S>
-__device__ __forceinline__ T widen(S s, int cls) {
-  if constexpr (sizeof(S) == 4) {
-    return cls == GM_C_I32 ? (T)Raw<int32_t>::get(s) : (T)Raw<float>::get(s);
-  } else {
-    switch (cls) {
-      case GM_C_I32: return (T)Raw<int32_t>::get(s);
-      case GM_C_F32: return (T)Raw<float>::get(s);
-      case GM_C_I64: return (T)Raw<int64_t>::get(s);
-      default: return (T)Raw<double>::get(s);
-    }
-  }
-}
-
-// convert one slot between classes; `nan_if` marks the sentinel -> NaN substitution
-template <typename S>
-__device__ __forceinline__ S convert_slot(S s, int from, int to) {
-  if (from == to) return s;
-  if (to == GM_C_I32) return (S)Raw<int32_t>::put(widen<int32_t>(s, from));
-  if (to == GM_C_F32) return (S)Raw<float>::put(widen<float>(s, from));
-  if constexpr (sizeof(S) == 8) {
-    if (to == GM_C_I64) return (S)Raw<int64_t>::put(widen<int64_t>(s, from));
-    return (S)Raw<double>::put(widen<double>(s, from));
-  }
-  return s;
-}
-
-template <typename S>
-__device__ __forceinline__ bool slot_equals(S s, uint64_t k, int cls) {
-  if (cls == GM_C_I32) return Raw<int32_t>::get(s) == Raw<int32_t>::get(k);
-  if (cls == GM_C_F32) return Raw<float>::get(s) == Raw<float>::get(k);
-  if constexpr (sizeof(S) == 8) {
-    if (cls == GM_C_I64) return Raw<int64_t>::get(s) == Raw<int64_t>::get(k);
-    return Raw<double>::get(s) == Raw<double>::get(k);
-  }
-  return false;
-}
-
-template <typename S> __device__ __forceinline__ S nan_slot(int cls) {
-  if (cls == GM_C_F32) return (S)0x7fc00000u;
-  if constexpr (sizeof(S) == 8) return (S)0x7ff8000000000000ULL;
-  return (S)0;
-}
-
-// ---- arithmetic helpers ---------------------------------------------------------
-__device__ __forceinline__ int32_t w_add(int32_t a, int32_t b) { return (int32_t)((uint32_t)a + (uint32_t)b); }
-__device__ __forceinline__ int64_t w_add(int64_t a, int64_t b) { return (int64_t)((uint64_t)a + (uint64_t)b); }
-__device__ __forceinline__ float w_add(float a, float b) { return a + b; }
-__device__ __forceinline__ double w_add(double a, double b) { return a + b; }
-__device__ __forceinline__ int32_t w_sub(int32_t a, int32_t b) { return (int32_t)((uint32_t)a - (uint32_t)b); }
-__device__ __forceinline__ int64_t w_sub(int64_t a, int64_t b) { return (int64_t)((uint64_t)a - (uint64_t)b); }
-__device__ __forceinline__ float w_sub(float a, float b) { return a - b; }
-__device__ __forceinline__ double w_sub(double a, double b) { return a - b; }
-__device__ __forceinline__ int32_t w_mul(int32_t a, int32_t b) { return (int32_t)((uint32_t)a * (uint32_t)b); }
-__device__ __forceinline__ int64_t w_mul(int64_t a, int64_t b) { return (int64_t)((uint64_t)a * (uint64_t)b); }
-__device__ __forceinline__ float w_mul(float a, float b) { return a * b; }
-__device__ __forceinline__ double w_mul(double a, double b) { return a * b; }
-
-template <typename T> __device__ __forceinline__ T w_div(T a, T b) {
-  if constexpr (IsFloat<T>::value) return a / b; else return b == 0 ? T(0) : a / b;
-}
-// numpy integer power: square-and-multiply with wrap-around.  A negative
-// exponent raises in numpy; here it yields 0 (documented limitation).
-template <typename T> __device__ __noinline__ T int_pow(T base, T e) {
-  if (e < 0) return 0;
-  T r = 1;
-  while (e) {
-    if (e & 1) r = w_mul(r, base);
-    e >>= 1;
-    if (e) base = w_mul(base, base);
-  }
-  return r;
-}
-// transcendentals are kept out of line: rare, large, and they would otherwise
-// dictate the register allocation of the whole interpreter
-__device__ __noinline__ float  t_pow(float a, float b) { return powf(a, b); }
-__device__ __noinline__ double t_pow(double a, double b) { return pow(a, b); }
-__device__ __noinline__ float  t_exp(float a) { return expf(a); }
-__device__ __noinline__ double t_exp(double a) { return exp(a); }
-__device__ __noinline__ float  t_log(float a) { return logf(a); }
-__device__ __noinline__ double t_log(double a) { return log(a); }
-__device__ __noinline__ float  t_log10(float a) { return log10f(a); }
-__device__ __noinline__ double t_log10(double a) { return log10(a); }
-
-template <typename T> __device__ __forceinline__ T w_pow(T a, T b) {
-  if constexpr (IsFloat<T>::value) return t_pow(a, b); else return int_pow<T>(a, b);
-}
-template <typename T> __device__ __forceinline__ T w_exp(T a) {
-  if constexpr (IsFloat<T>::value) return t_exp(a); else return a;
-}
-template <typename T> __device__ __forceinline__ T w_log(T a) {
-  if constexpr (IsFloat<T>::value) return t_log(a); else return a;
-}
-template <typename T> __device__ __forceinline__ T w_log10(T a) {
-  if constexpr (IsFloat<T>::value) return t_log10(a); else return a;
-}
-template <typename T> __device__ __forceinline__ bool finite_(T v) {
-  if constexpr (IsFloat<T>::value) return isfinite(v); else return true;
-}
-template <typename T> __device__ __forceinline__ T abs_(T v) {
-  if constexpr (IsFloat<T>::value) return fabs(v); else return v < 0 ? -v : v;
-}
-// np.isclose(x, y): less_equal(abs(x - y), tol) & isfinite(y) | (x == y)
-template <typename T> __device__ __forceinline__ bool close_(T x, T y, T tol, bool y_finite) {
-  return ((abs_(w_sub(x, y)) <= tol) && y_finite) || (x == y);
-}
 
 // ---- mbarrier / TMA bulk copy wrappers (PTX) -----------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -261,21 +118,19 @@ __device__ __forceinline__ void with_class(int cls, F&& f) {
   }
 }
 
-template <typename To, typename From> __device__ __forceinline__ To astype(From v) { return (To)v; }
-
-// acc[i] (class From) -> class To; the sentinel becomes NaN when asked (float targets)
-template <typename From, typename To, int V, typename S>
-__device__ __forceinline__ void convert_loop(S (&x)[V], bool nanify, uint64_t k) {
-  const From nd = Raw<From>::get(k);
+// acc[i] = f(acc[i], i) for the V pixels of the thread
+template <int V, typename S, typename F> __device__ __forceinline__ void each(S (&acc)[V], F&& f) {
 #pragma unroll
-  for (int i = 0; i < V; ++i) {
-    const From v = Raw<From>::get(x[i]);
-    To r = astype<To>(v);
-    if constexpr (IsFloat<To>::value) r = (nanify && v == nd) ? quiet_nan<To>() : r;
-    x[i] = (S)Raw<To>::put(r);
-  }
+  for (int i = 0; i < V; ++i) acc[i] = f(acc[i], i);
 }
 
+// operand b of pixel i: a slot in shared memory (register file or a staged input that already is a
+// slot of the right class)
+template <typename S> __device__ __forceinline__ uint64_t b_at(const S* __restrict__ bp, int i) {
+  return (uint64_t)bp[i * THREADS + threadIdx.x];
+}
+
+// x[i] (class `from`) -> class `to`; the sentinel k becomes NaN when asked (float targets)
 template <int W, int V, typename S>
 __device__ __forceinline__ void convert_all(S (&x)[V], int from, int to, bool nanify, uint64_t k) {
   if (from == to) return;
@@ -283,7 +138,7 @@ __device__ __forceinline__ void convert_all(S (&x)[V], int from, int to, bool na
     typedef decltype(ft) From;
     with_class<W>(to, [&](auto tt) {
       typedef decltype(tt) To;
-      if constexpr (!std::is_same<From, To>::value) convert_loop<From, To, V, S>(x, nanify, k);
+      if constexpr (!std::is_same<From, To>::value) each(x, [&](S v, int) { return cvt<From, To>(v, nanify, k); });
     });
   });
 }
@@ -336,233 +191,92 @@ __device__ __forceinline__ void write_output(unsigned char* base, int dtype, con
 }
 
 // ---- typed instructions ------------------------------------------------------------------------
-// Binary arithmetic / comparison: acc and b both hold class T.  b comes from shared
-// memory (register or staged 32/64-bit input: `bp`) or is the immediate k0.
-template <typename T, int V, bool IMM, typename S>
-__device__ __forceinline__ void exec_binary(const GmInstr& in, S (&acc)[V], const S* __restrict__ bp) {
+// Binary arithmetic / comparison: acc and b both hold class T; b is the immediate k0 (IMM) or a
+// slot in shared memory (`bp`).
+template <int OP, typename T, bool IMM, int V, typename S>
+__device__ __forceinline__ void binary_loop(const GmInstr& in, S (&acc)[V], const S* __restrict__ bp) {
   const bool fa = in.flags & GM_F_ND_A, fb = (in.flags & GM_F_ND_B) && !IMM;
-  const T nda = Raw<T>::get(in.k[1]), ndb = Raw<T>::get(in.k[2]);
-  const T bimm = Raw<T>::get(in.k[0]);
-  const int tid = threadIdx.x;
-#define GM_B(i) (IMM ? bimm : Raw<T>::get(bp[(i) * THREADS + tid]))
-#define GM_MATH(EXPR)                                                          \
-  {                                                                            \
-    const T fill = Raw<T>::get(in.k[3]);                                       \
-    _Pragma("unroll") for (int i = 0; i < V; ++i) {                            \
-      const T x = Raw<T>::get(acc[i]);                                         \
-      const T y = GM_B(i);                                                     \
-      const T r = (EXPR);                                                      \
-      const bool bad = (fa && x == nda) || (fb && y == ndb) || !finite_(r);    \
-      acc[i] = (S)Raw<T>::put(bad ? fill : r);                                 \
-    }                                                                          \
-  }
-#define GM_CMP(EXPR)                                                           \
-  {                                                                            \
-    const S fill = (S)in.k[3];                                                 \
-    _Pragma("unroll") for (int i = 0; i < V; ++i) {                            \
-      const T x = Raw<T>::get(acc[i]);                                         \
-      const T y = GM_B(i);                                                     \
-      const bool bad = (fa && x == nda) || (fb && y == ndb);                   \
-      acc[i] = bad ? fill : (S)((EXPR) ? 1u : 0u);                             \
-    }                                                                          \
-  }
+  const uint64_t k0 = in.k[0], k1 = in.k[1], k2 = in.k[2], k3 = in.k[3];
+  each(acc, [&](S a, int i) {
+    const uint64_t b = IMM ? k0 : b_at(bp, i);
+    if constexpr (OP >= GM_OP_EQ) return compare<OP, T>(a, b, fa, fb, k1, k2, k3);
+    else return math<OP, T>(a, b, fa, fb, k1, k2, k3);
+  });
+}
+
+template <typename T, bool IMM, int V, typename S>
+__device__ __forceinline__ void exec_binary(const GmInstr& in, S (&acc)[V], const S* __restrict__ bp) {
   switch (in.op) {
-    case GM_OP_ADD:  GM_MATH(w_add(x, y)) break;
-    case GM_OP_SUB:  GM_MATH(w_sub(x, y)) break;
-    case GM_OP_RSUB: GM_MATH(w_sub(y, x)) break;
-    case GM_OP_MUL:  GM_MATH(w_mul(x, y)) break;
-    case GM_OP_DIV:  GM_MATH(w_div(x, y)) break;
-    case GM_OP_RDIV: GM_MATH(w_div(y, x)) break;
-    case GM_OP_POW:  GM_MATH(w_pow(x, y)) break;
-    case GM_OP_RPOW: GM_MATH(w_pow(y, x)) break;
-    case GM_OP_EQ: GM_CMP(x == y) break;
-    case GM_OP_NE: GM_CMP(x != y) break;
-    case GM_OP_GT: GM_CMP(x > y) break;
-    case GM_OP_GE: GM_CMP(x >= y) break;
-    case GM_OP_LT: GM_CMP(x < y) break;
-    case GM_OP_LE: GM_CMP(x <= y) break;
+    case GM_OP_ADD:  binary_loop<GM_OP_ADD, T, IMM>(in, acc, bp); break;
+    case GM_OP_SUB:  binary_loop<GM_OP_SUB, T, IMM>(in, acc, bp); break;
+    case GM_OP_RSUB: binary_loop<GM_OP_RSUB, T, IMM>(in, acc, bp); break;
+    case GM_OP_MUL:  binary_loop<GM_OP_MUL, T, IMM>(in, acc, bp); break;
+    case GM_OP_DIV:  binary_loop<GM_OP_DIV, T, IMM>(in, acc, bp); break;
+    case GM_OP_RDIV: binary_loop<GM_OP_RDIV, T, IMM>(in, acc, bp); break;
+    case GM_OP_POW:  binary_loop<GM_OP_POW, T, IMM>(in, acc, bp); break;
+    case GM_OP_RPOW: binary_loop<GM_OP_RPOW, T, IMM>(in, acc, bp); break;
+    case GM_OP_EQ: binary_loop<GM_OP_EQ, T, IMM>(in, acc, bp); break;
+    case GM_OP_NE: binary_loop<GM_OP_NE, T, IMM>(in, acc, bp); break;
+    case GM_OP_GT: binary_loop<GM_OP_GT, T, IMM>(in, acc, bp); break;
+    case GM_OP_GE: binary_loop<GM_OP_GE, T, IMM>(in, acc, bp); break;
+    case GM_OP_LT: binary_loop<GM_OP_LT, T, IMM>(in, acc, bp); break;
+    case GM_OP_LE: binary_loop<GM_OP_LE, T, IMM>(in, acc, bp); break;
     default: break;
   }
-#undef GM_B
-#undef GM_MATH
-#undef GM_CMP
 }
 
 // Unary instructions that look at acc (class A) in the compare class T.
-template <typename T, typename A, int W, int V, typename S>
+template <typename T, typename A, int V, typename S>
 __device__ __forceinline__ void exec_unary(const GmInstr& in, S (&acc)[V], const DevTable* __restrict__ tabs) {
   const bool fa = in.flags & GM_F_ND_A;
-  const A nda = Raw<A>::get(in.k[1]);
+  const uint64_t k0 = in.k[0], k1 = in.k[1], k2 = in.k[2], k3 = in.k[3], k4 = in.k[4], k5 = in.k[5];
   switch (in.op) {
-    case GM_OP_EXP: case GM_OP_LOG: case GM_OP_LOG10: {
-      if constexpr (sizeof(T) <= W && IsFloat<T>::value && std::is_same<T, A>::value) {
-        const T fill = Raw<T>::get(in.k[3]);
-#pragma unroll
-        for (int i = 0; i < V; ++i) {
-          const T x = Raw<T>::get(acc[i]);
-          const T r = in.op == GM_OP_EXP ? w_exp(x) : in.op == GM_OP_LOG ? w_log(x) : w_log10(x);
-          const bool bad = (fa && x == nda) || !finite_(r);
-          acc[i] = (S)Raw<T>::put(bad ? fill : r);
-        }
+    case GM_OP_EXP: case GM_OP_LOG: case GM_OP_LOG10:
+      if constexpr (IsFloat<T>::value && std::is_same<T, A>::value) {
+        if (in.op == GM_OP_EXP) each(acc, [&](S a, int) { return transcend<GM_OP_EXP, T>(a, fa, k1, k3); });
+        else if (in.op == GM_OP_LOG) each(acc, [&](S a, int) { return transcend<GM_OP_LOG, T>(a, fa, k1, k3); });
+        else each(acc, [&](S a, int) { return transcend<GM_OP_LOG10, T>(a, fa, k1, k3); });
       }
       break;
-    }
     case GM_OP_MASK: {
-      // raster/misc.py:208-222: data -> value (k0), no data -> fill (k3)
-      const T nd = Raw<T>::get(in.k[1]), tol = Raw<T>::get(in.k[4]);
       const bool has = in.flags & GM_F_ND_T, cl = in.flags & GM_F_CLOSE, fin = in.flags & GM_F_ND_FINITE;
-      const S val = (S)in.k[0], fill = (S)in.k[3];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const T x = astype<T>(Raw<A>::get(acc[i]));
-        const bool nod = has && (cl ? close_(x, nd, tol, fin) : (x == nd));
-        acc[i] = nod ? fill : val;
-      }
+      each(acc, [&](S a, int) { return mask<T, A>(a, has, cl, fin, k0, k1, k3, k4); });
       break;
     }
-    case GM_OP_MASKBELOW: {
-      // raster/misc.py:249-250 (k0 threshold in class T, k5 sentinel as slot bits)
-      const T thr = Raw<T>::get(in.k[0]);
-      const S nd = (S)in.k[5];
-#pragma unroll
-      for (int i = 0; i < V; ++i) acc[i] = (astype<T>(Raw<A>::get(acc[i])) < thr) ? nd : acc[i];
+    case GM_OP_MASKBELOW:
+      each(acc, [&](S a, int) { return mask_below<T, A>(a, k0, k5); });
       break;
-    }
-    case GM_OP_STEP: {
-      // raster/misc.py:316-326 (k0 location in class T; k1 sentinel in class A;
-      // k2/k3/k4 left/at/right as slot bits)
-      const T loc = Raw<T>::get(in.k[0]);
-      const S left = (S)in.k[2], at = (S)in.k[3], right = (S)in.k[4];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const A raw = Raw<A>::get(acc[i]);
-        const T x = astype<T>(raw);
-        S r = acc[i];
-        r = x < loc ? left : r;
-        r = x == loc ? at : r;
-        r = x > loc ? right : r;
-        acc[i] = (fa && raw == nda) ? acc[i] : r;
-      }
+    case GM_OP_STEP:
+      each(acc, [&](S a, int) { return step<T, A>(a, fa, k0, k1, k2, k3, k4); });
       break;
-    }
     case GM_OP_CLASSIFY: {
-      // np.digitize(values, bins, right) (raster/misc.py:396), bins ascending
       const DevTable& t = tabs[in.aux];
       const bool right = in.flags & GM_F_RIGHT;
-      const S fill = (S)in.k[3];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const A raw = Raw<A>::get(acc[i]);
-        const T x = astype<T>(raw);
-        int lo = 0, hi = t.n;
-        if (x != x) lo = t.n;  // NaN sorts last
-        else
-          while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            const T e = Raw<T>::get((uint64_t)t.keys[mid]);
-            const bool go = right ? (e < x) : (e <= x);
-            if (go) lo = mid + 1; else hi = mid;
-          }
-        acc[i] = (fa && raw == nda) ? fill : (S)(uint32_t)lo;
-      }
+      each(acc, [&](S a, int) { return classify<T, A>(a, fa, right, t.keys, t.n, k1, k3); });
       break;
     }
     default: break;
   }
 }
 
-// FillNoData step (raster/elemwise.py:752-755): acc = isdata(b) ? astype(b) : acc; the
-// sentinel test (np.isclose for floats) runs in class T = class of b; To = class of acc.
-// With aux != 0 the step REDUCES instead of replacing (reduce_rasters, raster/reduction.py:38-119):
-// acc = isdata(b) ? red(acc, astype(b)) : acc with red = max / min / sum / product in a float
-// class where NaN marks "no value yet" (NaN cells of b are skipped as np.nan* functions do), or
-// count (acc += 1 in any class).
-template <typename To> __device__ __forceinline__ To overlay_reduce(int kind, To a, To b) {
-  if (kind == GM_RED_COUNT) return (To)(a + (To)1);
-  if constexpr (IsFloat<To>::value) {
-    if (b != b) return a;
-    if (a != a) return b;
-    switch (kind) {
-      case GM_RED_MAX: return b > a ? b : a;
-      case GM_RED_MIN: return b < a ? b : a;
-      case GM_RED_SUM: return a + b;
-      default: return a * b;
-    }
-  }
-  return b;
-}
-
-template <typename T, typename To, int V, typename S>
-__device__ __forceinline__ void exec_overlay(const GmInstr& in, S (&acc)[V], const S* __restrict__ bp) {
-  const T nd = Raw<T>::get(in.k[2]), tol = Raw<T>::get(in.k[4]);
-  const bool has = in.flags & GM_F_ND_T, cl = in.flags & GM_F_CLOSE, fin = in.flags & GM_F_ND_FINITE;
-  const int kind = (int)in.aux;
-  const int tid = threadIdx.x;
-#pragma unroll
-  for (int i = 0; i < V; ++i) {
-    const T y = Raw<T>::get(bp[i * THREADS + tid]);
-    const bool nod = has && (cl ? close_(y, nd, tol, fin) : (y == nd));
-    const To fresh = astype<To>(y);
-    const To next = kind == GM_RED_REPLACE ? fresh : overlay_reduce<To>(kind, Raw<To>::get(acc[i]), fresh);
-    acc[i] = nod ? acc[i] : (S)Raw<To>::put(next);
-  }
-}
-
-// Reclassify (raster/misc.py:505-514): mapped -> target, else fill (select) or
-// astype(values).  With GM_F_ND_T only the "result has data" boolean is produced
-// (enough when the result merely masks another raster), which keeps the whole
-// program in 32-bit slots.  The source sentinel (k1, GM_F_ND_A) maps onto the fill.
-template <typename A, bool DENSE, bool ND_ONLY, int W, int V, typename S>
+template <typename A, bool DENSE, bool ND_ONLY, int V, typename S>
 __device__ __forceinline__ void exec_reclass(const GmInstr& in, S (&acc)[V], const DevTable& t) {
-  const bool select = in.flags & GM_F_SELECT, fa = in.flags & GM_F_ND_A;
-  const int64_t nd_key = (int64_t)in.k[1];
-  const S fill = (S)in.k[3];
-  // result for [miss, mapped, mapped-onto-fill] when only the data flag is wanted
-  const unsigned has_data_lut = (select ? 0u : 1u) | 2u;
-#pragma unroll
-  for (int i = 0; i < V; ++i) {
-    const int64_t key = (int64_t)Raw<A>::get(acc[i]);
-    int found = 0;  // 0 miss, 1 mapped, 2 mapped onto the fill value
-    uint64_t val = in.k[3];
-    if constexpr (DENSE) {
-      const uint64_t idx = (uint64_t)(key - t.base);
-      if (idx < (uint64_t)t.n) {
-        found = t.hit[idx];
-        if constexpr (!ND_ONLY) val = found ? t.vals[idx] : val;
-      }
-    } else {
-      int lo = 0, hi = t.n;
-      while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (t.keys[mid] < key) lo = mid + 1; else hi = mid;
-      }
-      if (lo < t.n && t.keys[lo] == key) {
-        found = t.hit ? t.hit[lo] : 1;
-        if constexpr (!ND_ONLY) val = t.vals[lo];
-      }
-    }
-    found = (fa && key == nd_key) ? 2 : found;
-    if constexpr (ND_ONLY) {
-      acc[i] = (S)((has_data_lut >> found) & 1u);
-    } else if constexpr (W == 8) {
-      // unmapped cells keep astype(values): class A -> the (64-bit) target class
-      S keep;
-      if (in.cls_out == GM_C_F64) keep = (S)Raw<double>::put((double)Raw<A>::get(acc[i]));
-      else keep = (S)Raw<int64_t>::put((int64_t)Raw<A>::get(acc[i]));
-      acc[i] = found ? (S)val : (select ? fill : keep);
-    }
-  }
+  const bool select = in.flags & GM_F_SELECT, fa = in.flags & GM_F_ND_A, out_f64 = in.cls_out == GM_C_F64;
+  const uint64_t k1 = in.k[1], k3 = in.k[3];
+  each(acc, [&](S a, int) {
+    return reclass<A, DENSE, ND_ONLY>(a, select, fa, out_f64, t.keys, t.vals, t.hit, t.n, t.base, k1, k3);
+  });
 }
 
-template <typename A, int W, int V, typename S>
+template <typename A, int V, typename S>
 __device__ __forceinline__ void dispatch_reclass(const GmInstr& in, S (&acc)[V], const DevTable& t) {
   const bool nd_only = in.flags & GM_F_ND_T;
   if (t.kind == GM_TABLE_DENSE) {
-    if (nd_only) exec_reclass<A, true, true, W, V, S>(in, acc, t);
-    else exec_reclass<A, true, false, W, V, S>(in, acc, t);
+    if (nd_only) exec_reclass<A, true, true>(in, acc, t);
+    else exec_reclass<A, true, false>(in, acc, t);
   } else {
-    if (nd_only) exec_reclass<A, false, true, W, V, S>(in, acc, t);
-    else exec_reclass<A, false, false, W, V, S>(in, acc, t);
+    if (nd_only) exec_reclass<A, false, true>(in, acc, t);
+    else exec_reclass<A, false, false>(in, acc, t);
   }
 }
 
@@ -616,10 +330,10 @@ eval_kernel(const __grid_constant__ EvalParams p) {
   auto issue_loads = [&](int64_t tile, int stage) {
     // one thread: arm the barrier with the byte count, then one bulk copy per input
     uint32_t total = 0;
-    for (int k = 0; k < p.n_inputs; ++k) total += (uint32_t)TILE * dsize(p.in_dtype[k]);
+    for (int k = 0; k < p.n_inputs; ++k) total += (uint32_t)TILE * dtype_size(p.in_dtype[k]);
     mbar_expect_tx(&bars[stage], total);
     for (int k = 0; k < p.n_inputs; ++k) {
-      const uint32_t bytes = (uint32_t)TILE * dsize(p.in_dtype[k]);
+      const uint32_t bytes = (uint32_t)TILE * dtype_size(p.in_dtype[k]);
       bulk_load(in_stage_ptr(stage) + p.in_off[k],
                 reinterpret_cast<const unsigned char*>(p.in[k]) + (size_t)tile * bytes, bytes, &bars[stage]);
     }
@@ -642,7 +356,7 @@ eval_kernel(const __grid_constant__ EvalParams p) {
     } else {
       // ragged last tile: plain guarded copies into the stage
       for (int k = 0; k < p.n_inputs; ++k) {
-        const int sz = dsize(p.in_dtype[k]);
+        const int sz = dtype_size(p.in_dtype[k]);
         const unsigned char* g = reinterpret_cast<const unsigned char*>(p.in[k]) + (size_t)base * sz;
         unsigned char* d = in_stage_ptr(stage) + p.in_off[k];
         const int64_t valid = (n - base) * sz;
@@ -716,64 +430,61 @@ eval_kernel(const __grid_constant__ EvalParams p) {
         case GM_OP_ISNODATA: {
           const bool fa = in.flags & GM_F_ND_A;
           const bool want_nodata = op == GM_OP_ISNODATA;
+          const uint64_t k1 = in.k[1];
           with_class<W>(in.cls_a, [&](auto tag) {
             typedef decltype(tag) A;
-            const A nd = Raw<A>::get(in.k[1]);
-#pragma unroll
-            for (int i = 0; i < V; ++i) {
-              const bool is_nd = fa && Raw<A>::get(acc[i]) == nd;
-              acc[i] = (S)((is_nd == want_nodata) ? 1u : 0u);
-            }
+            each(acc, [&](S a, int) { return is_data<A>(a, fa, want_nodata, k1); });
           });
           break;
         }
         case GM_OP_CLIP: {
-          const S nd = (S)in.k[1];
+          const uint64_t k1 = in.k[1], k2 = in.k[2];
           if (in.flags & GM_F_B_BOOL) {
-#pragma unroll
-            for (int i = 0; i < V; ++i) acc[i] = ((uint32_t)bp[i * THREADS + tid] == 0u) ? nd : acc[i];
+            each(acc, [&](S a, int i) { return clip<int32_t, 1>(a, b_at(bp, i), k1, k2); });
           } else if (in.flags & GM_F_ND_B) {
             with_class<W>(in.cls_b, [&](auto tag) {
               typedef decltype(tag) B;
-              const B ndb = Raw<B>::get(in.k[2]);
-#pragma unroll
-              for (int i = 0; i < V; ++i) acc[i] = (Raw<B>::get(bp[i * THREADS + tid]) == ndb) ? nd : acc[i];
+              each(acc, [&](S a, int i) { return clip<B, 2>(a, b_at(bp, i), k1, k2); });
             });
           }
           break;
         }
         case GM_OP_AND: case GM_OP_OR: case GM_OP_XOR: case GM_OP_NOT: {
           const bool imm = in.src_kind == GM_SRC_IMM;
-          const bool yimm = in.k[0] != 0;
-#pragma unroll
-          for (int i = 0; i < V; ++i) {
-            const bool x = (uint32_t)acc[i] != 0u;
-            const bool y = op == GM_OP_NOT ? false : (imm ? yimm : ((uint32_t)bp[i * THREADS + tid] != 0u));
-            const bool r = op == GM_OP_AND ? (x && y) : op == GM_OP_OR ? (x || y) : op == GM_OP_XOR ? (x != y) : !x;
-            acc[i] = (S)(r ? 1u : 0u);
-          }
+          const uint64_t yimm = in.k[0] != 0;
+          auto y = [&](int i) { return imm ? yimm : b_at(bp, i); };
+          if (op == GM_OP_AND) each(acc, [&](S a, int i) { return logic<GM_OP_AND>(a, y(i)); });
+          else if (op == GM_OP_OR) each(acc, [&](S a, int i) { return logic<GM_OP_OR>(a, y(i)); });
+          else if (op == GM_OP_XOR) each(acc, [&](S a, int i) { return logic<GM_OP_XOR>(a, y(i)); });
+          else each(acc, [&](S a, int) { return logic<GM_OP_NOT>(a, 0); });
           break;
         }
         case GM_OP_RECLASS:
-          if (in.cls_a == GM_C_I32) dispatch_reclass<int32_t, W, V, S>(in, acc, tabs[in.aux]);
-          else if constexpr (W == 8) dispatch_reclass<int64_t, W, V, S>(in, acc, tabs[in.aux]);
+          if (in.cls_a == GM_C_I32) dispatch_reclass<int32_t>(in, acc, tabs[in.aux]);
+          else if constexpr (W == 8) dispatch_reclass<int64_t>(in, acc, tabs[in.aux]);
           break;
-        case GM_OP_OVERLAY:
+        case GM_OP_OVERLAY: {
+          const bool has = in.flags & GM_F_ND_T, cl = in.flags & GM_F_CLOSE, fin = in.flags & GM_F_ND_FINITE;
+          const int kind = (int)in.aux;
+          const uint64_t k2 = in.k[2], k4 = in.k[4];
           with_class<W>(in.cls, [&](auto tag) {
             typedef decltype(tag) T;
             with_class<W>(in.cls_out, [&](auto otag) {
               typedef decltype(otag) To;
-              exec_overlay<T, To, V, S>(in, acc, bp);
+              each(acc, [&](S a, int i) {
+                return overlay<T, To>(a, b_at(bp, i), has, cl, fin, kind, k2, k4);
+              });
             });
           });
           break;
+        }
         case GM_OP_EXP: case GM_OP_LOG: case GM_OP_LOG10:
         case GM_OP_MASK: case GM_OP_MASKBELOW: case GM_OP_STEP: case GM_OP_CLASSIFY:
           with_class<W>(in.cls, [&](auto tag) {
             typedef decltype(tag) T;
             with_class<W>(in.cls_a, [&](auto atag) {
               typedef decltype(atag) A;
-              exec_unary<T, A, W, V, S>(in, acc, tabs);
+              exec_unary<T, A>(in, acc, tabs);
             });
           });
           break;
@@ -781,8 +492,8 @@ eval_kernel(const __grid_constant__ EvalParams p) {
           const bool imm = in.src_kind == GM_SRC_IMM;
           with_class<W>(in.cls, [&](auto tag) {
             typedef decltype(tag) T;
-            if (imm) exec_binary<T, V, true, S>(in, acc, bp);
-            else exec_binary<T, V, false, S>(in, acc, bp);
+            if (imm) exec_binary<T, true>(in, acc, bp);
+            else exec_binary<T, false>(in, acc, bp);
           });
           break;
         }
@@ -795,7 +506,7 @@ eval_kernel(const __grid_constant__ EvalParams p) {
     if (full) {
       if (tid == 0) {
         for (int k = 0; k < p.n_outputs; ++k) {
-          const uint32_t bytes = (uint32_t)TILE * dsize(p.out_dtype[k]);
+          const uint32_t bytes = (uint32_t)TILE * dtype_size(p.out_dtype[k]);
           bulk_store(reinterpret_cast<unsigned char*>(p.out[k]) + (size_t)tile * bytes,
                      out_stage_ptr(stage) + p.out_off[k], bytes);
         }
@@ -803,7 +514,7 @@ eval_kernel(const __grid_constant__ EvalParams p) {
       }
     } else {
       for (int k = 0; k < p.n_outputs; ++k) {
-        const int sz = dsize(p.out_dtype[k]);
+        const int sz = dtype_size(p.out_dtype[k]);
         unsigned char* g = reinterpret_cast<unsigned char*>(p.out[k]) + (size_t)base * sz;
         const unsigned char* s = out_stage_ptr(stage) + p.out_off[k];
         const int64_t valid = (n - base) * sz;
@@ -854,11 +565,14 @@ static int validate(const GmProgram* prog, const GmArray* inputs) {
     if (direct_b) {
       // a staged input is only a valid b operand when its storage already is a slot
       const int dt = inputs[in.src].dtype;
-      if (dsize(dt) != prog->word || natural_class(dt) != in.cls_b)
+      if (dtype_size(dt) != prog->word || natural_class(dt) != in.cls_b)
         return fail("gm_eval_program: input used as operand without conversion");
     }
     if (is_binary(in.op) && (in.cls_a != in.cls || (in.src_kind != GM_SRC_NONE && in.cls_b != in.cls)))
       return fail("gm_eval_program: arithmetic operands must already hold the compute class");
+    if (in.op == GM_OP_OVERLAY && in.aux != GM_RED_REPLACE && in.aux != GM_RED_COUNT &&
+        in.cls_out != GM_C_F32 && in.cls_out != GM_C_F64)
+      return fail("gm_eval_program: overlay max / min / sum / product need a float accumulator");
   }
   return 0;
 }
@@ -875,11 +589,11 @@ static int launch_eval(EvalParams& p, const GmProgram* prog, size_t table_bytes,
   int in_stage = 0, out_stage = 0;
   for (int k = 0; k < prog->n_inputs; ++k) {
     p.in_off[k] = in_stage;
-    in_stage += (tile * dsize(p.in_dtype[k]) + 127) / 128 * 128;
+    in_stage += (tile * dtype_size(p.in_dtype[k]) + 127) / 128 * 128;
   }
   for (int k = 0; k < prog->n_outputs; ++k) {
     p.out_off[k] = out_stage;
-    out_stage += (tile * dsize(p.out_dtype[k]) + 127) / 128 * 128;
+    out_stage += (tile * dtype_size(p.out_dtype[k]) + 127) / 128 * 128;
   }
   p.in_stage_bytes = in_stage;
   p.out_stage_bytes = out_stage;
@@ -969,6 +683,7 @@ extern "C" int gm_eval_program(const GmProgram* prog, const GmArray* inputs, GmA
 
   for (int i = 0; i < prog->n_inputs && !rc; ++i) {
     if (array_count(inputs[i]) != n_pixels) { rc = fail("gm_eval_program: input size mismatch"); break; }
+    if (!dtype_size(inputs[i].dtype)) { rc = fail("gm_eval_program: bad input dtype"); break; }
     if (((uintptr_t)inputs[i].data & 15u) && inputs[i].space == GM_DEVICE) {
       rc = fail("gm_eval_program: device input not 16-byte aligned"); break;
     }
@@ -978,6 +693,7 @@ extern "C" int gm_eval_program(const GmProgram* prog, const GmArray* inputs, GmA
   }
   for (int i = 0; i < prog->n_outputs && !rc; ++i) {
     if (array_count(outputs[i]) != n_pixels) { rc = fail("gm_eval_program: output size mismatch"); break; }
+    if (!dtype_size(outputs[i].dtype)) { rc = fail("gm_eval_program: bad output dtype"); break; }
     if (((uintptr_t)outputs[i].data & 15u) && outputs[i].space == GM_DEVICE) {
       rc = fail("gm_eval_program: device output not 16-byte aligned"); break;
     }

@@ -1,9 +1,10 @@
 // Specialising back end of the fused evaluator.
 //
 // gm_eval_program hands a validated GmProgram to jit_launch().  The program is
-// translated ONCE into a straight-line CUDA kernel (gm_jit_prelude.cuh holds one
-// device function per bytecode instruction; classes and flags become template
-// arguments, constants literals, small lookup tables __device__ arrays), compiled
+// translated ONCE into a straight-line CUDA kernel that calls, per instruction, the
+// device function of gm_eval_ops.cuh that the interpreter runs too (classes become
+// template arguments, flags and constants literals, small lookup tables __device__
+// arrays; gm_jit_prelude.cuh adds the memory access of generated code), compiled
 // for sm_100a with NVRTC (-fmad=false, IEEE division) and cached by a hash of the
 // program.  The generated kernel keeps every pixel in registers:
 //
@@ -16,7 +17,7 @@
 //     live in shared memory (see JitLayout).
 //
 // The interpreter in gm_eval.cu stays the zero-latency path for small rasters; the
-// two are checked against each other and against the oracle by the parity tests.
+// parity tests check the two against each other and against the oracle.
 #include "gm_common.cuh"
 #include "gm_jit.h"
 #include <dlfcn.h>
@@ -102,6 +103,7 @@ static std::string hex(uint64_t v) {
 }
 static std::string num(long long v) { return std::to_string(v); }
 static const char* tf(bool b) { return b ? "true" : "false"; }
+static std::string lit(int v) { return "Lit<" + num(v) + ">()"; }   // Lit of the prelude
 
 // Where each lookup table lives.  A baked table's contents are part of the module (and of the
 // cache key): a dense ND_ONLY Reclassify table of at most 64 entries as two 32-bit literal words
@@ -175,8 +177,8 @@ static std::string operand_b(const GmInstr& in, int pc) {
 
 static std::string convert_expr(const std::string& x, int from, int to, bool nanify, const std::string& k, int word) {
   if (from == to || !class_fits(from, word) || !class_fits(to, word)) return x;
-  return std::string("cvt<") + class_type(from) + ", " + class_type(to) + ", " + tf(nanify) + ">(" + x +
-         ", " + k + ")";
+  return std::string("cvt<") + class_type(from) + ", " + class_type(to) + ">(" + x + ", " + tf(nanify) + ", " +
+         k + ")";
 }
 
 static std::string table_args(const GmProgram* prog, int t) {
@@ -233,8 +235,8 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in, co
     case GM_OP_ISDATA:
     case GM_OP_ISNODATA:
       if (class_fits(in.cls_a, word))
-        s = std::string("acc = is_data<") + class_type(in.cls_a) + ", " + tf(fa) + ", " +
-            tf(in.op == GM_OP_ISNODATA) + ">(acc, " + kref(pc, 1) + ");";
+        s = std::string("acc = is_data<") + class_type(in.cls_a) + ">(acc, " + tf(fa) + ", " +
+            tf(in.op == GM_OP_ISNODATA) + ", " + kref(pc, 1) + ");";
       break;
     case GM_OP_CLIP: {
       int mode = (in.flags & GM_F_B_BOOL) ? 1 : (fb ? 2 : 0);
@@ -258,32 +260,32 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in, co
         const unsigned lut = ((in.flags & GM_F_SELECT) ? 0u : 1u) | 2u;   // as in reclass
         uint32_t w[2] = {0, 0};
         for (int i = 0; i < g.n; ++i) w[i / 32] |= ((lut >> g.hit[i]) & 1u) << (i % 32);
-        s = std::string("acc = reclass_bits<") + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ">(acc, " +
+        s = std::string("acc = reclass_bits(acc, ") + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ", " +
             num(w[0]) + "u, " + num(w[1]) + "u, " + num(g.n) + "u, " + num(g.base) + ", " + kref(pc, 1) + ");";
         break;
       }
       s = std::string("acc = reclass<") + A + ", " + tf(g.kind == GM_TABLE_DENSE) + ", " +
-          tf(in.flags & GM_F_ND_T) + ", " + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ", " +
-          tf(in.cls_out == GM_C_F64) + ">(acc, " + table_args(prog, in.aux) + ", " + num(g.n) + ", " +
+          tf(in.flags & GM_F_ND_T) + ">(acc, " + tf(in.flags & GM_F_SELECT) + ", " + tf(fa) + ", " +
+          tf(in.cls_out == GM_C_F64) + ", " + table_args(prog, in.aux) + ", " + num(g.n) + ", " +
           num(g.base) + "LL, " + kref(pc, 1) + ", " + kref(pc, 3) + ");";
       break;
     }
     case GM_OP_OVERLAY:
       if (class_fits(in.cls, word) && class_fits(in.cls_out, word))
-        s = std::string("acc = overlay<") + class_type(in.cls) + ", " + class_type(in.cls_out) + ", " +
-            tf(in.flags & GM_F_ND_T) + ", " + tf(in.flags & GM_F_CLOSE) + ", " + tf(in.flags & GM_F_ND_FINITE) +
-            ", " + num((int)in.aux) + ">(acc, " + b + ", " + kref(pc, 2) + ", " + kref(pc, 4) + ");";
+        s = std::string("acc = overlay<") + class_type(in.cls) + ", " + class_type(in.cls_out) + ">(acc, " + b +
+            ", " + lit((in.flags & GM_F_ND_T) != 0) + ", " + lit((in.flags & GM_F_CLOSE) != 0) + ", " +
+            lit((in.flags & GM_F_ND_FINITE) != 0) + ", " + lit((int)in.aux) + ", " + kref(pc, 2) + ", " + kref(pc, 4) + ");";
       break;
     case GM_OP_EXP: case GM_OP_LOG: case GM_OP_LOG10:
       if (class_fits(in.cls, word) && class_is_float(in.cls) && in.cls == in.cls_a)
-        s = "acc = transcend<" + num(in.op) + ", " + class_type(in.cls) + ", " + tf(fa) + ">(acc, " +
+        s = "acc = transcend<" + num(in.op) + ", " + class_type(in.cls) + ">(acc, " + tf(fa) + ", " +
             kref(pc, 1) + ", " + kref(pc, 3) + ");";
       break;
     case GM_OP_MASK:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
-        s = std::string("acc = mask<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ", " +
-            tf(in.flags & GM_F_ND_T) + ", " + tf(in.flags & GM_F_CLOSE) + ", " + tf(in.flags & GM_F_ND_FINITE) +
-            ">(acc, " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 3) + ", " + kref(pc, 4) + ");";
+        s = std::string("acc = mask<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ">(acc, " +
+            lit((in.flags & GM_F_ND_T) != 0) + ", " + lit((in.flags & GM_F_CLOSE) != 0) + ", " + lit((in.flags & GM_F_ND_FINITE) != 0) +
+            ", " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 3) + ", " + kref(pc, 4) + ");";
       break;
     case GM_OP_MASKBELOW:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
@@ -292,14 +294,14 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in, co
       break;
     case GM_OP_STEP:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
-        call = std::string("step<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ", " + tf(fa) +
-               ">(acc, " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 2) + ", " + kref(pc, 3) + ", " +
+        call = std::string("step<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ">(acc, " + tf(fa) +
+               ", " + kref(pc, 0) + ", " + kref(pc, 1) + ", " + kref(pc, 2) + ", " + kref(pc, 3) + ", " +
                kref(pc, 4) + arm + ")";
       break;
     case GM_OP_CLASSIFY:
       if (class_fits(in.cls, word) && class_fits(in.cls_a, word))
-        s = std::string("acc = classify<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ", " + tf(fa) +
-            ", " + tf(in.flags & GM_F_RIGHT) + ">(acc, t" + num(in.aux) + "k, " + num(prog->tables[in.aux].n) +
+        s = std::string("acc = classify<") + class_type(in.cls) + ", " + class_type(in.cls_a) + ">(acc, " +
+            tf(fa) + ", " + tf(in.flags & GM_F_RIGHT) + ", t" + num(in.aux) + "k, " + num(prog->tables[in.aux].n) +
             ", " + kref(pc, 1) + ", " + kref(pc, 3) + ");";
       break;
     default: {  // binary arithmetic / comparison
@@ -307,13 +309,13 @@ static std::string emit_instruction(const GmProgram* prog, const GmInstr& in, co
       const bool imm = in.src_kind == GM_SRC_IMM;
       const bool is_cmp = in.op >= GM_OP_EQ && in.op <= GM_OP_LE;
       s = std::string("acc = ") + (is_cmp ? "compare<" : "math<") + num(in.op) + ", " + class_type(in.cls) +
-          ", " + tf(fa) + ", " + tf(fb && !imm) + ">(acc, " + b + ", " + kref(pc, 1) + ", " + kref(pc, 2) +
+          ">(acc, " + b + ", " + tf(fa) + ", " + tf(fb && !imm) + ", " + kref(pc, 1) + ", " + kref(pc, 2) +
           ", " + kref(pc, 3) + ");";
       break;
     }
   }
   if (!call.empty())
-    s = fold ? std::string("acc = data_flag<") + tf(fold->op == GM_OP_ISNODATA) + ">(" + call + ");"
+    s = fold ? "acc = data_flag<S>(" + call + ", " + tf(fold->op == GM_OP_ISNODATA) + ");"
              : "acc = " + call + ";";
   return s;
 }

@@ -17,7 +17,7 @@ from ..utils import get_dtype_max, get_uint_dtype, get_int_dtype
 C_I32, C_I64, C_F32, C_F64 = 0, 1, 2, 3
 _WIDE = (C_I64, C_F64)
 
-# GmOp (order matters: it is the enum in include/geokernels.h)
+# GmOp (order matters: it is the enum in include/gm_bytecode.h)
 _OPS = [
     "LOAD", "ST", "OUT", "CVT", "ADD", "SUB", "RSUB", "MUL", "DIV", "RDIV", "POW", "RPOW",
     "EXP", "LOG", "LOG10", "EQ", "NE", "GT", "GE", "LT", "LE", "AND", "OR", "XOR", "NOT",

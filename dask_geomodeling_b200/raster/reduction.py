@@ -4,7 +4,7 @@ Drop-in for the reference's raster/reduction.py: ``reduce_rasters`` (:38-119) an
 block (:215-231).  The reference stacks the rasters into an (n, t, y, x) float array with NaN for
 'no data' and calls NumPy's nan-functions along the first axis; here the rasters are the inputs
 of ONE evaluator program that keeps the running result of a pixel in a register (OVERLAY steps
-with a reduction kind, include/geokernels.h) -- one pass over the inputs, no stack.  Inside a
+with a reduction kind, include/gm_bytecode.h) -- one pass over the inputs, no stack.  Inside a
 view the program is fused with the element-wise blocks around it (core/fusion.py).
 
 Statistics on the CUDA path: last, first, count, max, min (any dtype: exact in the float dtype
