@@ -11,8 +11,10 @@
 //   * a thread owns groups of V = 16 / (widest element) consecutive pixels, so the
 //     widest raster moves as 128-bit accesses and every warp access of every raster
 //     is one fully used contiguous segment (no shared-memory staging needed);
-//   * U groups per thread are loaded before the first is evaluated (U*V = 16 pixels,
-//     >= 96 B in flight per thread on cfg2), streaming cache hints on both sides;
+//   * U groups per thread make a chunk (U*V = 16 pixels, 96 B per thread on cfg2), loaded before
+//     it is evaluated, streaming cache hints on both sides; where two chunks of input fit the
+//     register budget (kTwoSetWords), a block walks K consecutive chunks in two register sets and
+//     issues the loads of chunk c + 1 before it evaluates chunk c;
 //   * a small dense Reclassify table is two 32-bit literal words, other baked lookup tables
 //     live in shared memory (see JitLayout).
 //
@@ -110,12 +112,25 @@ static std::string lit(int v) { return "Lit<" + num(v) + ">()"; }   // Lit of th
 // (`bits`, reclass_bits), any other baked table in shared memory (`in_smem`).  A table that is not
 // baked is read from global memory through the pointers of the parameter block.
 struct JitLayout {
-  int V, U;
+  int V, U;        // pixels per group, groups per thread and chunk
+  bool two_sets;   // the hot loop prefetches the next chunk into a second register set (see generate)
   bool baked[GM_MAX_TABLES];
   bool in_smem[GM_MAX_TABLES];
   bool bits[GM_MAX_TABLES];
 };
 
+// The two-set hot loop holds two chunks of input in registers: 2 * U * (32-bit words of one group of
+// every input).  It is used while that stays within kTwoSetWords and the program has no tables in
+// shared memory; cfg2 (int16 + float32: 48 words) then compiles to 64 registers without spills, so
+// 4 blocks of 256 stay resident per SM.  Wider programs (cfg1, two float32 inputs: 64 words, 45 -> 77
+// registers and 13.8 -> 21.8 instructions per pixel unbaked; four float32 inputs: 80 -> 154
+// registers; eight float64 inputs spill) keep the single-set loop.
+static const int kTwoSetWords = 48;
+// Chunks per block of the two-set loop, at most: on one B200 at 1000 W (cfg2 chain, bench.py --legs
+// chain, before the warp barrier of the loads was added) 1, 2, 4 and 8 took 0.336, 0.318, 0.291 and
+// 0.297 ms per step, the single-set loop with one chunk per block 0.309 ms.  Fewer on small rasters,
+// so that the grid still fills the resident blocks of every SM (see jit_launch).
+static const int kMaxChunksPerBlock = 4;
 static const int kBakeLimit = 2048;  // table entries baked into the module / held in smem
 static const int kBitsLimit = 64;    // entries of a table held as two 32-bit words
 
@@ -144,11 +159,16 @@ static JitLayout plan_layout(const GmProgram* prog, const int* in_dtype, const i
   L.U = std::max(2, 16 / L.V);
   int total = 0;
   for (int t = 0; t < prog->n_tables; ++t) total += prog->tables[t].n;
+  bool smem_tables = false;
   for (int t = 0; t < GM_MAX_TABLES; ++t) {
     L.baked[t] = t < prog->n_tables && total <= kBakeLimit;
     L.bits[t] = L.baked[t] && bits_table(prog, t);
     L.in_smem[t] = L.baked[t] && !L.bits[t];
+    smem_tables = smem_tables || L.in_smem[t];
   }
+  int words = 0;   // 32-bit words of one group of every input
+  for (int i = 0; i < prog->n_inputs; ++i) words += std::max(1, L.V * dtype_size(in_dtype[i]) / 4);
+  L.two_sets = !smem_tables && 2 * L.U * words <= kTwoSetWords;
   return L;
 }
 
@@ -351,7 +371,7 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
   src += "#define GM_WORD " + num(prog->word) + "\n";
   src += kPrelude;
   src += "\nstruct Params { const void* in[" + num(GM_MAX_INPUTS) + "]; void* out[" + num(GM_MAX_OUTPUTS) +
-         "]; long long n; const int64_t* tk[" + num(GM_MAX_TABLES) + "]; const uint64_t* tv[" +
+         "]; long long n; long long chunks_per_block; const int64_t* tk[" + num(GM_MAX_TABLES) + "]; const uint64_t* tv[" +
          num(GM_MAX_TABLES) + "]; const uint8_t* th[" + num(GM_MAX_TABLES) + "]; unsigned long long k[" +
          num(GM_MAX_INSTR) + "][6]; };\n";
   emit_table_data(src, prog, L);
@@ -446,30 +466,62 @@ static std::string generate(const GmProgram* prog, const int* in_dtype, const in
   src += "  const long long groups = p.n / " + num(V) + ";\n";
   src += "  const long long chunk = 256LL * " + num(U) + ";\n";
   src += "  const long long n_chunks = groups / chunk;\n";
-  // full chunks: U groups per thread, all loads first
-  src += "  for (long long c = blockIdx.x; c < n_chunks; c += gridDim.x) {\n";
-  src += "    const long long g0 = c * chunk + tid;\n";
-  for (int i = 0; i < prog->n_inputs; ++i)
-    src += "    uint32_t a" + num(i) + "[" + num(U) + "][" + num(words(in_dtype[i])) + "];\n";
-  src += "    #pragma unroll\n    for (int u = 0; u < " + num(U) + "; ++u) {\n";
-  for (int i = 0; i < prog->n_inputs; ++i) {
-    const int bytes = V * dtype_size(in_dtype[i]);
-    src += "      load_group<" + num(bytes) + ">(a" + num(i) + "[u], in" + num(i) + " + (g0 + u * 256LL) * " + num(bytes) + ");\n";
+  // full chunks: U groups per thread.  The loads of a chunk are emitted before its evaluation; `set`
+  // selects a register set of the two-set loop (-1: the single set), `g0` is the chunk's first group
+  // of this thread.
+  auto load_set = [&](int set, const std::string& g0, bool fence) {
+    const std::string idx = set < 0 ? "" : "[" + num(set) + "]";
+    std::string t = "      #pragma unroll\n      for (int u = 0; u < " + num(U) + "; ++u) {\n";
+    for (int i = 0; i < prog->n_inputs; ++i) {
+      const int bytes = V * dtype_size(in_dtype[i]);
+      t += "        load_group<" + num(bytes) + ">(a" + num(i) + idx + "[u], in" + num(i) + " + (" + g0 +
+           " + u * 256LL) * " + num(bytes) + ");\n";
+    }
+    return t + (fence ? "        __syncwarp();\n" : "") + "      }\n";
+  };
+  auto eval_set = [&](int set, const std::string& g0) {
+    const std::string idx = set < 0 ? "" : "[" + num(set) + "]";
+    std::string t = "      #pragma unroll\n      for (int u = 0; u < " + num(U) + "; ++u) {\n";
+    for (int i = 0; i < prog->n_outputs; ++i) t += "        uint32_t w" + num(i) + "[" + num(words(out_dtype[i])) + "];\n";
+    t += "        group(p";
+    bool first = false;
+    for (int i = 0; i < prog->n_inputs; ++i) { t += std::string(first ? "" : ", ") + "a" + num(i) + idx + "[u]"; first = false; }
+    for (int i = 0; i < prog->n_outputs; ++i) { t += std::string(first ? "" : ", ") + "w" + num(i); first = false; }
+    t += tab_args + ");\n";
+    for (int i = 0; i < prog->n_outputs; ++i) {
+      const int bytes = V * dtype_size(out_dtype[i]);
+      t += "        store_group<" + num(bytes) + ">(out" + num(i) + " + (" + g0 + " + u * 256LL) * " + num(bytes) +
+           ", w" + num(i) + ");\n";
+    }
+    return t + "      }\n";
+  };
+  if (L.two_sets) {
+    // p.chunks_per_block consecutive chunks per block in two register sets: the loads of chunk c + 1
+    // are issued before chunk c is evaluated.  The warp barrier after each group's loads keeps ptxas
+    // from sinking them into the evaluation (tools/jit_sass.py: without it the unbaked cfg2 kernel
+    // issues them after ~140 of ~350 instructions; one barrier after all of them is not enough).
+    src += "  const long long K = p.chunks_per_block;\n";
+    src += "  for (long long c0 = (long long)blockIdx.x * K; c0 < n_chunks; c0 += (long long)gridDim.x * K) {\n";
+    src += "    const long long c1 = c0 + K < n_chunks ? c0 + K : n_chunks;\n";
+    for (int i = 0; i < prog->n_inputs; ++i)
+      src += "    uint32_t a" + num(i) + "[2][" + num(U) + "][" + num(words(in_dtype[i])) + "];\n";
+    src += load_set(0, "c0 * chunk + tid", true);
+    src += "    for (long long c = c0; c < c1; c += 2) {\n";
+    src += "      if (c + 1 < c1) {\n" + load_set(1, "(c + 1) * chunk + tid", true) + "      }\n";
+    src += eval_set(0, "c * chunk + tid");
+    src += "      if (c + 1 == c1) break;\n";
+    src += "      if (c + 2 < c1) {\n" + load_set(0, "(c + 2) * chunk + tid", true) + "      }\n";
+    src += eval_set(1, "(c + 1) * chunk + tid");
+    src += "    }\n  }\n";
+  } else {
+    // one chunk at a time, all its loads first (ptxas may still sink some of them)
+    src += "  for (long long c = blockIdx.x; c < n_chunks; c += gridDim.x) {\n";
+    src += "    const long long g0 = c * chunk + tid;\n";
+    for (int i = 0; i < prog->n_inputs; ++i)
+      src += "    uint32_t a" + num(i) + "[" + num(U) + "][" + num(words(in_dtype[i])) + "];\n";
+    src += load_set(-1, "g0", false) + eval_set(-1, "g0");
+    src += "  }\n";
   }
-  src += "    }\n";
-  src += "    #pragma unroll\n    for (int u = 0; u < " + num(U) + "; ++u) {\n";
-  for (int i = 0; i < prog->n_outputs; ++i)
-    src += "      uint32_t w" + num(i) + "[" + num(words(out_dtype[i])) + "];\n";
-  src += "      group(p";
-  first = false;
-  for (int i = 0; i < prog->n_inputs; ++i) { src += std::string(first ? "" : ", ") + "a" + num(i) + "[u]"; first = false; }
-  for (int i = 0; i < prog->n_outputs; ++i) { src += std::string(first ? "" : ", ") + "w" + num(i); first = false; }
-  src += tab_args + ");\n";
-  for (int i = 0; i < prog->n_outputs; ++i) {
-    const int bytes = V * dtype_size(out_dtype[i]);
-    src += "      store_group<" + num(bytes) + ">(out" + num(i) + " + (g0 + u * 256LL) * " + num(bytes) + ", w" + num(i) + ");\n";
-  }
-  src += "    }\n  }\n";
   // remaining whole groups: one per thread
   src += "  for (long long g = n_chunks * chunk + (long long)blockIdx.x * 256 + tid; g < groups; g += (long long)gridDim.x * 256) {\n";
   for (int i = 0; i < prog->n_inputs; ++i) {
@@ -674,6 +726,7 @@ struct JitParams {
   const void* in[GM_MAX_INPUTS];
   void* out[GM_MAX_OUTPUTS];
   long long n;
+  long long chunks_per_block;   // of the two-set loop; 1 otherwise
   const int64_t* tk[GM_MAX_TABLES];
   const uint64_t* tv[GM_MAX_TABLES];
   const uint8_t* th[GM_MAX_TABLES];
@@ -743,16 +796,22 @@ int jit_launch(const GmProgram* prog, const void* const* in, const int* in_dtype
     p.tv[t] = (const uint64_t*)tvals[t];
     p.th[t] = (const uint8_t*)thit[t];
   }
-  // One block per chunk of 256 * U groups.  A grid of resident blocks that strides over the chunks
-  // streams slower (tools/chain_ceiling.cu on one B200: 0.29-0.30 ms against 0.263 ms for the cfg2
-  // pattern), so the grid is capped at the resident blocks only when every block first copies its
-  // lookup tables into shared memory, which a block per chunk would repeat ~50 times as often.
-  const int64_t per_block = 256LL * L.U * L.V;
+  // One block per chunk of 256 * U groups, or per K chunks in the two-set loop.  A grid of resident
+  // blocks that strides over the chunks streams slower (tools/chain_ceiling.cu on one B200: 0.29-0.30 ms
+  // against 0.263 ms for the cfg2 pattern), so the grid is capped at the resident blocks only when every
+  // block first copies its lookup tables into shared memory (those programs keep the single-set loop).
+  // K shrinks on small rasters, so that the grid still fills every SM's resident blocks.
+  const int64_t resident = (int64_t)sm_count() * k->blocks_per_sm;
+  const int64_t chunk_px = 256LL * L.U * L.V;
+  p.chunks_per_block = 1;
+  if (L.two_sets)
+    p.chunks_per_block = std::max<int64_t>(1, std::min<int64_t>(kMaxChunksPerBlock, n / chunk_px / resident));
+  const int64_t per_block = chunk_px * p.chunks_per_block;
   int64_t grid = (n + per_block - 1) / per_block;
   bool smem_tables = false;
   for (int t = 0; t < prog->n_tables; ++t) smem_tables = smem_tables || L.in_smem[t];
-  const int64_t cap = smem_tables ? (int64_t)sm_count() * k->blocks_per_sm : (int64_t)INT32_MAX;
-  if (grid > cap) grid = cap;
+  if (smem_tables && grid > resident) grid = resident;
+  if (grid > INT32_MAX) grid = INT32_MAX;
   if (grid < 1) grid = 1;
   void* args[] = {&p};
   cudaError_t e = cudaLaunchKernel((const void*)k->kernel, dim3((unsigned)grid), dim3(256), args, 0, s);

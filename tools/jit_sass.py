@@ -1,11 +1,16 @@
 """What the specialiser makes of a program, without a GPU: generate the fused kernel through
 ``gm_jit_source``, compile it with NVRTC for sm_100a (the options of ``gm_jit.cu``), disassemble it
-with ``cuobjdump -sass`` and report for the hot loop (the loop over full chunks of U groups):
+with ``cuobjdump -sass`` and report for the hot loop (the loop over full chunks of U groups).  In the
+two-set loop (programs whose two chunks of input fit ``kTwoSetWords`` of gm_jit.cu) one pass of it
+evaluates two chunks, c from one register set and c + 1 from the other; the single-set loop evaluates
+one chunk per pass:
 
-  * instructions per pixel (loop instructions / (U * V) pixels),
+  * instructions per pixel (loop instructions / (chunks per pass * U * V) pixels),
   * the opcode mix,
-  * the position of each LDG in the loop, and whether all of them come before the first compare
-    (the first ISETP / FSETP / DSETP: evaluation has started),
+  * for each chunk of the pass (two-set loop: each half, up to its stores), the position of each
+    LDG in it and whether all of them come before its first compare (the first ISETP / FSETP /
+    DSETP: evaluation has started).  In the two-set loop the LDGs of a half load the NEXT chunk, so
+    "all before" means chunk c + 1 is in flight while chunk c is evaluated,
   * registers and spills (ptxas).
 
 The baked variant (``gm_jit_baked_source``) has the program's constants as literals: the kernel
@@ -51,8 +56,16 @@ def shapes():
     big = Node("reclassify", [Leaf(0)], dtype="int64", fillvalue=np.iinfo("i8").max,
                data=[(k, 1) for k in range(0, 400, 2)], select=False)
     big = Node("isdata", [Node("clip", [Leaf(1), big])])
+    def add_chain(n, dtype):
+        t = (np.dtype(dtype), np.finfo(dtype).max)
+        node = Leaf(0)
+        for i in range(1, n):
+            node = Node("add", [node, Leaf(i)], dtype=dtype, fillvalue=t[1])
+        return node, [t] * n
     return {
         "cfg2": (Node("isdata", [st]), [(np.dtype("i2"), 32767), F4]),
+        "add4_f4": add_chain(4, "f4"),
+        "add8_f4": add_chain(8, "f4"),
         "cfg1": (cfg1, [F4, F4]),
         "reclass200": (big, [(np.dtype("i2"), 32767), F4]),
     }
@@ -124,26 +137,45 @@ def hot_loop(instrs):
     raise RuntimeError("no loop found")
 
 
-def report(name, src):
+def analyse(src):
+    """Hot-loop facts of a generated source: a dict with two_sets, pixels (per loop pass), loop (its
+    instructions), halves (per chunk of the pass: LDG positions and the first compare, relative to
+    it), registers, spills (bytes stored and loaded) and the ptxas log."""
     m_v, m_u = re.search(r"p\.n / (\d+);", src), re.search(r"chunk = 256LL \* (\d+);", src)
-    pixels = int(m_v.group(1)) * int(m_u.group(1))
     cubin, log = nvrtc_compile(src)
     instrs, text = sass(cubin)
     loop = hot_loop(instrs)
     ops = [op.split(".")[0] for _, op, _ in loop]
-    ldg = [i for i, op in enumerate(ops) if op == "LDG"]
-    first_cmp = next((i for i, op in enumerate(ops) if op in ("ISETP", "FSETP", "DSETP")), len(ops))
+    two_sets = "p.chunks_per_block" in src
+    stg = [i for i, op in enumerate(ops) if op == "STG"]
+    cut = stg[len(stg) // 2 - 1] + 1          # after the stores of the first chunk
+    halves = []
+    for lo, hi in (((0, cut), (cut, len(ops))) if two_sets else ((0, len(ops)),)):
+        part = ops[lo:hi]
+        halves.append({"ldg": [i for i, op in enumerate(part) if op == "LDG"],
+                       "first_compare": next((i for i, op in enumerate(part) if op in ("ISETP", "FSETP", "DSETP")),
+                                             len(part))})
     regs = re.search(r"Used (\d+) registers", log)
     spill = re.search(r"(\d+) bytes spill stores, (\d+) bytes spill loads", log)
+    return {"two_sets": two_sets, "pixels": (2 if two_sets else 1) * int(m_v.group(1)) * int(m_u.group(1)), "loop": loop, "ops": ops, "halves": halves,
+            "registers": int(regs.group(1)) if regs else None,
+            "spills": int(spill.group(1)) + int(spill.group(2)) if spill else None, "log": log, "text": text}
+
+
+def report(name, src):
+    a = analyse(src)
+    ops, pixels = a["ops"], a["pixels"]
     mix = collections.Counter(ops).most_common()
-    print("{}: {} instructions per {} pixels = {:.2f} per pixel; {} registers, spills {} / {} bytes".format(
-        name, len(loop), pixels, len(loop) / pixels, regs.group(1) if regs else "?",
-        spill.group(1) if spill else "?", spill.group(2) if spill else "?"))
-    print("  LDG at {} of {}; first compare at {}; all LDGs before it: {}".format(
-        ldg, len(loop), first_cmp, bool(ldg) and max(ldg) < first_cmp))
+    print("{}: {} instructions per {} pixels = {:.2f} per pixel; {} registers, spills {} bytes".format(
+        name, len(ops), pixels, len(ops) / pixels, a["registers"], a["spills"]))
+    for h, half in enumerate(a["halves"]):
+        ldg = half["ldg"]
+        print("  {}: LDG at {}; first compare at {}; all LDGs before it: {}".format(
+            "half {} (next chunk's loads)".format(h) if a["two_sets"] else "chunk", ldg, half["first_compare"],
+            bool(ldg) and max(ldg) < half["first_compare"]))
     print("  LDS {}, S2R {}".format(ops.count("LDS"), ops.count("S2R")))
     print("  mix: " + ", ".join("{} {}".format(c, op) for op, c in mix))
-    return text
+    return a["text"]
 
 
 def main():
