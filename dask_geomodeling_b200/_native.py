@@ -124,6 +124,18 @@ class GmWarp(ctypes.Structure):
     ]
 
 
+class GmStackInput(ctypes.Structure):
+    _fields_ = [
+        ("data", ctypes.c_void_p),
+        ("dtype", ctypes.c_int32),
+        ("cls", ctypes.c_uint8),
+        ("flags", ctypes.c_uint8),
+        ("reserved", ctypes.c_uint16),
+        ("k2", ctypes.c_uint64),
+        ("k4", ctypes.c_uint64),
+    ]
+
+
 # every symbol include/geokernels.h declares: name -> (restype, argtypes)
 _vp, _i, _i64, _d = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
 _P = ctypes.POINTER
@@ -159,6 +171,9 @@ SYMBOLS = {
                                  _P(_i64)]),
     "gm_jit_check": (_i, [_P(GmProgram), _P(ctypes.c_int32), _P(ctypes.c_int32), _P(_i64)]),
     "gm_jit_compile_count": (_i64, []),
+    "gm_reduce_stack": (_i, [_P(GmStackInput), _i64, _i, _i, ctypes.c_uint64, ctypes.c_uint64, _P(GmArray), _vp]),
+    "gm_place": (_i, [_P(GmArray), _P(GmArray), _vp, _vp, _i64, _P(GmStackInput), _i, _i, ctypes.c_uint64,
+                      ctypes.c_uint64, _vp]),
     "gm_resample_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _d, _d, _d, _d, _vp]),
     "gm_warp_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _P(GmWarp), _P(_i64), _vp]),
     "gm_hillshade": (_i, [_P(GmArray), _P(GmArray), _vp, _i, _d, _d, _d, _d, _d, _vp]),

@@ -45,6 +45,16 @@ __host__ __device__ inline int dtype_size(int dt) {
   return 0;
 }
 
+// GmClass a stored value is read into (what the evaluator's loads produce)
+__host__ __device__ inline int natural_class(int dt) {
+  switch (dt) {
+    case GM_F32: return GM_C_F32;
+    case GM_F64: return GM_C_F64;
+    case GM_U32: case GM_I64: return GM_C_I64;
+    default: return GM_C_I32;
+  }
+}
+
 // non-finite float source values become no data in the resample / warp gathers
 template <typename T> __device__ __forceinline__ bool is_finite(T v) { return true; }
 template <> __device__ __forceinline__ bool is_finite<float>(float v) { return isfinite(v); }

@@ -529,15 +529,6 @@ static bool wide(int cls) { return cls == GM_C_I64 || cls == GM_C_F64; }
 static bool is_binary(int op) {
   return (op >= GM_OP_ADD && op <= GM_OP_RPOW) || (op >= GM_OP_EQ && op <= GM_OP_LE);
 }
-static int natural_class(int dtype) {
-  switch (dtype) {
-    case GM_F32: return GM_C_F32;
-    case GM_F64: return GM_C_F64;
-    case GM_U32: case GM_I64: return GM_C_I64;
-    default: return GM_C_I32;
-  }
-}
-
 static int validate(const GmProgram* prog, const GmArray* inputs) {
   if (!prog) return fail("gm_eval_program: null program");
   if (prog->n_instr < 1 || prog->n_instr > GM_MAX_INSTR) return fail("gm_eval_program: bad instruction count");

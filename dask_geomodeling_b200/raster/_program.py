@@ -133,6 +133,64 @@ def _compare_dtype(dtypes_and_scalars):
     return np.result_type(*dtypes_and_scalars)
 
 
+def has_data_test(dtype, nodata):
+    """The has-data test of an OVERLAY step (utils.get_index: np.isclose for floats, == otherwise)
+    on a raster of ``dtype`` with no data value ``nodata``: (cmp class, flags, k2, k4)."""
+    dtype = np.dtype(dtype)
+    flags, cmp_cls, k2, k4 = 0, dtype_class(dtype), 0, 0
+    if nodata is not None:
+        if dtype.kind == "f":
+            cmp_dtype, y, tol, fin = _isclose_terms(dtype, nodata)
+            cmp_cls = dtype_class(cmp_dtype)
+            flags = F_ND_T | F_CLOSE | (F_ND_FINITE if fin else 0)
+            k2, k4 = _bits(y, cmp_cls), _bits(tol, cmp_cls)
+        else:
+            s = sentinel(dtype, nodata)
+            if s is not None:
+                flags, k2 = F_ND_T, _bits(s, cmp_cls)
+    return cmp_cls, flags, k2, k4
+
+
+def reduce_setup(statistic, dtype, nodata):
+    """(GmReduce kind, accumulator dtype, initial value) of reduce_rasters' ``statistic`` into
+    ``dtype``: 'last' / 'first' overlay, 'count' counts, 'max' / 'min' / 'sum' / 'product' reduce
+    in the float dtype NumPy's nan-functions would use (np.result_type(dtype, float16)), where a
+    NaN accumulator means "no value yet"."""
+    if statistic in ("last", "first"):
+        return 0, dtype, _cast_into(nodata, dtype)
+    if statistic == "count":
+        return RED_KINDS["count"], dtype, 0
+    work = np.result_type(dtype, np.float16)
+    if statistic in ("sum", "product") and work != dtype:
+        raise NotImplementedError(
+            "reduce_rasters('{}') of {} rasters accumulates in {} on the CPU path; the CUDA path "
+            "reduces float32 / float64 rasters only".format(statistic, dtype, work))
+    acc_dtype = np.dtype("f8") if work == np.float64 else np.dtype("f4")
+    return RED_KINDS[statistic], acc_dtype, float("nan")
+
+
+def stack_params(statistic, dtype, nodata):
+    """Arguments of gm_reduce_stack / gm_place for ``statistic`` into ``dtype`` with no data
+    ``nodata``, the epilogue of _Compiler.op_reduce: (kind, acc class, init bits, fill bits)."""
+    dtype = np.dtype(dtype)
+    kind, acc_dtype, init = reduce_setup(statistic, dtype, nodata)
+    A, T = dtype_class(acc_dtype), dtype_class(dtype)
+    fill = 0
+    if statistic not in ("last", "first", "count"):
+        fill = _bits(_cast_into(0 if statistic == "sum" else nodata, dtype), T)
+    return kind, A, _bits(init, A), fill
+
+
+def stack_input(values, nodata):
+    """GmStackInput of one raster (DeviceArray or None) with its has-data test."""
+    desc = _native.GmStackInput()
+    cls, flags, k2, k4 = has_data_test(values.dtype, nodata)
+    desc.data = values.ptr if _native.is_device(values) else None
+    desc.dtype = _native.dtype_code(values.dtype)
+    desc.cls, desc.flags, desc.k2, desc.k4 = cls, flags, k2, k4
+    return desc
+
+
 class _Typed(object):
     __slots__ = ("dtype", "nodata")
 
@@ -494,18 +552,7 @@ class _Compiler(object):
                 self.spill_to_reg(c)
         self.emit("LOAD", cls_b=T, cls_out=T, src=(SRC_IMM, 0), k=(_bits(fill, T),))
         for c in n.children:
-            tc = self.operand_type(c)
-            flags, cmp_cls, k2, k4 = 0, tc.cls, 0, 0
-            if tc.nodata is not None:
-                if tc.dtype.kind == "f":
-                    cmp_dtype, y, tol, fin = _isclose_terms(tc.dtype, tc.nodata)
-                    cmp_cls = dtype_class(cmp_dtype)
-                    flags = F_ND_T | F_CLOSE | (F_ND_FINITE if fin else 0)
-                    k2, k4 = _bits(y, cmp_cls), _bits(tol, cmp_cls)
-                else:
-                    s = sentinel(tc.dtype, tc.nodata)
-                    if s is not None:
-                        flags, k2 = F_ND_T, _bits(s, cmp_cls)
+            tc, cmp_cls, flags, k2, k4 = self._overlay_operand(c)
             saved = None
             if isinstance(c, Leaf):  # the sentinel test happens inside OVERLAY, in cmp_cls
                 saved, self.leaves[c.index] = self.leaves[c.index], _Typed(tc.dtype, None)
@@ -522,21 +569,9 @@ class _Compiler(object):
         return _Typed(dtype, fill)
 
     def _overlay_operand(self, c):
-        """Flags and constants of an OVERLAY step for child ``c`` (its has-data test is
-        utils.get_index: np.isclose for floats, == otherwise): (typed, cmp class, flags, k2, k4)."""
+        """(typed, cmp class, flags, k2, k4) of an OVERLAY step for child ``c``."""
         tc = self.operand_type(c)
-        flags, cmp_cls, k2, k4 = 0, tc.cls, 0, 0
-        if tc.nodata is not None:
-            if tc.dtype.kind == "f":
-                cmp_dtype, y, tol, fin = _isclose_terms(tc.dtype, tc.nodata)
-                cmp_cls = dtype_class(cmp_dtype)
-                flags = F_ND_T | F_CLOSE | (F_ND_FINITE if fin else 0)
-                k2, k4 = _bits(y, cmp_cls), _bits(tol, cmp_cls)
-            else:
-                s = sentinel(tc.dtype, tc.nodata)
-                if s is not None:
-                    flags, k2 = F_ND_T, _bits(s, cmp_cls)
-        return tc, cmp_cls, flags, k2, k4
+        return (tc,) + has_data_test(tc.dtype, tc.nodata)
 
     def op_reduce(self, n):
         """reduce_rasters (raster/reduction.py:38-119): 'last' / 'first' overlay the children,
@@ -554,18 +589,7 @@ class _Compiler(object):
         for c in children:
             if self.is_complex(c):
                 self.spill_to_reg(c)
-        if statistic in ("last", "first"):
-            kind, acc_dtype, init = 0, dtype, _cast_into(nodata, dtype)
-        elif statistic == "count":
-            kind, acc_dtype, init = RED_KINDS["count"], dtype, 0
-        else:
-            work = np.result_type(dtype, np.float16)
-            if statistic in ("sum", "product") and work != dtype:
-                raise NotImplementedError(
-                    "reduce_rasters('{}') of {} rasters accumulates in {} on the CPU path; the CUDA path "
-                    "reduces float32 / float64 rasters only".format(statistic, dtype, work))
-            acc_dtype = np.dtype("f8") if work == np.float64 else np.dtype("f4")
-            kind, init = RED_KINDS[statistic], float("nan")
+        kind, acc_dtype, init = reduce_setup(statistic, dtype, nodata)
         A = dtype_class(acc_dtype)
         self.emit("LOAD", cls_b=A, cls_out=A, src=(SRC_IMM, 0), k=(_bits(init, A),))
         for c in children:
@@ -846,6 +870,25 @@ def run_program(prog, inputs, out_dtypes, shape, keep_on_device):
     if any_device and not keep_on_device:
         outputs = [o.to_host() for o in outputs]
     return outputs
+
+
+def run_stack(statistic, stack, dtype, nodata, keep_on_device):
+    """reduce_rasters over a stack of any length with ONE gm_reduce_stack launch; ``stack`` =
+    [(values, no data value), ...] of one shape.  Results go where run_program puts them."""
+    if statistic == "first":
+        stack = stack[::-1]
+    kind, acc_cls, init, fill = stack_params(statistic, dtype, nodata)
+    shape = tuple(stack[0][0].shape)
+    staged = [v if _native.is_device(v) else _native.DeviceArray.from_host(np.ascontiguousarray(v))
+              for v, _ in stack]
+    inputs = (_native.GmStackInput * len(stack))()
+    for i, (v, (_, nd)) in enumerate(zip(staged, stack)):
+        inputs[i] = stack_input(v, nd)
+    out = _native.DeviceArray(shape, dtype)
+    _native.check(_native.lib().gm_reduce_stack(inputs, len(stack), kind, acc_cls, init, fill,
+                                                ctypes.byref(_native.as_gm_array(out)),
+                                                _native.current_stream()))
+    return out if keep_on_device else out.to_host()
 
 
 def evaluate(roots, leaves, keep_on_device=False, compiled=None):

@@ -5,7 +5,9 @@ block (:215-231).  The reference stacks the rasters into an (n, t, y, x) float a
 'no data' and calls NumPy's nan-functions along the first axis; here the rasters are the inputs
 of ONE evaluator program that keeps the running result of a pixel in a register (OVERLAY steps
 with a reduction kind, include/gm_bytecode.h) -- one pass over the inputs, no stack.  Inside a
-view the program is fused with the element-wise blocks around it (core/fusion.py).
+view the program is fused with the element-wise blocks around it (core/fusion.py).  Stacks the
+evaluator cannot take (more than GM_MAX_INPUTS rasters) go to gm_reduce_stack, which runs the same
+OVERLAY step over any number of rasters in one launch.
 
 Statistics on the CUDA path: last, first, count, max, min (any dtype: exact in the float dtype
 NumPy would use), sum and product (float32 / float64 rasters: sequential in the raster order, as
@@ -15,7 +17,8 @@ of rasters raise NotImplementedError (TemporalAggregate offers them along the ti
 import numpy as np
 
 from ..utils import Extent, parse_percentile_statistic
-from . import _lowering
+from .. import _native, _state
+from . import _lowering, _program
 from ._program import Node
 from .base import RasterBlock
 from .elemwise import BaseElementwise
@@ -44,21 +47,38 @@ def _lower_reduce(statistic):
     return lower
 
 
+def statistic_name(statistic):
+    """The name of ``statistic`` without a percentile ("p90" -> "percentile"); KeyError if unknown."""
+    if statistic in STATISTICS:
+        return statistic
+    name, percentile = parse_percentile_statistic(statistic)
+    if percentile is None:
+        raise KeyError('Unknown statistic "{}"'.format(statistic))
+    return name
+
+
+def on_device(name):
+    """``name`` (a statistic_name); NotImplementedError for a statistic the CUDA path lacks."""
+    if name not in ON_DEVICE:
+        raise NotImplementedError(
+            "reduce_rasters: statistic '{}' is not part of the CUDA raster path "
+            "(available: {})".format(name, ", ".join(ON_DEVICE)))
+    return name
+
+
+def device_statistic(statistic):
+    """``statistic`` as the CUDA stack reductions name it; raises for those they do not offer."""
+    return on_device(statistic_name(statistic))
+
+
 def reduce_rasters(stack, statistic, no_data_value=None, dtype=None):
     """Apply ``statistic`` pixel by pixel to a list of raster payloads (dicts with "values" and
     "no_data_value"), skipping 'no data'.  Output dtype and no data value default to those of
     the first raster; sums and counts hold 0 where every input is 'no data'."""
-    if statistic not in STATISTICS:
-        name, percentile = parse_percentile_statistic(statistic)
-        if percentile is None:
-            raise KeyError('Unknown statistic "{}"'.format(statistic))
-        statistic = name
+    statistic = statistic_name(statistic)
     if len(stack) == 0:
         raise ValueError("Cannot reduce a zero-length stack")
-    if statistic not in ON_DEVICE:
-        raise NotImplementedError(
-            "reduce_rasters: statistic '{}' is not part of the CUDA raster path "
-            "(available: {})".format(statistic, ", ".join(ON_DEVICE)))
+    on_device(statistic)
     shape = tuple(stack[0]["values"].shape)
     if any(tuple(d["values"].shape) != shape for d in stack[1:]):
         raise ValueError("all rasters of the stack must have the same shape")
@@ -67,9 +87,16 @@ def reduce_rasters(stack, statistic, no_data_value=None, dtype=None):
     if no_data_value is None:
         no_data_value = stack[0]["no_data_value"]
     kwargs = {"dtype": np.dtype(dtype).name, "fillvalue": no_data_value}
-    result = _lowering.run_single(lambda ops: _lower_reduce(statistic)([kwargs] + ops), list(stack))
-    result["no_data_value"] = no_data_value
-    return result
+    if len(stack) <= _native.GM_MAX_INPUTS:
+        try:
+            result = _lowering.run_single(lambda ops: _lower_reduce(statistic)([kwargs] + ops), list(stack))
+            result["no_data_value"] = no_data_value
+            return result
+        except _program.FusionLimit:
+            pass    # the stack kernel below takes any length
+    values = _program.run_stack(statistic, [(d["values"], d.get("no_data_value")) for d in stack],
+                                np.dtype(dtype), no_data_value, _state.keep_on_device())
+    return {"values": values, "no_data_value": no_data_value}
 
 
 def wrap_reduction_function(statistic):

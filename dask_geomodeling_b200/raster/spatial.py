@@ -11,6 +11,7 @@ import ctypes
 import numpy as np
 
 from .. import _native, _state, utils
+from . import _program
 from .base import BaseSingle
 
 __all__ = ["Dilate", "Smooth", "MovingMax", "HillShade", "Place"]
@@ -416,7 +417,7 @@ class Place(BaseSingle):
 
     @staticmethod
     def process(process_kwargs, *multi):
-        from .reduction import reduce_rasters
+        from .reduction import device_statistic, reduce_rasters
 
         mode = process_kwargs["mode"]
         if mode in ("meta", "time"):
@@ -448,27 +449,30 @@ class Place(BaseSingle):
         dst_h, dst_w = round((y2 - y1) / size_y), round((x2 - x1) / size_x)
         depth, src_h, src_w = source.shape
         shape = (depth, dst_h, dst_w)
-        if not _native.is_device(source):
-            source = _native.DeviceArray.from_host(np.ascontiguousarray(source))
-        holder, nodata_ptr = _native.scalar_ptr(nodata, dtype)
-        lib, stream = _native.lib(), _native.current_stream()
-        src_desc = _native.as_gm_array(source)
-        stack = []
+        offsets = []
         for cx, cy in process_kwargs["coordinates"]:
             di = round((cx - x1) / size_x - anchor_px[0])
             dj = round((cy - y1) / size_y - anchor_px[1])
             dj = dst_h - src_h - dj          # rows count from the northern edge
             if di <= -src_w or di >= dst_w or dj <= -src_h or dj >= dst_h:
                 continue                      # shifted completely outside
-            placed = _native.DeviceArray(shape, dtype)
-            dst_desc = _native.as_gm_array(placed)
-            # placed[:, j, i] = source[:, j - dj, i - di], 'no data' outside the source
-            _native.check(lib.gm_resample_nn(ctypes.byref(src_desc), ctypes.byref(dst_desc), nodata_ptr,
-                                             float(-di), 1.0, float(-dj), 1.0, stream))
-            stack.append({"values": placed, "no_data_value": nodata})
-        if not stack:
+            offsets.append((di, dj))
+        if not offsets:
             return {"values": np.full(shape, nodata, dtype), "no_data_value": nodata}
-        result = reduce_rasters(stack, process_kwargs["statistic"])
-        if not _state.keep_on_device() and _native.is_device(result["values"]):
-            result["values"] = result["values"].to_host()
-        return result
+        # out[:, j, i] = reduction over the copies of source[:, j - dj, i - di]; outside the source
+        # and at non-finite source cells a copy holds 'nodata' (as gm_resample_nn fills it)
+        statistic = device_statistic(process_kwargs["statistic"])
+        if statistic == "first":
+            offsets = offsets[::-1]
+        kind, acc_cls, init, fill = _program.stack_params(statistic, dtype, nodata)
+        if not _native.is_device(source):
+            source = _native.DeviceArray.from_host(np.ascontiguousarray(source))
+        holder, nodata_ptr = _native.scalar_ptr(nodata, dtype)
+        test = _program.stack_input(source, nodata)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int32)
+        out = _native.DeviceArray(shape, dtype)
+        _native.check(_native.lib().gm_place(
+            ctypes.byref(_native.as_gm_array(source)), ctypes.byref(_native.as_gm_array(out)), nodata_ptr,
+            offsets.ctypes.data, len(offsets), ctypes.byref(test), kind, acc_cls, init, fill,
+            _native.current_stream()))
+        return {"values": out if _state.keep_on_device() else out.to_host(), "no_data_value": nodata}

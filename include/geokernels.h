@@ -148,6 +148,33 @@ int  gm_jit_check(const GmProgram* prog, const int32_t* in_dtype, const int32_t*
                   int64_t* cubin_bytes);
 int64_t gm_jit_compile_count(void);
 
+/* reduce_rasters over stacks of any length (raster/reduction.py:38-119) and Place at any number of
+ * coordinates (raster/spatial.py:657-731).  Each raster of a stack is reduced exactly as by a
+ * GM_OP_OVERLAY step of kind `kind` (GmReduce) into an accumulator of class `acc_cls` that starts at
+ * `init`; its has-data test is that of GM_OP_OVERLAY (utils.get_index: np.isclose for floats, ==
+ * otherwise) on the stored value converted to class `cls`.  The result is stored in the output
+ * dtype: for max / min / sum / product a NaN accumulator (no raster had data) becomes `fill`
+ * (raw bits of the output's class), other values are converted; last / count store acc as it is.
+ * 'first' is 'last' over the reversed stack.                                                      */
+typedef struct GmStackInput {
+  const void* data;    /* device pointer, n_pixels cells; any alignment                          */
+  int32_t dtype;       /* GmDType of the storage                                                  */
+  uint8_t cls;         /* GmClass the value is tested and reduced in                              */
+  uint8_t flags;       /* GM_F_ND_T | GM_F_CLOSE | GM_F_ND_FINITE                                 */
+  uint16_t reserved;
+  uint64_t k2, k4;     /* sentinel, isclose tolerance: raw bits of class `cls`                    */
+} GmStackInput;
+/* one kernel launch whatever n_inputs is; `inputs` is a host array, `out` a device array        */
+int  gm_reduce_stack(const GmStackInput* inputs, int64_t n_inputs, int kind, int acc_cls,
+                     uint64_t init, uint64_t fill, GmArray* out, void* stream);
+/* out[b, j, i] = reduction over copies c (in order) of src[b, j - dj_c, i - di_c]; a cell outside
+ * the source or holding a non-finite float is `nodata` (src dtype), as gm_resample_nn makes it.
+ * `offsets` = host (di_0, dj_0, di_1, dj_1, ...); `test` = has-data test of the source (its
+ * data is ignored).  Work is proportional to the output tiles each copy meets.                  */
+int  gm_place(const GmArray* src, GmArray* dst, const void* nodata, const int32_t* offsets,
+              int64_t n_copies, const GmStackInput* test, int kind, int acc_cls, uint64_t init,
+              uint64_t fill, void* stream);
+
 /* input adaptor: nearest-neighbour resample of a source window into the
  * request grid; equals the aligned crop/pad for aligned requests
  * (raster/sources.py:119-149, MemorySource).  src_i = floor(i0 + (i+0.5)*si)  */
