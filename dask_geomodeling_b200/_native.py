@@ -174,6 +174,9 @@ SYMBOLS = {
     "gm_reduce_stack": (_i, [_P(GmStackInput), _i64, _i, _i, ctypes.c_uint64, ctypes.c_uint64, _P(GmArray), _vp]),
     "gm_place": (_i, [_P(GmArray), _P(GmArray), _vp, _vp, _i64, _P(GmStackInput), _i, _i, ctypes.c_uint64,
                       ctypes.c_uint64, _vp]),
+    "gm_reduce_stack_stat": (_i, [_P(GmStackInput), _i64, _i, _i, ctypes.c_uint64, _P(GmArray), _vp]),
+    "gm_place_stat": (_i, [_P(GmArray), _P(GmArray), _vp, _vp, _i64, _P(GmStackInput), _i, _i, ctypes.c_uint64,
+                           _vp]),
     "gm_resample_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _d, _d, _d, _d, _vp]),
     "gm_warp_nn": (_i, [_P(GmArray), _P(GmArray), _vp, _P(GmWarp), _P(_i64), _vp]),
     "gm_hillshade": (_i, [_P(GmArray), _P(GmArray), _vp, _i, _d, _d, _d, _d, _d, _vp]),

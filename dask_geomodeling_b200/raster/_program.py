@@ -31,6 +31,8 @@ F_NAN = 32  # LOAD / MATB / CVT: sentinel -> NaN (shares the bit of F_RIGHT)
 
 DENSE_TABLE_LIMIT = 4096
 RED_KINDS = {"max": 1, "min": 2, "sum": 3, "product": 4, "count": 5}   # GmReduce
+STACK_STATS = {"mean": 0, "var": 1, "std": 2, "argmin": 3, "argmax": 4}  # GmStackStat
+FLOAT_ONLY = ("sum", "product", "mean", "std", "var")   # statistics of float32 / float64 outputs
 
 
 class FusionLimit(Exception):
@@ -160,13 +162,20 @@ def reduce_setup(statistic, dtype, nodata):
         return 0, dtype, _cast_into(nodata, dtype)
     if statistic == "count":
         return RED_KINDS["count"], dtype, 0
+    work = working_dtype(statistic, dtype)
+    acc_dtype = np.dtype("f8") if work == np.float64 else np.dtype("f4")
+    return RED_KINDS[statistic], acc_dtype, float("nan")
+
+
+def working_dtype(statistic, dtype):
+    """The float dtype NumPy's nan-functions compute ``statistic`` in for an output of ``dtype``
+    (np.result_type(dtype, float16)); NotImplementedError where the CUDA path does not follow."""
     work = np.result_type(dtype, np.float16)
-    if statistic in ("sum", "product") and work != dtype:
+    if statistic in FLOAT_ONLY and work != dtype:
         raise NotImplementedError(
             "reduce_rasters('{}') of {} rasters accumulates in {} on the CPU path; the CUDA path "
             "reduces float32 / float64 rasters only".format(statistic, dtype, work))
-    acc_dtype = np.dtype("f8") if work == np.float64 else np.dtype("f4")
-    return RED_KINDS[statistic], acc_dtype, float("nan")
+    return work
 
 
 def stack_params(statistic, dtype, nodata):
@@ -179,6 +188,15 @@ def stack_params(statistic, dtype, nodata):
     if statistic not in ("last", "first", "count"):
         fill = _bits(_cast_into(0 if statistic == "sum" else nodata, dtype), T)
     return kind, A, _bits(init, A), fill
+
+
+def stack_stat_params(statistic, dtype, nodata):
+    """Arguments of gm_reduce_stack_stat / gm_place_stat for ``statistic`` (mean, var, std, argmin,
+    argmax) into ``dtype`` with no data ``nodata``: (GmStackStat, bytes of the working dtype, fill
+    bits of the output's class)."""
+    dtype = np.dtype(dtype)
+    work = working_dtype(statistic, dtype)
+    return STACK_STATS[statistic], work.itemsize, _bits(_cast_into(nodata, dtype), dtype_class(dtype))
 
 
 def stack_input(values, nodata):
@@ -872,22 +890,39 @@ def run_program(prog, inputs, out_dtypes, shape, keep_on_device):
     return outputs
 
 
+def _stack_inputs(stack):
+    """(GmStackInput array, device arrays kept alive) of [(values, no data value), ...]."""
+    staged = [v if _native.is_device(v) else _native.DeviceArray.from_host(np.ascontiguousarray(v))
+              for v, _ in stack]
+    inputs = (_native.GmStackInput * len(stack))()
+    for i, (v, (_, nd)) in enumerate(zip(staged, stack)):
+        inputs[i] = stack_input(v, nd)
+    return inputs, staged
+
+
 def run_stack(statistic, stack, dtype, nodata, keep_on_device):
     """reduce_rasters over a stack of any length with ONE gm_reduce_stack launch; ``stack`` =
     [(values, no data value), ...] of one shape.  Results go where run_program puts them."""
     if statistic == "first":
         stack = stack[::-1]
     kind, acc_cls, init, fill = stack_params(statistic, dtype, nodata)
-    shape = tuple(stack[0][0].shape)
-    staged = [v if _native.is_device(v) else _native.DeviceArray.from_host(np.ascontiguousarray(v))
-              for v, _ in stack]
-    inputs = (_native.GmStackInput * len(stack))()
-    for i, (v, (_, nd)) in enumerate(zip(staged, stack)):
-        inputs[i] = stack_input(v, nd)
-    out = _native.DeviceArray(shape, dtype)
+    inputs, staged = _stack_inputs(stack)
+    out = _native.DeviceArray(tuple(stack[0][0].shape), dtype)
     _native.check(_native.lib().gm_reduce_stack(inputs, len(stack), kind, acc_cls, init, fill,
                                                 ctypes.byref(_native.as_gm_array(out)),
                                                 _native.current_stream()))
+    return out if keep_on_device else out.to_host()
+
+
+def run_stack_stat(statistic, stack, dtype, nodata, keep_on_device):
+    """run_stack for mean, var, std, argmin and argmax (gm_reduce_stack_stat): computed in the
+    working dtype np.result_type(dtype, float16), stored in ``dtype``."""
+    stat, work_bytes, fill = stack_stat_params(statistic, dtype, nodata)
+    inputs, staged = _stack_inputs(stack)
+    out = _native.DeviceArray(tuple(stack[0][0].shape), dtype)
+    _native.check(_native.lib().gm_reduce_stack_stat(inputs, len(stack), stat, work_bytes, fill,
+                                                     ctypes.byref(_native.as_gm_array(out)),
+                                                     _native.current_stream()))
     return out if keep_on_device else out.to_host()
 
 

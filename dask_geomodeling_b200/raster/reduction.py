@@ -9,10 +9,15 @@ view the program is fused with the element-wise blocks around it (core/fusion.py
 evaluator cannot take (more than GM_MAX_INPUTS rasters) go to gm_reduce_stack, which runs the same
 OVERLAY step over any number of rasters in one launch.
 
-Statistics on the CUDA path: last, first, count, max, min (any dtype: exact in the float dtype
-NumPy would use), sum and product (float32 / float64 rasters: sequential in the raster order, as
-NumPy's axis-0 reduction).  mean / std / var / median / argmin / argmax / percentiles of a stack
-of rasters raise NotImplementedError (TemporalAggregate offers them along the time axis).
+mean, var, std, argmin and argmax keep more than one value per pixel, which an OVERLAY step does
+not: a stack of any length, also of one raster, goes to gm_reduce_stack_stat, one launch that
+stacks the rasters in NumPy's working dtype (np.result_type(dtype, float16)) and reduces them as
+np.nanmean / nanvar / nanstd / nanargmin / nanargmax do (var and std read the stack twice).
+
+Statistics on the CUDA path: last, first, count, max, min, argmin, argmax (any dtype: exact in the
+float dtype NumPy would use), sum, product, mean, var and std (float32 / float64 outputs:
+sequential in the raster order, as NumPy's axis-0 reduction).  median and percentiles of a stack of
+rasters raise NotImplementedError (TemporalAggregate offers them along the time axis).
 """
 import numpy as np
 
@@ -27,7 +32,8 @@ __all__ = ["Max"]
 
 STATISTICS = ("first", "last", "count", "sum", "mean", "min", "max", "argmin", "argmax", "std", "var",
               "median", "product")
-ON_DEVICE = ("first", "last", "count", "sum", "min", "max", "product")
+ON_DEVICE = ("first", "last", "count", "sum", "min", "max", "product", "mean", "var", "std", "argmin",
+             "argmax")
 
 
 def check_statistic(statistic):
@@ -86,6 +92,11 @@ def reduce_rasters(stack, statistic, no_data_value=None, dtype=None):
         dtype = stack[0]["values"].dtype
     if no_data_value is None:
         no_data_value = stack[0]["no_data_value"]
+    payloads = [(d["values"], d.get("no_data_value")) for d in stack]
+    if statistic in _program.STACK_STATS:
+        values = _program.run_stack_stat(statistic, payloads, np.dtype(dtype), no_data_value,
+                                         _state.keep_on_device())
+        return {"values": values, "no_data_value": no_data_value}
     kwargs = {"dtype": np.dtype(dtype).name, "fillvalue": no_data_value}
     if len(stack) <= _native.GM_MAX_INPUTS:
         try:
@@ -94,8 +105,7 @@ def reduce_rasters(stack, statistic, no_data_value=None, dtype=None):
             return result
         except _program.FusionLimit:
             pass    # the stack kernel below takes any length
-    values = _program.run_stack(statistic, [(d["values"], d.get("no_data_value")) for d in stack],
-                                np.dtype(dtype), no_data_value, _state.keep_on_device())
+    values = _program.run_stack(statistic, payloads, np.dtype(dtype), no_data_value, _state.keep_on_device())
     return {"values": values, "no_data_value": no_data_value}
 
 

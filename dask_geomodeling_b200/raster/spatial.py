@@ -464,15 +464,19 @@ class Place(BaseSingle):
         statistic = device_statistic(process_kwargs["statistic"])
         if statistic == "first":
             offsets = offsets[::-1]
-        kind, acc_cls, init, fill = _program.stack_params(statistic, dtype, nodata)
+        if statistic in _program.STACK_STATS:
+            # mean / var / std / argmin / argmax: a copy enters the stack when it puts a data cell
+            # inside the request, so argmin / argmax count only those copies (gm_place_stat)
+            place, args = _native.lib().gm_place_stat, _program.stack_stat_params(statistic, dtype, nodata)
+        else:
+            place, args = _native.lib().gm_place, _program.stack_params(statistic, dtype, nodata)
         if not _native.is_device(source):
             source = _native.DeviceArray.from_host(np.ascontiguousarray(source))
         holder, nodata_ptr = _native.scalar_ptr(nodata, dtype)
         test = _program.stack_input(source, nodata)
         offsets = np.ascontiguousarray(offsets, dtype=np.int32)
         out = _native.DeviceArray(shape, dtype)
-        _native.check(_native.lib().gm_place(
+        _native.check(place(
             ctypes.byref(_native.as_gm_array(source)), ctypes.byref(_native.as_gm_array(out)), nodata_ptr,
-            offsets.ctypes.data, len(offsets), ctypes.byref(test), kind, acc_cls, init, fill,
-            _native.current_stream()))
+            offsets.ctypes.data, len(offsets), ctypes.byref(test), *args, _native.current_stream()))
         return {"values": out if _state.keep_on_device() else out.to_host(), "no_data_value": nodata}

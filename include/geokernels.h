@@ -175,6 +175,29 @@ int  gm_place(const GmArray* src, GmArray* dst, const void* nodata, const int32_
               int64_t n_copies, const GmStackInput* test, int kind, int acc_cls, uint64_t init,
               uint64_t fill, void* stream);
 
+/* The statistics of reduce_rasters that keep more than one value per pixel, over the same stacks:
+ * the rasters are stacked in the working float dtype W (`work_bytes` = 2, 4 or 8: float16 / 32 /
+ * 64), a slot holding the value converted to W where the has-data test holds and NaN elsewhere,
+ * then reduced as NumPy's nan-functions reduce axis 0:
+ *   mean:   sum in W in stack order, divided by the count in float64, rounded to W   (np.nanmean)
+ *   var:    sum of W((x - mean)^2) in stack order, divided likewise; ddof 0          (np.nanvar)
+ *   std:    sqrt(var) in W                                                            (np.nanstd)
+ *   argmin / argmax: first index reaching the extreme, a NaN slot counting as +inf / -inf
+ *                    (np.nanargmin / np.nanargmax), converted to the output dtype.
+ * A pixel where every slot is NaN holds `fill` (raw bits of the output's class); other results,
+ * NaN and inf included, are stored as they are.  mean / var / std need W == the output dtype. */
+enum GmStackStat { GM_STACK_MEAN = 0, GM_STACK_VAR = 1, GM_STACK_STD = 2, GM_STACK_ARGMIN = 3,
+                  GM_STACK_ARGMAX = 4 };
+/* one kernel launch whatever n_inputs is (var and std read the stack twice within it)           */
+int  gm_reduce_stack_stat(const GmStackInput* inputs, int64_t n_inputs, int stat, int work_bytes,
+                          uint64_t fill, GmArray* out, void* stream);
+/* gm_place with a GmStackStat.  A cell outside a copy's footprint is a NaN slot.  The stack holds
+ * the copies that put at least one data cell (any band) inside `dst`, in order, so the index of
+ * argmin / argmax is a copy's rank among those.                                                  */
+int  gm_place_stat(const GmArray* src, GmArray* dst, const void* nodata, const int32_t* offsets,
+                   int64_t n_copies, const GmStackInput* test, int stat, int work_bytes, uint64_t fill,
+                   void* stream);
+
 /* input adaptor: nearest-neighbour resample of a source window into the
  * request grid; equals the aligned crop/pad for aligned requests
  * (raster/sources.py:119-149, MemorySource).  src_i = floor(i0 + (i+0.5)*si)  */

@@ -4,13 +4,18 @@ at N = 8 (time and bytes), and
 gm_place of a 256^2 float32 source at N = 8, 1 000 and 100 000 coordinates into 16384^2 (last,
 max, sum), against the former copy-and-reduce path at N = 8.
 
+With --stats: mean, var, std and argmax (gm_reduce_stack_stat) over N = 4, 16, 64 float32 8192^2
+rasters next to sum (gm_reduce_stack) in the same run, and Place of the 256^2 source at 1 000
+coordinates into 16384^2 for sum, mean and argmax (gm_place_stat).
+
 Times are CUDA events around back-to-back calls on resident inputs (8192^2 float32 inputs are
 268 MB each, beyond the 126 MB L2).  Algorithmic bytes: one read of every input cell and one write
-of every output cell; for Place one write of the output (the source stays in L2).  The share of HBM
-is taken against 6451.5 GB/s, the device-to-device copy rate measured on this project's B200
-(DESIGN §3).  Prints one JSON line; the GPU name and power limit are read in the same run.
+of every output cell (var and std read their stack twice in the kernel, but need it once); for
+Place one write of the output (the source stays in L2).  The share of HBM is taken against
+6451.5 GB/s, the device-to-device copy rate measured on this project's B200 (DESIGN §3).  Prints
+one JSON line; the GPU name and power limit are read in the same run.
 
-Usage: python tools/stack_bench.py [--iters 10] [--out FILE]
+Usage: python tools/stack_bench.py [--stats] [--iters 10] [--out FILE]
 """
 import argparse
 import ctypes
@@ -52,8 +57,70 @@ def main():
     parser.add_argument("--iters", type=int, default=10)
     parser.add_argument("--size", type=int, default=8192)
     parser.add_argument("--place-size", type=int, default=16384)
+    parser.add_argument("--stats", action="store_true", help="mean / var / std / argmax instead")
     parser.add_argument("--out", default=None)
     args = parser.parse_args()
+    results = stats_bench(args) if args.stats else stack_bench(args)
+    line = json.dumps(results)
+    print(line)
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
+
+
+def device_stack(rng, n, size, dtype, nodata):
+    from dask_geomodeling_b200 import _native
+
+    out = []
+    for k in range(n):
+        if np.dtype(dtype).kind == "f":
+            v = rng.standard_normal((1, size, size), dtype=np.float32).astype(dtype)
+        else:
+            v = rng.integers(-1000, 1000, (1, size, size)).astype(dtype)
+        v[0, :: 7 + k % 5] = nodata
+        out.append((_native.DeviceArray.from_host(v), nodata))
+    return out
+
+
+def rate(nbytes, ms):
+    return {"ms": round(ms, 4), "gbs": round(nbytes / ms / 1e6, 1), "hbm_share": round(nbytes / ms / 1e6 / HBM_GBS, 3)}
+
+
+def stats_bench(args):
+    import torch
+    from dask_geomodeling_b200 import _native, _state
+    from dask_geomodeling_b200.raster import _program, spatial
+
+    side = torch.cuda.Stream()
+    results = {"gpu": gpu_info(), "hbm_gbs": HBM_GBS, "reduce": [], "place": []}
+    size, rng = args.size, np.random.default_rng(0)
+    with torch.cuda.stream(side), _native.use_stream(side.cuda_stream), _state.device_resident():
+        f32 = device_stack(rng, 64, size, "f4", np.float32(-9999.0))
+        for n in (4, 16, 64):
+            stack = f32[:n]
+            nbytes = (n + 1) * size * size * 4
+            for statistic in ("sum", "mean", "var", "std", "argmax"):
+                run = _program.run_stack if statistic == "sum" else _program.run_stack_stat
+                ms = timed(lambda: run(statistic, stack, np.dtype("f4"), -9999.0, True), args.iters)
+                results["reduce"].append(dict({"n": n, "dtype": "float32", "statistic": statistic},
+                                              **rate(nbytes, ms)))
+        del f32
+        psize = args.place_size
+        src = rng.uniform(1, 100, (1, 256, 256)).astype("f4")
+        src[src < 10] = -9999.0
+        payload = {"values": _native.DeviceArray.from_host(src), "no_data_value": -9999.0}
+        coordinates = [(float(x), float(y)) for x, y in zip(rng.uniform(0, psize, 1000), rng.uniform(0, psize, 1000))]
+        for statistic in ("sum", "mean", "argmax"):
+            kwargs = {"mode": "warp", "anchor": (0.0, 256.0), "coordinates": coordinates,
+                      "src_bbox": (0.0, 0.0, 256.0, 256.0), "dst_bbox": (0.0, 0.0, float(psize), float(psize)),
+                      "cellsize": (1.0, 1.0), "statistic": statistic}
+            ms = timed(lambda: spatial.Place.process(kwargs, payload), max(2, args.iters // 2))
+            results["place"].append(dict({"n": 1000, "statistic": statistic}, **rate(psize * psize * 4, ms)))
+    return results
+
+
+def stack_bench(args):
 
     import torch
     from dask_geomodeling_b200 import _native, _state
@@ -67,19 +134,8 @@ def main():
     size = args.size
     rng = np.random.default_rng(0)
 
-    def device_stack(n, dtype, nodata):
-        out = []
-        for k in range(n):
-            if np.dtype(dtype).kind == "f":
-                v = rng.standard_normal((1, size, size), dtype=np.float32).astype(dtype)
-            else:
-                v = rng.integers(-1000, 1000, (1, size, size)).astype(dtype)
-            v[0, :: 7 + k % 5] = nodata
-            out.append((_native.DeviceArray.from_host(v), nodata))
-        return out
-
     with torch.cuda.stream(side), _native.use_stream(side.cuda_stream), _state.device_resident():
-        f32 = device_stack(64, "f4", np.float32(-9999.0))
+        f32 = device_stack(rng, 64, size, "f4", np.float32(-9999.0))
         for n in (4, 8, 16, 64):
             for statistic in ("max", "sum", "last"):
                 stack = f32[:n]
@@ -100,7 +156,7 @@ def main():
                                identical_bytes=evaluated.to_host().tobytes() == b.tobytes())
                 results["reduce"].append(row)
         del f32
-        i16 = device_stack(16, "i2", -32768)
+        i16 = device_stack(rng, 16, size, "i2", -32768)
         ms = timed(lambda: _program.run_stack("max", i16, np.dtype("i2"), -32768, True), args.iters)
         nbytes = 17 * size * size * 2
         results["reduce"].append({"n": 16, "dtype": "int16", "statistic": "max", "ms": round(ms, 4),
@@ -129,12 +185,7 @@ def main():
                     b = old_place(_native, lib, reduce_rasters, src, payload, kwargs)["values"].to_host()
                     row.update(old_ms=round(old_ms, 4), identical_bytes=a.tobytes() == b.tobytes())
                 results["place"].append(row)
-    line = json.dumps(results)
-    print(line)
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write(line + "\n")
+    return results
 
 
 def old_place(_native, lib, reduce_rasters, src, payload, kwargs):
