@@ -5,6 +5,7 @@
 #include "gm_common.cuh"
 #include <cfloat>
 #include <cstdlib>
+#include <cstring>
 #include <cmath>
 #include <limits>
 #include <algorithm>
@@ -262,56 +263,6 @@ hillshade_quad_kernel(const T* __restrict__ src, uint8_t* __restrict__ dst, T no
 // ---------------------------------------------------------------------------------
 // MovingMax (raster/spatial.py:192-213): circular footprint, chord per row
 // ---------------------------------------------------------------------------------
-constexpr int MM_TX = 32, MM_TY = 8, MM_MAXR = 32;
-
-template <typename T>
-__global__ void __launch_bounds__(MM_TX * MM_TY)
-moving_max_kernel(const T* __restrict__ src, T* __restrict__ dst, T nodata, int has_nodata,
-                  int bands, int H, int W, int r, const int* __restrict__ half_width) {
-  // shared tile with halo; no data is replaced by the dtype minimum on load
-  extern __shared__ __align__(16) unsigned char mm_smem[];
-  T* tile = reinterpret_cast<T*>(mm_smem);
-  __shared__ int hw[2 * MM_MAXR + 1];
-  const int tw = MM_TX + 2 * r, th = MM_TY + 2 * r;
-  const int SW = W + 2 * r;
-  const int64_t in_plane = (int64_t)(H + 2 * r) * SW, out_plane = (int64_t)H * W;
-  const int tid = threadIdx.y * MM_TX + threadIdx.x;
-  if (tid < 2 * r + 1) hw[tid] = half_width[tid];
-  const int x0 = blockIdx.x * MM_TX, y0 = blockIdx.y * MM_TY;
-  const T lowest = Lowest<T>::value();
-  for (int b = blockIdx.z; b < bands; b += gridDim.z) {
-    __syncthreads();
-    for (int i = tid; i < tw * th; i += MM_TX * MM_TY) {
-      const int ty = i / tw, tx = i - ty * tw;
-      const int gy = y0 + ty, gx = x0 + tx;  // coordinates in the haloed source
-      T v = lowest;
-      if (gy < H + 2 * r && gx < SW) {
-        v = __ldg(src + (int64_t)b * in_plane + (int64_t)gy * SW + gx);
-        if (has_nodata && v == nodata) v = lowest;
-      }
-      tile[i] = v;
-    }
-    __syncthreads();
-    const int x = x0 + threadIdx.x, y = y0 + threadIdx.y;
-    if (x < W && y < H) {
-      T best = lowest;
-      for (int dy = -r; dy <= r; ++dy) {
-        const int w = hw[dy + r];
-        const T* row = tile + (threadIdx.y + r + dy) * tw + threadIdx.x + r;
-        for (int dx = -w; dx <= w; ++dx) {
-          const T v = row[dx];
-          best = v > best ? v : best;
-        }
-      }
-      // restore no data only where the centre was no data and nothing was found
-      const T centre = __ldg(src + (int64_t)b * in_plane + (int64_t)(y + r) * SW + (x + r));
-      if (has_nodata && best == lowest && centre == nodata) best = nodata;
-      dst[(int64_t)b * out_plane + (int64_t)y * W + x] = best;
-    }
-  }
-}
-
-
 // Tiled version for radii up to MM2_MAXR.  The disc is a stack of horizontal chords
 // with only a few distinct half-widths (size 11: 2, 3, 4, 5), so per tile
 //   1. the source tile + halo goes to shared memory (no data -> dtype minimum),
@@ -833,6 +784,178 @@ static int try_moving_max_fixed(int size, const Staged& in, Staged& out, T nd, i
   return -1;
 }
 
+// Radii above 8, 8-byte cells from radius 7, and radius <= 8 where the tiled kernel's tile does
+// not fit; any dtype, no size cap: the disc as 2r + 1 chords, each chord an O(1) range-maximum query.
+// A block owns MMC_TX output columns x MMC_GROUPS * MMC_ROWS output rows and streams the
+// source rows they depend on from top to bottom.  Per source row
+//   1. the segment of MMC_TX + 2r cells is staged as level 0 (no data -> dtype minimum); the
+//      loads of the next row are issued before this row's levels are built,
+//   2. level k of the range-maximum ("sparse") table holds at p the maximum of cells
+//      [p, p + 2^k), built from level k - 1 with one barrier per level,
+//   3. a chord [x - w, x + w] of footprint row dy is max(M_k[x - w], M_k[x + w - 2^k + 1]),
+//      k = floor(log2(2w + 1)); the host table `chord` holds both offsets per dy, and every
+//      thread folds into the output rows of its group in reach one 3-input maximum per column.
+// A thread keeps the running maxima of MMC_ROWS rows x MMC_COLS columns in registers.
+// Work per pixel: 2r + 1 chords of two shared loads each, plus the table build, about
+// log2(2r + 1) operations per staged cell shared by the block's rows.  Shared memory:
+// levels x (MMC_TX + 2r) cells; the limit that leaves is checked on the host.
+constexpr int MMC_THREADS = 256, MMC_GROUPS = 4, MMC_GROUP = MMC_THREADS / MMC_GROUPS, MMC_COLS = 4;
+constexpr int MMC_TX = MMC_GROUP * MMC_COLS;   // 256 output columns
+constexpr int MMC_ROWS = 8;                    // output rows per group: MMC_GROUPS * 8 per block
+constexpr int MMC_PREFETCH = 8;                // staged cells per thread held in registers
+
+template <typename T, bool FULL>
+__device__ __forceinline__ void mmc_fold(const T* levels, const int2* __restrict__ chord, int sg, int r,
+                                         int u, T (&best)[MMC_ROWS][MMC_COLS]) {
+#pragma unroll
+  for (int j = 0; j < MMC_ROWS; ++j) {
+    const int d = sg - j;     // footprint row dy + r of output row j
+    if (FULL || (unsigned)d <= (unsigned)(2 * r)) {
+      const int2 o = __ldg(chord + d);
+      const T* a = levels + o.x + u;
+      const T* b = levels + o.y + u;
+#pragma unroll
+      for (int c = 0; c < MMC_COLS; ++c) best[j][c] = vmax3<T>(best[j][c], a[c * MMC_GROUP], b[c * MMC_GROUP]);
+    }
+  }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(MMC_THREADS, 1)   // ~200 registers: 2 blocks per SM spill
+moving_max_chord_kernel(const T* __restrict__ src, T* __restrict__ dst, T nodata, int has_nodata,
+                        int bands, int H, int W, int r, int n_levels, int pitch,
+                        const int2* __restrict__ chord) {
+  extern __shared__ __align__(16) unsigned char mm_smem[];
+  T* levels = reinterpret_cast<T*>(mm_smem);          // n_levels x pitch, then MMC_TX sentinel cells
+  const int tid = threadIdx.x, g = tid / MMC_GROUP, u = tid % MMC_GROUP;
+  const int SW = W + 2 * r, SH = H + 2 * r;
+  const int64_t in_plane = (int64_t)SH * SW, out_plane = (int64_t)H * W;
+  const int x0 = blockIdx.x * MMC_TX, y0 = blockIdx.y * (MMC_GROUPS * MMC_ROWS);
+  const int seg = MMC_TX + 2 * r;
+  const int n_src = min(MMC_GROUPS * MMC_ROWS, H - y0) + 2 * r;   // source rows the block's outputs need
+  const T lowest = Lowest<T>::value();
+  // footprint rows without a chord (even sizes) point at the sentinel cells
+  for (int i = tid; i < MMC_TX; i += MMC_THREADS) levels[n_levels * pitch + i] = lowest;
+  for (int b = blockIdx.z; b < bands; b += gridDim.z) {
+    const T* plane = src + (int64_t)b * in_plane;
+    T pf[MMC_PREFETCH];
+    auto fetch = [&](int s) {       // unconditional loads on clamped addresses
+      const T* row = plane + (int64_t)min(y0 + s, SH - 1) * SW;
+#pragma unroll
+      for (int m = 0; m < MMC_PREFETCH; ++m) pf[m] = __ldg(row + min(x0 + tid + m * MMC_THREADS, SW - 1));
+    };
+    auto clean = [&](T v, int s, int i) {
+      return (y0 + s < SH && x0 + i < SW && !(has_nodata && v == nodata)) ? v : lowest;
+    };
+    auto stage = [&](int s) {       // level 0 of source row s
+#pragma unroll
+      for (int m = 0; m < MMC_PREFETCH; ++m) {
+        const int i = tid + m * MMC_THREADS;
+        if (i < seg) levels[i] = clean(pf[m], s, i);
+      }
+      const T* row = plane + (int64_t)min(y0 + s, SH - 1) * SW;
+      for (int i = tid + MMC_PREFETCH * MMC_THREADS; i < seg; i += MMC_THREADS)
+        levels[i] = clean(__ldg(row + min(x0 + i, SW - 1)), s, i);
+    };
+    T best[MMC_ROWS][MMC_COLS];
+#pragma unroll
+    for (int j = 0; j < MMC_ROWS; ++j)
+#pragma unroll
+      for (int c = 0; c < MMC_COLS; ++c) best[j][c] = lowest;
+    fetch(0);
+    stage(0);
+    for (int s = 0; s < n_src; ++s) {
+      __syncthreads();                                  // level 0 of row s is in place
+      if (s + 1 < n_src) fetch(s + 1);
+      for (int k = 1; k < n_levels; ++k) {
+        const int half = 1 << (k - 1), n = seg - 2 * half + 1;
+        T* lk = levels + k * pitch;
+        const T* prev = lk - pitch;
+        for (int p = tid; p < n; p += MMC_THREADS) lk[p] = vmax<T>(prev[p], prev[p + half]);
+        __syncthreads();
+      }
+      // output rows g * MMC_ROWS + j of this group take footprint row s - g * MMC_ROWS - j - r
+      const int sg = s - g * MMC_ROWS;
+      if (sg >= 0 && sg - (MMC_ROWS - 1) <= 2 * r) {
+        if (sg >= MMC_ROWS - 1 && sg <= 2 * r) mmc_fold<T, true>(levels, chord, sg, r, u, best);
+        else mmc_fold<T, false>(levels, chord, sg, r, u, best);
+      }
+      __syncthreads();                                  // every thread is done with row s
+      if (s + 1 < n_src) stage(s + 1);
+    }
+#pragma unroll
+    for (int j = 0; j < MMC_ROWS; ++j) {
+      const int y = y0 + g * MMC_ROWS + j;
+      if (y >= H) break;
+#pragma unroll
+      for (int c = 0; c < MMC_COLS; ++c) {
+        const int x = x0 + u + c * MMC_GROUP;
+        if (x >= W) continue;
+        T v = best[j][c];
+        // restore no data only where the centre was no data and nothing was found
+        if (has_nodata && v == lowest && __ldg(plane + (int64_t)(y + r) * SW + (x + r)) == nodata) v = nodata;
+        dst[(int64_t)b * out_plane + (int64_t)y * W + x] = v;
+      }
+    }
+  }
+}
+
+static int floor_log2(int v) { int k = 0; while ((2 << k) <= v) ++k; return k; }
+
+// shared memory of moving_max_chord_kernel for the chord half-widths `hw` (levels x pitch cells,
+// then the sentinel cells)
+template <typename T>
+static size_t chord_smem(int r, int max_hw, int* n_levels, int* pitch) {
+  *n_levels = floor_log2(2 * max_hw + 1) + 1;
+  const int vec = 16 / (int)sizeof(T);
+  *pitch = (MMC_TX + 2 * r + vec - 1) / vec * vec;
+  return ((size_t)*n_levels * *pitch + MMC_TX) * sizeof(T);
+}
+
+template <typename T>
+static int launch_moving_max_chord(const Staged& in, Staged& out, T nd, int has_nodata, int bands, int H,
+                                   int W, int size, const std::vector<int>& hw, cudaStream_t s) {
+  const int r = size / 2;
+  const int max_hw = *std::max_element(hw.begin(), hw.end());
+  int n_levels = 0, pitch = 0;
+  const size_t smem = chord_smem<T>(r, std::max(max_hw, 0), &n_levels, &pitch);
+  int dev = 0, limit = 0;
+  GM_CUDA(cudaGetDevice(&dev));
+  GM_CUDA(cudaDeviceGetAttribute(&limit, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  if (smem > (size_t)limit) {
+    int largest = size, lv, pt;
+    while (largest > 1 && chord_smem<T>(largest / 2, largest / 2, &lv, &pt) > (size_t)limit) largest -= 2;
+    return fail("gm_moving_max: size " + std::to_string(size) + " needs " + std::to_string(smem) +
+                " bytes of shared memory per block for " + std::to_string(sizeof(T)) +
+                "-byte cells, above the device's " + std::to_string(limit) + "; the largest size for this dtype is " +
+                std::to_string(largest));
+  }
+  // per footprint row: offsets of the two level-k windows that cover its chord, relative to the
+  // block's first output column
+  std::vector<int2> chord(2 * r + 1);
+  for (int d = 0; d <= 2 * r; ++d) {
+    const int w = hw[d];
+    if (w < 0) {
+      chord[d] = make_int2(n_levels * pitch, n_levels * pitch);   // the sentinel cells
+      continue;
+    }
+    const int k = floor_log2(2 * w + 1);
+    chord[d] = make_int2(k * pitch + r - w, k * pitch + r + w - (1 << k) + 1);
+  }
+  void* dev_chord = nullptr;
+  if (upload(&dev_chord, chord.data(), (int64_t)chord.size() * sizeof(int2), s)) return 1;
+  auto kernel = moving_max_chord_kernel<T>;
+  if (smem > 48 * 1024)
+    GM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid3(W, H, bands, MMC_TX, MMC_GROUPS * MMC_ROWS), MMC_THREADS, smem, s>>>(
+      (const T*)in.dev, (T*)out.dev, nd, has_nodata, bands, H, W, r, n_levels, pitch, (const int2*)dev_chord);
+  cudaError_t e = cudaGetLastError();
+  cudaFreeAsync(dev_chord, s);
+  if (e != cudaSuccess) return fail(std::string("moving_max launch: ") + cudaGetErrorString(e));
+  count_launch();
+  return 0;
+}
+
 // ---------------------------------------------------------------------------------
 // Dilate (raster/spatial.py:146-155): 6-connected 3-D cross, values in order
 // ---------------------------------------------------------------------------------
@@ -1340,7 +1463,6 @@ template <typename T>
 static int run_moving_max(const Staged& in, Staged& out, const void* nodata, int has_nodata,
                           int bands, int H, int W, int SW, int size, cudaStream_t s) {
   const int r = size / 2;
-  if (r > MM_MAXR) return fail("gm_moving_max: size too large (max 65)");
   // chord half-widths of the disc x^2 + y^2 < (size/2)^2 (utils.py:536-547)
   std::vector<int> hw(2 * r + 1);
   const double rad2 = (size / 2.0) * (size / 2.0);
@@ -1358,7 +1480,14 @@ static int run_moving_max(const Staged& in, Staged& out, const void* nodata, int
   if (SW != W + 2 * r)
     return fail("gm_moving_max: a source wider than the output plus its halo (pitch padding) is only "
                 "supported for 4-byte rasters and odd sizes 3..15");
-  if (r >= 1 && r <= MM2_MAXR) {
+  // The tiled kernel up to radius 8, except 8-byte cells at radius 7 and 8, where the chord
+  // kernel is faster (16384^2 on a B200, profiles/r07_moving_max_sizes.json: int64 size 15 14.2
+  // against 17.2 ms, float64 size 17 17.5 against 18.9; every 1-, 2- and 4-byte case and int64
+  // up to size 11 run 1.6-4x faster tiled).  GM_MOVING_MAX_KERNEL=tiled or =chord overrides the
+  // choice up to radius 8, so that tools/moving_max_bench.py can time the two against each other.
+  const char* kernel_env = getenv("GM_MOVING_MAX_KERNEL");
+  const bool tiled = kernel_env ? strcmp(kernel_env, "tiled") == 0 : !(sizeof(T) == 8 && r >= 7);
+  if (r >= 1 && r <= MM2_MAXR && tiled) {
     MMFootprint fp;
     memset(&fp, 0, sizeof(fp));
     for (int i = 0; i < 2 * MM2_MAXR + 1; ++i) fp.level[i] = -1;
@@ -1384,20 +1513,8 @@ static int run_moving_max(const Staged& in, Staged& out, const void* nodata, int
       return 0;
     }
   }
-  void* dev_hw = nullptr;
-  if (upload(&dev_hw, hw.data(), (int64_t)hw.size() * sizeof(int), s)) return 1;
-  const size_t smem = (size_t)(MM_TX + 2 * r) * (MM_TY + 2 * r) * sizeof(T);
-  auto kernel = moving_max_kernel<T>;
-  if (smem > 48 * 1024)
-    GM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid3(W, H, bands, MM_TX, MM_TY), dim3(MM_TX, MM_TY), smem, s>>>(
-      (const T*)in.dev, (T*)out.dev, has_nodata ? read_scalar<T>(nodata) : T(0), has_nodata, bands,
-      H, W, r, (const int*)dev_hw);
-  cudaError_t e = cudaGetLastError();
-  cudaFreeAsync(dev_hw, s);
-  if (e != cudaSuccess) return fail(std::string("moving_max launch: ") + cudaGetErrorString(e));
-  count_launch();
-  return 0;
+  return launch_moving_max_chord<T>(in, out, has_nodata ? read_scalar<T>(nodata) : T(0), has_nodata, bands, H,
+                                    W, size, hw, s);
 }
 
 template <typename T>
