@@ -5,7 +5,7 @@ from datetime import datetime, timedelta
 import numpy as np
 import pytest
 
-from dask_geomodeling_b200 import raster, workloads
+from dask_geomodeling_b200 import _native, raster, workloads
 from oracle import raster as R
 
 pytestmark = pytest.mark.gpu
@@ -27,8 +27,8 @@ def times(n):
     return [datetime(2000, 1, 1) + timedelta(hours=i) for i in range(n)]
 
 
-# (19, 45): 855 cells, no whole 16-byte pixel groups -> the one-pixel-per-thread kernels;
-# (16, 48): 768 cells -> the streaming kernels (16-byte loads, several pixels per thread)
+# (19, 45): 855 cells, no whole 16-byte pixel groups -> one pixel per thread (VEC = 1);
+# (16, 48): 768 cells -> 16-byte loads, several pixels per thread
 SHAPES = [(19, 45), (16, 48)]
 
 
@@ -98,4 +98,63 @@ def test_temporal_aggregate_view():
     view = raster.TemporalAggregate(src, "6h", "sum")
     got = view.get_data(**workloads.request(32, 32, start=datetime(1970, 1, 1), stop=datetime(1970, 1, 2)))
     expected, _ = R.temporal_aggregate(values, nodata, "sum", [range(0, 6), range(6, 12)])
+    np.testing.assert_array_equal(got["values"], expected)
+
+
+def offset_on_device(values):
+    """``values`` on the device one element past a 16-byte aligned base: the plane is whole
+    16-byte groups, the pointer is not."""
+    flat = np.concatenate([np.zeros(1, values.dtype), values.ravel()])
+    base = _native.DeviceArray.from_host(flat)
+    view = _native.DeviceArray(values.shape, values.dtype, ptr=base.ptr + values.dtype.itemsize, owner=base)
+    assert view.ptr % 16 != 0
+    return view
+
+
+@pytest.mark.parametrize("statistic", ["sum", "mean", "std"])
+def test_aggregate_unaligned_source(statistic):
+    values, nodata = stack("f4", shape=(16, 48))
+    expected, _ = R.temporal_aggregate(values, nodata, statistic, [range(11)])
+    kwargs = dict(mode="vals", start=times(11)[-1], stop=None, frequency=None, timezone=None,
+                  closed=None, label=None, dtype=expected.dtype.str, statistic=statistic)
+    got = raster.TemporalAggregate.process(kwargs, {"time": times(11)},
+                                           {"values": offset_on_device(values), "no_data_value": nodata})
+    np.testing.assert_array_equal(np.asarray(got["values"]), expected)
+
+
+def test_cumulative_unaligned_source():
+    values, nodata = stack("f4", frames=10, shape=(16, 48))
+    ts = times(10)
+    expected, _ = R.cumulative(values, nodata, "sum", [range(10)], np.ones(10, bool))
+    kwargs = dict(mode="vals", start=ts[0], stop=ts[-1], frequency=None, timezone=None,
+                  closed="right", label="right", dtype=expected.dtype.str, statistic="sum")
+    got = raster.Cumulative.process(kwargs, {"time": ts},
+                                    {"values": offset_on_device(values), "no_data_value": nodata})
+    np.testing.assert_array_equal(np.asarray(got["values"]), expected)
+
+
+@pytest.mark.parametrize("statistic", ["median", "p90"])
+def test_aggregate_long_bin_float64(statistic):
+    # 600 frames of an int32 source: float64 working dtype, 1024 sort slots per pixel
+    values, nodata = stack("i4", frames=600)
+    name, q = (statistic, None) if not statistic.startswith("p") else ("percentile", float(statistic[1:]))
+    expected, _ = R.temporal_aggregate(values, nodata, name, [range(600)], q)
+    kwargs = dict(mode="vals", start=times(600)[-1], stop=None, frequency=None, timezone=None,
+                  closed=None, label=None, dtype=expected.dtype.str, statistic=statistic)
+    got = raster.TemporalAggregate.process(kwargs, {"time": times(600)},
+                                           {"values": values, "no_data_value": nodata})
+    assert expected.dtype == np.float64
+    np.testing.assert_array_equal(got["values"], expected)
+
+
+def test_sum_int64_past_2_53():
+    # int64 samples are added in float64, as NumPy adds them: 3 * (2**53 + 1) -> 3 * 2**53
+    values = np.full((3, 16, 48), 2 ** 53 + 1, dtype=np.int64)
+    nodata = R.dtype_max(np.int64)
+    expected, _ = R.temporal_aggregate(values, nodata, "sum", [range(3)])
+    assert expected[0, 0, 0] == 3 * 2 ** 53
+    kwargs = dict(mode="vals", start=times(3)[-1], stop=None, frequency=None, timezone=None,
+                  closed=None, label=None, dtype=expected.dtype.str, statistic="sum")
+    got = raster.TemporalAggregate.process(kwargs, {"time": times(3)},
+                                           {"values": values, "no_data_value": nodata})
     np.testing.assert_array_equal(got["values"], expected)
